@@ -2,12 +2,12 @@
 """bench.py — BASELINE.json configs[1]: PCSR 1e5 x 1e5 with 1e7 nnz resident in HBM; one step = one batched update of
 1M logical entries (both orientations) followed by one SpMV (A * x, dense x).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-Prints ONE JSON line (contract in the task statement).
+Prints ONE JSON line.
   value              whole-job Mupdates/s with inputs resident in HBM on the stationary chain (each 1M-update batch inserts
-                     ~0.5M new entries, overwrites a few, deletes the previous batch's inserts): K steps per repeat, `repeats`
-                     back-to-back repeats so that the timed region lasts >= 1 s (the clock sampler lands inside it)
+                     ~0.5M new entries, overwrites a few, deletes the previous batch's inserts): exactly K timed steps after
+                     max(W, 3) warm-up steps
   value_insert_only  configs[1] as written: fresh 1e7-nnz matrix -> ONE batched insert of 1M new entries -> SpMV (the matrix is
                      restored from a pristine device clone outside the timed bracket of every repetition)
   e2e                the stationary step through the host-pointer C-ABI calls (pinned host buffers; every H2D copy of the batch
@@ -17,6 +17,9 @@ Prints ONE JSON line (contract in the task statement).
   roofline / spmv    dominant kernel of the step / the SpMV kernel against the measured HBM peak
   cpu_baseline       the CPU oracle (C++ restatement of the reference, 1 core) on the same W+K steps
 `--impl reference` times the oracle on the same W+K batches (same generator, same x) and prints the same checksum.
+`--dump-outputs DIR` writes what the timed path returned after its last step (outputs_of_last_step) and y of the insert-only
+step as float64 .npy files, ~34 MB; the inputs depend on W and K only, so two builds run with the same arguments can be
+compared file by file.
 """
 import argparse
 import ctypes as C
@@ -40,6 +43,7 @@ SEED = 0xD5A00002
 BYTES_PER_UPDATE = 80          # SURVEY.md §8d: 2 orientations x (24 B triple read + 16 B cell write)
 BYTES_PER_UPDATE_ONE = 40      # one orientation (what a single kernel launch of the update pipeline processes)
 SPMV_RTOL = 1e-12              # north_star: Float64 SpMV within 1e-12 relative
+DUMP_SAMPLE = 1 << 20          # stored entries in the seeded sample of --dump-outputs (3 arrays x 8 MB)
 
 
 def make_workload(ncycle, m=M_ROWS, n=N_COLS, nnz0=NNZ0, nb=BATCH, seed=SEED):
@@ -167,6 +171,22 @@ def rel_err(y, yo):
     return float(r.max()) if len(r) else 0.0
 
 
+def outputs_of_last_step(A, y, last_batch):
+    """What a caller of the timed step holds after its last step: y = A * x, the values stored at the last batch's (i, j)
+    (getindex), and a seeded sample of DUMP_SAMPLE stored entries (rows, cols, vals in column-major order, to_coo).  ~33 MB."""
+    import dsa_b200 as D
+    rows, cols, vals = D.to_coo(A)
+    pick = np.sort(np.random.default_rng(SEED).choice(len(rows), min(DUMP_SAMPLE, len(rows)), replace=False))
+    return {"y": y, "batch_vals": A.get_batch(last_batch[0], last_batch[1]),
+            "entries_rows": rows[pick], "entries_cols": cols[pick], "entries_vals": vals[pick]}
+
+
+def dump_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def oracle_chain(coo, batches, x, insert_only=None):
     """The reference's CPU path on the same inputs: build, then per step a loop of setindex! over the batch (the reference has
     no batched update, matrix.jl:119-121) + mat * x.  One host core (C++ oracle; Julia is not installed).  Returns the
@@ -240,11 +260,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the oracle legs (cpu_baseline AND the parity check)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-c4", action="store_true", help="multi-GPU arm: skip the full-size configs[3] run")
-    ap.add_argument("--min-timed-s", type=float, default=1.0, help="the K-step region is repeated until this much time is covered")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or world > 1 or os.environ.get("DSA_BENCH_FORCE_DIST") == "1"):
+        ap.error("--dump-outputs is implemented for the single-GPU arm of --impl ours")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -296,7 +320,7 @@ def main():
         step_dev(s)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    # repeat 0: exactly K steps; afterwards the structure has seen batches 0 .. W+K-1 = one full cycle -> parity snapshot
+    # the timed region: exactly K steps; afterwards the structure has seen batches 0 .. W+K-1 = one full cycle -> parity snapshot
     launches0 = L.dsa_launch_count()
     t_w0 = time.perf_counter()
     e0.record(stream)
@@ -304,30 +328,14 @@ def main():
         step_dev(s)
     e1.record(stream)
     torch.cuda.synchronize()
-    ms_first = e0.elapsed_time(e1)
-    launches_first = L.dsa_launch_count() - launches0
+    ms_total = e0.elapsed_time(e1)
+    launches = L.dsa_launch_count() - launches0
     windows.append((t_w0, time.perf_counter()))
     y_gpu = d_y.cpu().numpy().copy()
     nnz_gpu = A.info(1)["nnz"]
-    # repeats 1 .. R-1: the same K-step region back to back, continuing around the cycle, until >= min_timed_s is covered
-    R = int(min(400, max(1, np.ceil(1.1 * args.min_timed_s * 1e3 / max(ms_first, 1e-3)) + 1)))   # the first repeat is the slowest
-    ms_rest = 0.0
+    dumped = outputs_of_last_step(A, y_gpu, batches[(W + K - 1) % P]) if args.dump_outputs else None
     s_next = W + K
-    if R > 1:
-        torch.cuda.synchronize()
-        t_w0 = time.perf_counter()
-        e0.record(stream)
-        for _ in range(R - 1):
-            for s in range(s_next, s_next + K):
-                step_dev(s)
-            s_next += K
-        e1.record(stream)
-        torch.cuda.synchronize()
-        ms_rest = e0.elapsed_time(e1)
-        windows.append((t_w0, time.perf_counter()))
-    launches = L.dsa_launch_count() - launches0
-    ms_total = ms_first + ms_rest
-    ms_step = ms_total / (R * K)
+    ms_step = ms_total / K
     value = BATCH / (ms_step * 1e-3) / 1e6
     checksum = float(y_gpu.sum())
 
@@ -435,18 +443,17 @@ def main():
         run_host(s_next, s_next + W)
         s_next += W
         torch.cuda.synchronize()
-        Re = int(min(100, max(1, R // 2)))
         t_w0 = time.perf_counter()
         e0.record(stream)
-        run_host(s_next, s_next + Re * K)
+        run_host(s_next, s_next + K)
         e1.record(stream)
         torch.cuda.synchronize()
         wall = time.perf_counter() - t_w0
         windows.append((t_w0, t_w0 + wall))
-        s_next += Re * K
-        ms_e2e = max(e0.elapsed_time(e1), wall * 1e3) / (Re * K)
+        s_next += K
+        ms_e2e = max(e0.elapsed_time(e1), wall * 1e3) / K
         e2e = {"value": BATCH / (ms_e2e * 1e-3) / 1e6, "unit": "Mupdates/s", "h2d_bytes_per_step": 24 * BATCH + 8 * N_COLS,
-               "d2h_bytes_per_step": 8 * M_ROWS, "ms_per_step": ms_e2e, "repeats": Re, "checksum": float(h_y.sum().item()),
+               "d2h_bytes_per_step": 8 * M_ROWS, "ms_per_step": ms_e2e, "steps": K, "checksum": float(h_y.sum().item()),
                "api": "dsa_matrix_stage_batch + dsa_matrix_apply_staged + dsa_matrix_spmv_dense (host pinned buffers)"}
         # the same step through the plain synchronous call (no overlap of the copy), for reference
         torch.cuda.synchronize()
@@ -482,15 +489,18 @@ def main():
 
     line = {
         "metric": "batched PCSR insert/delete Mupdates/s", "value": value, "unit": "Mupdates/s", "n_gpus": 1, "steps": K, "warmup": W,
-        "ms_per_step": ms_step, "repeats": R, "timed_region_s": ms_total * 1e-3, "ms_per_step_first_repeat": ms_first / K,
+        "ms_per_step": ms_step, "timed_steps": K, "timed_region_s": ms_total * 1e-3,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "value_insert_only": BATCH / (io_ms_step * 1e-3) / 1e6, "ms_per_step_insert_only": io_ms_step, "insert_only_repetitions": len(io_ms),
         "dtype": "int64 keys / f64 values", "data": "synthetic", "config": workload_config(1), "clocks": clocks, "e2e": e2e,
-        "gpu_launches": int(launches), "gpu_launches_per_step": launches_first / K, "parity": parity,
+        "gpu_launches": int(launches), "gpu_launches_per_step": launches / K, "parity": parity,
         "roofline": roofline, "spmv": spmv, "cpu_baseline": cpu,
         "update_effective_gbs": BYTES_PER_UPDATE * BATCH / (ms_step * 1e-3) / 1e9, "kernels": kernels, "checksum": checksum,
         "checksum_after_steps": W + K, "nnz_after": int(nnz_gpu),
     }
+    if dumped is not None:
+        dumped["y_insert_only"] = y_io
+        dump_outputs(args.dump_outputs, dumped)
     print(json.dumps(line))
     if parity.get("checked") and not parity["ok"]:
         sys.exit(3)

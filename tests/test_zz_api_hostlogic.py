@@ -335,3 +335,29 @@ def test_missing_dimension_is_guessed_on_its_own(backend):   # matrix.jl:15: m =
     assert B.size == (3, 9)
     y = A.mul_dense(np.ones(5), trans=True)
     assert len(y) == 7 and y[1] == 1.0 and y[6] == 2.0
+
+
+def test_bench_dump_outputs(backend, tmp_path, monkeypatch):
+    """bench.py --dump-outputs at a reduced size: the last batch's values read back last-writer-wins, the entry sample is a
+    seeded subset of to_coo, and every file is float64."""
+    import bench as B
+    monkeypatch.setattr(B, "N_OVER", 200)
+    monkeypatch.setattr(B, "DUMP_SAMPLE", 3000)
+    x, coo, batches, _ = B.make_workload(3, m=3000, n=3000, nnz0=20_000, nb=4000, seed=11)
+    A = D.dynamicsparse(coo[0], coo[1], coo[2], m=3000, n=3000)
+    for b in batches:
+        A.set_batch(*b)
+    y = A.mul_dense(x)
+    B.dump_outputs(str(tmp_path), B.outputs_of_last_step(A, y, batches[-1]))
+    got = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sorted(got) == ["batch_vals", "entries_cols", "entries_rows", "entries_vals", "y"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["y"], y)
+    bi, bj, bv = batches[-1]
+    lin = bi * 3001 + bj
+    last = len(lin) - 1 - np.unique(lin[::-1], return_index=True)[1]   # the last write of every (i, j) in the batch
+    assert np.array_equal(got["batch_vals"][last], bv[last])
+    r, c, v = D.to_coo(A)
+    pick = np.sort(np.random.default_rng(B.SEED).choice(len(r), 3000, replace=False))
+    assert np.array_equal(got["entries_rows"], r[pick]) and np.array_equal(got["entries_cols"], c[pick])
+    assert np.array_equal(got["entries_vals"], v[pick])
