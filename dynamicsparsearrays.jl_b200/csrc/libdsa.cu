@@ -1,5 +1,6 @@
 // libdsa — C ABI (include/dsa.h) over the device structures of pma.cuh / pcsr.cuh.
 // Host orchestration only: every data-parallel step is a kernel launched on the handle's stream.
+#include <cstdlib>
 #include <functional>
 #include <memory>
 #include <mutex>
@@ -25,7 +26,7 @@ DevicePool& device_pool(int device) {
 static thread_local std::string g_last_error;
 
 // ---------------------------------------------------------------------------------------------
-// Pcsr::set_batch_d — batched setindex! of one orientation (pcsr.jl:341-347 per op), DESIGN.md §4
+// batched setindex! of one orientation (pcsr.jl:341-347 per op), DESIGN.md §4; sequenced by matrix_set_batch_two
 // ---------------------------------------------------------------------------------------------
 struct BatchStats {
     int64_t missing, minkey, maxkey, maxpart_nz, maxkey_nz, minpart, maxbucket;
@@ -283,35 +284,13 @@ static void phase2_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
     exclusive_scan_i32<int32_t>(ws.batch.scan, flag, uidx, ntot, nuniq_dev, st);
     DSA_LAUNCH("gather_unique_ops", k_gather_unique_ops, grt, 256, 0, st, sk, perm, flag, uidx, ntot, n, kb, c.inkeys, c.vals, u_pid,
                u_key, u_val);
-    P.pma.apply_sorted_ops(ws.batch, u_pid, u_key, u_val, ntot, P.d_sem.p, P.d_next_slot.p, st, false, nuniq_dev, /*launch_only=*/true);
+    P.pma.apply_sorted_ops(ws.batch, u_pid, u_key, u_val, ntot, P.d_sem.p, P.d_next_slot.p, st, nuniq_dev, /*launch_only=*/true);
 }
 
 static void phase3(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t st) {
     P.pma.rebalance_finish(ws.batch, P.d_sem.p, st);
     if (c.bs.maxkey > P.max_inkey) P.max_inkey = c.bs.maxkey;
     if (!c.new_slots_h.empty()) P.rebuild_live_and_upload(st);   // the new partitions are placed now: they end the spans before them
-}
-
-void Pcsr::set_batch_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals, int64_t n,
-                       int64_t* max_part_nz, int64_t* max_key_nz, cudaStream_t st) {
-    if (n <= 0) return;
-    BatchCtx c;
-    c.inkeys = d_inkeys; c.partkeys = d_partkeys; c.vals = d_vals; c.n = n;
-    phase1_launch(*this, ws, c, st);
-    DSA_CUDA(cudaStreamSynchronize(st));
-    phase1_read(ws, c);
-    if (tile_refused(*this, c)) {
-        phase1_launch(*this, ws, c, st);
-        DSA_CUDA(cudaStreamSynchronize(st));
-        phase1_read(ws, c);
-    }
-    phase1_validate(*this, c, "in-array keys");
-    if (max_part_nz) *max_part_nz = c.bs.maxpart_nz;
-    if (max_key_nz) *max_key_nz = c.bs.maxkey_nz;
-    phase1_finish(*this, ws, c, st);
-    phase2_launch(*this, ws, c, st);
-    DSA_CUDA(cudaStreamSynchronize(st));
-    phase3(*this, ws, c, st);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -369,7 +348,7 @@ struct dsa_matrix {
     } slot[2];
     cudaStream_t copy_st = nullptr;
     int staged_head = 0, staged_count = 0;
-    // the column-major orientation's batch phases run on their own stream, forked from / joined to sh.st (DSA_TWO_STREAMS=0 disables)
+    // the column-major orientation's batch phases run on their own stream, forked from / joined to sh.st, when both orientations have ops
     cudaStream_t twin_st = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     ~dsa_matrix() {
@@ -418,8 +397,7 @@ static T* h2d(DBuf<T>& buf, const T* h, int64_t n, cudaStream_t st) {
 
 // ---- vector batch (plain PMA): sort by key, last writer wins, merge -----------------------------------------------
 static void vec_sorted_unique(dsa_vec* v, const int64_t* d_keys, const double* d_vals, int64_t n, bool build, int combine,
-                              int64_t** out_k, double** out_v, int64_t* nuniq_host, int64_t** nuniq_dev, int64_t* maxkey_nz,
-                              int64_t* maxkey) {
+                              int64_t** out_k, double** out_v, int64_t* nuniq_host, int64_t** nuniq_dev, int64_t* maxkey) {
     cudaStream_t st = v->sh.st;
     PcsrWorkspace& ws = v->ws;
     int64_t* mm = ws.cs.ensure(CS_WORDS);
@@ -459,7 +437,6 @@ static void vec_sorted_unique(dsa_vec* v, const int64_t* d_keys, const double* d
         DSA_CUDA(cudaMemcpyAsync(nuniq_host, tot, 8, cudaMemcpyDeviceToHost, st));
         DSA_CUDA(cudaStreamSynchronize(st));
     }
-    (void)maxkey_nz;
 }
 
 __global__ void __launch_bounds__(256) k_max_key_nonzero(const int64_t* __restrict__ keys, const double* __restrict__ vals, int64_t n,
@@ -498,33 +475,36 @@ static void vec_set_batch_dev(dsa_vec* v, const int64_t* d_keys, const double* d
     DSA_CUDA(cudaMemcpyAsync(&h_mx, mx, 8, cudaMemcpyDeviceToHost, st));
     int64_t *uk, *nu_dev, maxkey;
     double* uv;
-    vec_sorted_unique(v, d_keys, d_vals, n, false, 0, &uk, &uv, nullptr, &nu_dev, nullptr, &maxkey);   // syncs (h_mx valid after)
-    v->pma.apply_sorted_ops(v->ws.batch, nullptr, uk, uv, n, nullptr, nullptr, st, false, nu_dev);
+    vec_sorted_unique(v, d_keys, d_vals, n, false, 0, &uk, &uv, nullptr, &nu_dev, &maxkey);   // syncs (h_mx valid after)
+    v->pma.apply_sorted_ops(v->ws.batch, nullptr, uk, uv, n, nullptr, nullptr, st, nu_dev);
     if (h_mx != INT64_MIN && h_mx > v->n) v->n = h_mx;
 }
 
 // ---- matrix helpers -----------------------------------------------------------------------------------------------
-// The two orientations go through the batch phases together so that they share the host decisions.  A plain matrix batch feeds
-// both with the same triples; a shard of a distributed matrix feeds them different ones.
+// One orientation's part of a matrix batch: its structure, its scratch, its ops, the stream its phases run on and the two
+// dimensions its keys grow.
+struct OrientationBatch {
+    Pcsr& P;
+    PcsrWorkspace& ws;
+    BatchCtx c;
+    cudaStream_t st;
+    int64_t& part_dim;   // grown by the partition keys of non-zero writes
+    int64_t& key_dim;    // grown by the in-array keys of non-zero writes
+};
+
+// The orientations that have ops go through the batch phases together so that they share the host decisions.  A plain matrix
+// batch feeds both with the same triples; a shard of a distributed matrix feeds them different ones; the delete list of
+// deletecolumn! / deleterow! feeds only the twin of the purged orientation.
 // nc_dev / nr_dev (nullable): device-side op counts; nc / nr are then upper bounds (distributed batches).
 static void matrix_set_batch_two(dsa_matrix* A, const int64_t* rows_c, const int64_t* cols_c, const double* vals_c, int64_t nc,
                                  const int64_t* rows_r, const int64_t* cols_r, const double* vals_r, int64_t nr,
                                  const int64_t* nc_dev = nullptr, const int64_t* nr_dev = nullptr,
                                  const std::function<void()>* pre_mutate = nullptr) {
     cudaStream_t st = A->sh.st;
-    BatchCtx cc, cr;
-    cc.inkeys = rows_c; cc.partkeys = cols_c; cc.vals = vals_c; cc.n = nc; cc.n_dev = nc_dev;   // colmajor[row, col] = v  (matrix.jl:53-55)
-    cr.inkeys = cols_r; cr.partkeys = rows_r; cr.vals = vals_r; cr.n = nr; cr.n_dev = nr_dev;   // rowmajor[col, row] = v  (matrix.jl:57-59)
-    // The two orientations are independent (own structure, own workspace), so the column-major one runs on a second, low-priority
-    // stream (stc) that forks from st here; the row-major one stays on st and, being ahead, finishes first.
-    // DSA_TWO_STREAMS=0 puts everything back on one stream (stc == st).
-    static const bool two_streams = [] {
-        const char* e = getenv("DSA_TWO_STREAMS");
-        return !e || atoi(e) != 0;
-    }();
-    const bool use_two = two_streams && nc > 0 && nr > 0;
-    cudaStream_t stc = st;
-    if (use_two) {
+    // The two orientations are independent (own structure, own workspace), so when both have ops the column-major one runs on a
+    // second, low-priority stream that forks from st here; the row-major one stays on st and, being ahead, finishes first.
+    const bool two = nc > 0 && nr > 0;
+    if (two) {
         if (!A->twin_st) {
             int least = 0, greatest = 0;
             DSA_CUDA(cudaDeviceGetStreamPriorityRange(&least, &greatest));
@@ -532,52 +512,53 @@ static void matrix_set_batch_two(dsa_matrix* A, const int64_t* rows_c, const int
             DSA_CUDA(cudaEventCreateWithFlags(&A->ev_fork, cudaEventDisableTiming));
             DSA_CUDA(cudaEventCreateWithFlags(&A->ev_join, cudaEventDisableTiming));
         }
-        stc = A->twin_st;
         DSA_CUDA(cudaEventRecord(A->ev_fork, st));        // everything queued on st so far (input copies) precedes the twin's work
-        DSA_CUDA(cudaStreamWaitEvent(stc, A->ev_fork, 0));
+        DSA_CUDA(cudaStreamWaitEvent(A->twin_st, A->ev_fork, 0));
     }
+    // row-major first: rowmajor[col, row] = v (matrix.jl:57-59), then colmajor[row, col] = v (matrix.jl:53-55)
+    std::vector<OrientationBatch> obs;
+    obs.reserve(2);
+    if (nr > 0) obs.push_back({A->rowmajor, A->ws2, {cols_r, rows_r, vals_r, nr, nr_dev}, st, A->m, A->n});
+    if (nc > 0) obs.push_back({A->colmajor, A->ws, {rows_c, cols_c, vals_c, nc, nc_dev}, two ? A->twin_st : st, A->n, A->m});
     try {
-        if (nr > 0) phase1_launch(A->rowmajor, A->ws2, cr, st);
-        if (nc > 0) phase1_launch(A->colmajor, A->ws, cc, stc);
-        DSA_CUDA(cudaStreamSynchronize(st));
-        if (stc != st) DSA_CUDA(cudaStreamSynchronize(stc));
-        if (nc > 0) { phase1_read(A->ws, cc); nc = cc.n; }
-        if (nr > 0) { phase1_read(A->ws2, cr); nr = cr.n; }
-        {   // a refused tile-streamed attempt starts over on the general path (nothing was modified)
-            const bool rc = nc > 0 && tile_refused(A->colmajor, cc), rr = nr > 0 && tile_refused(A->rowmajor, cr);
-            if (rr) phase1_launch(A->rowmajor, A->ws2, cr, st);
-            if (rc) phase1_launch(A->colmajor, A->ws, cc, stc);
-            if (rr) DSA_CUDA(cudaStreamSynchronize(st));
-            if (rc) DSA_CUDA(cudaStreamSynchronize(stc));
-            if (rc) phase1_read(A->ws, cc);
-            if (rr) phase1_read(A->ws2, cr);
-        }
+        for (OrientationBatch& o : obs) phase1_launch(o.P, o.ws, o.c, o.st);
+        for (OrientationBatch& o : obs) DSA_CUDA(cudaStreamSynchronize(o.st));
+        for (OrientationBatch& o : obs) phase1_read(o.ws, o.c);   // c.n is exact from here on: a distributed batch may bring 0 ops
+        // a refused tile-streamed attempt starts over on the general path (nothing was modified)
+        std::vector<OrientationBatch*> redo;
+        for (OrientationBatch& o : obs)
+            if (o.c.n > 0 && tile_refused(o.P, o.c)) redo.push_back(&o);
+        for (OrientationBatch* o : redo) phase1_launch(o->P, o->ws, o->c, o->st);
+        for (OrientationBatch* o : redo) DSA_CUDA(cudaStreamSynchronize(o->st));
+        for (OrientationBatch* o : redo) phase1_read(o->ws, o->c);
         if (pre_mutate) (*pre_mutate)();   // caller-side validation that needs the first host synchronisation (may throw: nothing is mutated yet)
         // validate before mutate: rows are the in-array keys of the col-major structure, columns those of the row-major one
-        // (both orientations are checked before either one creates a column)
-        if (nc > 0) phase1_validate(A->colmajor, cc, "row and column keys");
-        if (nr > 0) phase1_validate(A->rowmajor, cr, "row and column keys");
-        if (nr > 0) phase1_finish(A->rowmajor, A->ws2, cr, st);
-        if (nc > 0) phase1_finish(A->colmajor, A->ws, cc, stc);
-        if (nr > 0) phase2_launch(A->rowmajor, A->ws2, cr, st);
-        if (nc > 0) phase2_launch(A->colmajor, A->ws, cc, stc);
-        DSA_CUDA(cudaStreamSynchronize(st));
-        if (nr > 0) phase3(A->rowmajor, A->ws2, cr, st);     // the row-major orientation is not held back by the other one
-        if (stc != st) DSA_CUDA(cudaStreamSynchronize(stc));
-        if (nc > 0) phase3(A->colmajor, A->ws, cc, stc);
-        if (stc != st) {   // later work on st that needs the column-major orientation sees its merges
-            DSA_CUDA(cudaEventRecord(A->ev_join, stc));
+        // (both orientations are checked before either one creates a column; the col-major one first, so that a batch both
+        // refuse reports the col-major one's reason)
+        for (auto o = obs.rbegin(); o != obs.rend(); ++o)
+            if (o->c.n > 0) phase1_validate(o->P, o->c, "row and column keys");
+        for (OrientationBatch& o : obs)
+            if (o.c.n > 0) phase1_finish(o.P, o.ws, o.c, o.st);
+        for (OrientationBatch& o : obs)
+            if (o.c.n > 0) phase2_launch(o.P, o.ws, o.c, o.st);
+        for (OrientationBatch& o : obs) {   // the row-major orientation's phase 3 is not held back by the other one
+            DSA_CUDA(cudaStreamSynchronize(o.st));
+            if (o.c.n > 0) phase3(o.P, o.ws, o.c, o.st);
+        }
+        if (two) {   // later work on st that needs the column-major orientation sees its merges
+            DSA_CUDA(cudaEventRecord(A->ev_join, A->twin_st));
             DSA_CUDA(cudaStreamWaitEvent(st, A->ev_join, 0));
         }
     } catch (...) {
-        if (stc != st) cudaStreamSynchronize(stc);
+        if (two) cudaStreamSynchronize(A->twin_st);
         throw;
     }
-    // matrix.jl:44-47: dimensions grow on non-zero writes
-    if (nc > 0 && cc.bs.maxkey_nz != INT64_MIN && cc.bs.maxkey_nz > A->m) A->m = cc.bs.maxkey_nz;
-    if (nc > 0 && cc.bs.maxpart_nz != INT64_MIN && cc.bs.maxpart_nz > A->n) A->n = cc.bs.maxpart_nz;
-    if (nr > 0 && cr.bs.maxpart_nz != INT64_MIN && cr.bs.maxpart_nz > A->m) A->m = cr.bs.maxpart_nz;
-    if (nr > 0 && cr.bs.maxkey_nz != INT64_MIN && cr.bs.maxkey_nz > A->n) A->n = cr.bs.maxkey_nz;
+    // matrix.jl:44-47: dimensions grow on non-zero writes (the statistics are INT64_MIN when there is none)
+    for (OrientationBatch& o : obs)
+        if (o.c.n > 0) {
+            o.part_dim = std::max(o.part_dim, o.c.bs.maxpart_nz);
+            o.key_dim = std::max(o.key_dim, o.c.bs.maxkey_nz);
+        }
 }
 static void matrix_set_batch_dev(dsa_matrix* A, const int64_t* d_rows, const int64_t* d_cols, const double* d_vals, int64_t n) {
     if (n <= 0) return;
@@ -588,7 +569,6 @@ static void matrix_delete(dsa_matrix* A, bool rows, const int64_t* ids, int64_t 
     if (n <= 0) return;
     cudaStream_t st = A->sh.st;
     Pcsr& primary = rows ? A->rowmajor : A->colmajor;
-    Pcsr& twin = rows ? A->colmajor : A->rowmajor;
     // validate before mutate (pcsr.jl:208)
     std::vector<int32_t> slots;
     {
@@ -605,19 +585,16 @@ static void matrix_delete(dsa_matrix* A, bool rows, const int64_t* ids, int64_t 
     DSA_CUDA(cudaMemcpyAsync(d_slots, slots.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
     DSA_CUDA(cudaMemcpyAsync(d_ids, ids, (size_t)n * 8, cudaMemcpyHostToDevice, st));
     // entries to delete from the twin: for (row, val) in view(matrix, :, col): rowmajor[col, row] = 0  (matrix.jl:97-99)
-    const int64_t tot = primary.gather_spans(A->ws, d_slots, n, d_ids, false, st);
+    // gathered into the primary orientation's own workspace: the twin's batch runs on the other one and reads the list in place
+    PcsrWorkspace& pws = rows ? A->ws2 : A->ws;
+    const int64_t tot = primary.gather_spans(pws, d_slots, n, d_ids, false, st);
     if (tot > 0) {
-        // twin partition key = in-array key of the primary cell, twin in-array key = deleted id, value 0.0
-        // copy out of the shared workspace: the twin batch reuses it
-        DBuf<int64_t> pk, ik;
+        // twin partition key = in-array key of the primary cell (tmp_k), twin in-array key = deleted id (tmp_owner), value 0.0
         DBuf<double> zeros;
-        pk.ensure((size_t)tot);
-        ik.ensure((size_t)tot);
         zeros.ensure((size_t)tot);
-        DSA_CUDA(cudaMemcpyAsync(pk.p, A->ws.tmp_k.p, (size_t)tot * 8, cudaMemcpyDeviceToDevice, st));
-        DSA_CUDA(cudaMemcpyAsync(ik.p, A->ws.tmp_owner.p, (size_t)tot * 8, cudaMemcpyDeviceToDevice, st));
         DSA_CUDA(cudaMemsetAsync(zeros.p, 0, (size_t)tot * 8, st));
-        twin.set_batch_d(A->ws, ik.p, pk.p, zeros.p, tot, nullptr, nullptr, st);
+        if (rows) matrix_set_batch_two(A, pws.tmp_owner.p, pws.tmp_k.p, zeros.p, tot, nullptr, nullptr, nullptr, 0);
+        else matrix_set_batch_two(A, nullptr, nullptr, nullptr, 0, pws.tmp_k.p, pws.tmp_owner.p, zeros.p, tot);
         DSA_CUDA(cudaStreamSynchronize(st));
     }
     primary.delete_slots(A->ws, slots, d_slots, st);   // deletecolumn!(colmajor, col)  (matrix.jl:100)
@@ -704,7 +681,7 @@ int dsa_vec_build(const int64_t* keys, const double* vals, int64_t n, int combin
         double* dv = h2d(v->stg.v, vals, n, st);
         int64_t *uk, *nu_dev, nu = 0, maxkey = 0;
         double* uv;
-        vec_sorted_unique(v.get(), dk, dv, n, true, combine, &uk, &uv, &nu, &nu_dev, nullptr, &maxkey);
+        vec_sorted_unique(v.get(), dk, dv, n, true, combine, &uk, &uv, &nu, &nu_dev, &maxkey);
         v->pma.build_from_sorted(uk, uv, nu, nullptr, st);
         v->n = len_given ? len : std::max<int64_t>(maxkey, 0);   // _guess_length (vector.jl:6) = maximum(keys; init = 0)
     }
@@ -818,7 +795,7 @@ int dsa_vec_shrink_size(dsa_vec_t* v, int64_t* n_out) {
     return DSA_OK;
     DSA_CATCH
 }
-static void export_cells(PcsrWorkspace& ws, Staging& stg, const PmaCore& p, uint8_t* occ, int64_t* keys, double* vals, cudaStream_t st) {
+static void export_cells(Staging& stg, const PmaCore& p, uint8_t* occ, int64_t* keys, double* vals, cudaStream_t st) {
     const int64_t cap = p.g.capacity;
     DBuf<uint8_t> d_occ;
     d_occ.ensure((size_t)cap);
@@ -829,11 +806,10 @@ static void export_cells(PcsrWorkspace& ws, Staging& stg, const PmaCore& p, uint
     DSA_CUDA(cudaMemcpyAsync(keys, dk, (size_t)cap * 8, cudaMemcpyDeviceToHost, st));
     DSA_CUDA(cudaMemcpyAsync(vals, dv, (size_t)cap * 8, cudaMemcpyDeviceToHost, st));
     DSA_CUDA(cudaStreamSynchronize(st));
-    (void)ws;
 }
 int dsa_vec_export(dsa_vec_t* v, uint8_t* occupied, int64_t* keys, double* vals) {
     DSA_TRY
-    export_cells(v->ws, v->stg, v->pma, occupied, keys, vals, v->sh.st);
+    export_cells(v->stg, v->pma, occupied, keys, vals, v->sh.st);
     return DSA_OK;
     DSA_CATCH
 }
@@ -1094,7 +1070,7 @@ int dsa_matrix_export(dsa_matrix_t* A, int which, uint8_t* occupied, int64_t* ke
     DSA_TRY
     Pcsr& P = which == DSA_COLMAJOR ? A->colmajor : A->rowmajor;
     cudaStream_t st = A->sh.st;
-    export_cells(A->ws, A->stg, P.pma, occupied, keys, vals, st);
+    export_cells(A->stg, P.pma, occupied, keys, vals, st);
     const int64_t ns = P.nslots();
     if (ns > 0) {
         DSA_CUDA(cudaMemcpyAsync(semaphores, P.d_sem.p, (size_t)ns * 8, cudaMemcpyDeviceToHost, st));
@@ -1104,49 +1080,6 @@ int dsa_matrix_export(dsa_matrix_t* A, int which, uint8_t* occupied, int64_t* ke
             col_keys[s] = P.slot_live[(size_t)s] ? P.slot_key[(size_t)s] : 0;
             col_live[s] = P.slot_live[(size_t)s];
         }
-    }
-    return DSA_OK;
-    DSA_CATCH
-}
-
-// ---- sharded use ------------------------------------------------------------------------------------------------------
-int dsa_matrix_build_one(dsa_matrix_t* A, int which, const int64_t* inkeys, const int64_t* partkeys, const double* vals, int64_t n,
-                         int combine) {
-    DSA_TRY
-    cudaStream_t st = A->sh.st;
-    Pcsr& P = which == DSA_COLMAJOR ? A->colmajor : A->rowmajor;
-    int64_t* dk = h2d(A->stg.a, inkeys, n, st);
-    int64_t* dp = h2d(A->stg.b, partkeys, n, st);
-    double* dv = h2d(A->stg.v, vals, n, st);
-    P.build_coo_d(A->ws, dk, dp, dv, n, combine, st);
-    DSA_CUDA(cudaStreamSynchronize(st));
-    return DSA_OK;
-    DSA_CATCH
-}
-int dsa_matrix_set_batch_one_d(dsa_matrix_t* A, int which, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals,
-                               int64_t n) {
-    DSA_TRY
-    Pcsr& P = which == DSA_COLMAJOR ? A->colmajor : A->rowmajor;
-    P.set_batch_d(which == DSA_COLMAJOR ? A->ws : A->ws2, d_inkeys, d_partkeys, d_vals, n, nullptr, nullptr, A->sh.st);
-    return DSA_OK;
-    DSA_CATCH
-}
-int dsa_matrix_set_batch_two_d(dsa_matrix_t* A, const int64_t* d_rows_c, const int64_t* d_cols_c, const double* d_vals_c, int64_t nc,
-                               const int64_t* d_rows_r, const int64_t* d_cols_r, const double* d_vals_r, int64_t nr) {
-    DSA_TRY
-    if (nc <= 0 && nr <= 0) return DSA_OK;
-    matrix_set_batch_two(A, d_rows_c, d_cols_c, d_vals_c, nc, d_rows_r, d_cols_r, d_vals_r, nr);
-    return DSA_OK;
-    DSA_CATCH
-}
-int dsa_matrix_spmv_dense_range_d(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t key_lo,
-                                  int64_t key_hi) {
-    DSA_TRY
-    cudaStream_t st = A->sh.st;
-    Pcsr& P = trans ? A->colmajor : A->rowmajor;
-    if (key_hi > key_lo) {
-        DSA_CUDA(cudaMemsetAsync(d_y, 0, (size_t)(key_hi - key_lo) * 8, st));
-        P.spmv_dense(A->ws, d_x, nx, d_y, key_lo, key_hi, st);
     }
     return DSA_OK;
     DSA_CATCH

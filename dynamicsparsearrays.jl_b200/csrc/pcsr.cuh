@@ -762,10 +762,6 @@ struct Pcsr {
     void build_coo_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals, int64_t n, int combine,
                      cudaStream_t st);
 
-    // batched setindex! (pcsr.jl:341-347 per op): see DESIGN.md §4
-    void set_batch_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals, int64_t n,
-                     int64_t* max_part_nz, int64_t* max_key_nz, cudaStream_t st);
-
     void get_batch_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, int64_t n, double* d_out, cudaStream_t st) {
         if (n <= 0) return;
         int32_t* op_slot = ws.op_slot.ensure((size_t)n);
@@ -805,7 +801,7 @@ struct Pcsr {
         DSA_LAUNCH("span_purge", k_span_purge, grid_for(nsl * 32, 256), 256, 0, st, pma.keys.p, pma.vals.p, d_slots, nsl, d_sem.p, d_next_slot.p, pma.g.capacity,
                    pma.leafcnt.p, ws.batch.touched, ilog2_i64(pma.g.segment_capacity));
         DSA_LAUNCH("clear_sems", k_clear_sems, grid_for(nsl, 256), 256, 0, st, d_sem.p, d_slots, nsl);
-        pma.rebalance_after(ws.batch, 0, d_sem.p, st);
+        pma.rebalance_after(ws.batch, d_sem.p, st);
         for (int32_t s : slots) slot_live[(size_t)s] = 0;   // pcsr.jl:202,209
         nb_partitions -= nsl;                                // pcsr.jl:191
         rebuild_live_and_upload(st);

@@ -150,11 +150,10 @@ __global__ void __launch_bounds__(256) k_locate(const int64_t* __restrict__ keys
                                                  const int64_t* __restrict__ op_key, const double* __restrict__ op_val, int64_t nops,
                                                  const int64_t* __restrict__ sem, const int32_t* __restrict__ next_slot,
                                                  int64_t* __restrict__ op_pos, uint8_t* __restrict__ op_flag,
-                                                 const int64_t* __restrict__ n_dev, const uint8_t* __restrict__ op_dead,
-                                                 int32_t* __restrict__ ins_flag) {
+                                                 const int64_t* __restrict__ n_dev, int32_t* __restrict__ ins_flag) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nops) return;
-    if (i >= (n_dev ? *n_dev : nops) || (op_dead && op_dead[i])) {   // beyond the unique ops / overwritten by a later op of the batch
+    if (i >= (n_dev ? *n_dev : nops)) {   // beyond the unique ops
         op_flag[i] = 0;
         ins_flag[i] = 0;
         return;
@@ -1058,11 +1057,10 @@ struct PmaCore {
     // The batch tail shared by every mutation: ops are located (op_pos/op_flag), deletes/purges already counted in leafcnt
     // + touched.  Builds the density tree, selects windows, merges/redistributes, resizes when the root fails.
     // d_sem (nullable) = semaphore positions to refresh.  Returns through nnz.
-    void rebalance_after(BatchWorkspace& ws, int64_t nins, int64_t* d_sem, cudaStream_t st) {
+    void rebalance_after(BatchWorkspace& ws, int64_t* d_sem, cudaStream_t st) {
         rebalance_launch(ws, st);
         DSA_CUDA(cudaStreamSynchronize(st));
         rebalance_finish(ws, d_sem, st);
-        (void)nins;
     }
 
     // first half: density tree + window selection + status read-back (enqueued; the caller synchronises the stream)
@@ -1193,14 +1191,14 @@ struct PmaCore {
 
     // sorted unique ops -> located, applied, merged.  op_pid/sem/next_sem nullable (plain PMA).
     void apply_sorted_ops(BatchWorkspace& ws, const int32_t* op_pid, const int64_t* op_key, const double* op_val, int64_t nops,
-                          int64_t* d_sem, const int32_t* d_next_slot, cudaStream_t st, bool scratch_ready = false,
-                          const int64_t* n_dev = nullptr, bool launch_only = false, const uint8_t* op_dead = nullptr) {
-        if (!scratch_ready) prepare_batch_scratch(ws, nops, st);
+                          int64_t* d_sem, const int32_t* d_next_slot, cudaStream_t st, const int64_t* n_dev = nullptr,
+                          bool launch_only = false) {
+        prepare_batch_scratch(ws, nops, st);
         if (nops > 0) {
             const unsigned gr = grid_for(nops, 256);
             int32_t* f32 = ws.flag32.ensure((size_t)nops);
             DSA_LAUNCH("locate", k_locate, gr, 256, 0, st, keys.p, g.capacity, op_pid, op_key, op_val, nops, d_sem, d_next_slot,
-                       ws.op_pos.p, ws.op_flag.p, n_dev, op_dead, f32);
+                       ws.op_pos.p, ws.op_flag.p, n_dev, f32);
             apply_located_ops<true>(ws, op_key, op_val, nops, d_sem, st);
         }
         rebalance_launch(ws, st);

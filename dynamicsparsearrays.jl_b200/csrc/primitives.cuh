@@ -1,117 +1,18 @@
 // libdsa device primitives: exclusive scan, min/max reduction, iota — hand-written, stream-ordered.
 #pragma once
-#include <cstdlib>
 #include "common.cuh"
 
 namespace dsa {
 
 // ---------------------------------------------------------------------------------------------
-// Exclusive prefix sum of int32 (three-phase: tile reduce -> scan of tile sums -> tile scan).
+// Exclusive prefix sum of int32 in one launch (chained scan with decoupled look-back).
 // Tile = 256 threads x 16 items.  out may alias in.
 // ---------------------------------------------------------------------------------------------
 constexpr int SCAN_THREADS = 256;
 constexpr int SCAN_ITEMS = 16;   // 4096 items per tile: the look-back chain of a 1M-item scan is 245 tiles long
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
-template <typename InT>
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_reduce(const InT* __restrict__ in, int64_t n, int32_t* __restrict__ tile_sums) {
-    __shared__ int32_t warp_sums[SCAN_THREADS / 32];
-    const int64_t base = (int64_t)blockIdx.x * SCAN_TILE;
-    int32_t s = 0;
-#pragma unroll
-    for (int i = 0; i < SCAN_ITEMS; ++i) {
-        int64_t idx = base + (int64_t)i * SCAN_THREADS + threadIdx.x;
-        if (idx < n) s += (int32_t)in[idx];
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) warp_sums[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        int32_t t = 0;
-#pragma unroll
-        for (int w = 0; w < SCAN_THREADS / 32; ++w) t += warp_sums[w];
-        tile_sums[blockIdx.x] = t;
-    }
-}
-
-// single block: exclusive scan of the tile sums in place; total -> *total_out (may be null)
-__global__ void __launch_bounds__(1024) k_scan_tile_sums(int32_t* __restrict__ tile_sums, int64_t ntiles, int64_t* __restrict__ total_out) {
-    __shared__ int32_t warp_tot[32];
-    __shared__ int32_t carry_s;
-    if (threadIdx.x == 0) carry_s = 0;
-    __syncthreads();
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int64_t base = 0; base < ntiles; base += 1024) {
-        int64_t idx = base + threadIdx.x;
-        int32_t v = idx < ntiles ? tile_sums[idx] : 0;
-        int32_t incl = v;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            int32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += t;
-        }
-        if (lane == 31) warp_tot[wid] = incl;
-        __syncthreads();
-        if (wid == 0) {
-            int32_t w = warp_tot[lane];
-            int32_t wi = w;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                int32_t t = __shfl_up_sync(0xffffffffu, wi, o);
-                if (lane >= o) wi += t;
-            }
-            warp_tot[lane] = wi - w;   // exclusive warp offsets
-        }
-        __syncthreads();
-        int32_t excl = carry_s + warp_tot[wid] + incl - v;
-        if (idx < ntiles) tile_sums[idx] = excl;
-        __syncthreads();
-        // block total of this chunk = last thread's inclusive value
-        if (threadIdx.x == 1023) carry_s = excl + v;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0 && total_out) *total_out = (int64_t)carry_s;
-}
-
-template <typename InT>
-__global__ void __launch_bounds__(SCAN_THREADS) k_scan_tile_apply(const InT* __restrict__ in, int32_t* __restrict__ out, int64_t n,
-                                                                    const int32_t* __restrict__ tile_offsets) {
-    // blocked arrangement inside the tile so each thread scans SCAN_ITEMS consecutive items
-    __shared__ int32_t warp_tot[SCAN_THREADS / 32];
-    const int64_t base = (int64_t)blockIdx.x * SCAN_TILE + (int64_t)threadIdx.x * SCAN_ITEMS;
-    int32_t v[SCAN_ITEMS];
-    int32_t s = 0;
-#pragma unroll
-    for (int i = 0; i < SCAN_ITEMS; ++i) {
-        int64_t idx = base + i;
-        v[i] = idx < n ? (int32_t)in[idx] : 0;
-        s += v[i];
-    }
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int32_t incl = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        int32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += t;
-    }
-    if (lane == 31) warp_tot[wid] = incl;
-    __syncthreads();
-    int32_t woff = 0;
-#pragma unroll
-    for (int w = 0; w < SCAN_THREADS / 32; ++w)
-        if (w < wid) woff += warp_tot[w];
-    int32_t run = tile_offsets[blockIdx.x] + woff + incl - s;
-#pragma unroll
-    for (int i = 0; i < SCAN_ITEMS; ++i) {
-        int64_t idx = base + i;
-        if (idx < n) out[idx] = run;
-        run += v[i];
-    }
-}
-
-// Default since round 1 (DSA_SCAN_ONEPASS=0 selects the three-phase version above): the same scan in ONE launch — chained scan
-// with decoupled look-back (parity suite green and layouts bit-identical with either version, profiles/exp_r01_update_switches.log).  Tiles are handed out by an atomic ticket (so a tile's predecessors have always started: forward progress), every
+// Tiles are handed out by an atomic ticket (so a tile's predecessors have always started: forward progress), every
 // tile publishes one 64-bit word {epoch:30 | flag:2 | sum:32} (aggregate first, inclusive prefix once known); a tile adds up its
 // predecessors' words back to the nearest inclusive one.  The epoch makes stale words of earlier calls invisible, so the state
 // array needs no clearing between calls; the tile that draws the last ticket resets the ticket counter.
@@ -202,18 +103,10 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_onepass(const InT* __rest
 }
 
 struct ScanWorkspace {
-    DBuf<int32_t> tile_sums;
-    DBuf<unsigned long long> state;   // one-pass variant: tile words + (last element) the ticket counter
+    DBuf<unsigned long long> state;   // tile words + (last element) the ticket counter
     size_t state_cap = 0;
     uint32_t epoch = 0;
 };
-inline bool scan_onepass_enabled() {
-    static const bool on = [] {
-        const char* e = getenv("DSA_SCAN_ONEPASS");
-        return !e || atoi(e) != 0;
-    }();
-    return on;
-}
 
 // out[i] = sum_{j<i} in[j]; *d_total (device int64, may be null) = sum of all
 template <typename InT>
@@ -223,23 +116,16 @@ inline void exclusive_scan_i32(ScanWorkspace& ws, const InT* d_in, int32_t* d_ou
         return;
     }
     const int64_t ntiles = (n + SCAN_TILE - 1) / SCAN_TILE;
-    if (scan_onepass_enabled()) {
-        ws.state.ensure((size_t)ntiles + 1);
-        if (ws.state.cap != ws.state_cap || ws.epoch >= (1u << 30) - 1) {   // new block (or epoch wrap): clear words + ticket once
-            DSA_CUDA(cudaMemsetAsync(ws.state.p, 0, ws.state.cap * sizeof(unsigned long long), st));
-            ws.state_cap = ws.state.cap;
-            ws.epoch = 0;
-        }
-        ws.epoch += 1;
-        uint32_t* ticket = reinterpret_cast<uint32_t*>(ws.state.p + (ws.state.cap - 1));
-        DSA_LAUNCH("scan_onepass", (k_scan_onepass<InT>), (unsigned)ntiles, SCAN_THREADS, 0, st, d_in, d_out, n, ntiles, ws.state.p, ticket,
-                   ws.epoch, d_total);
-        return;
+    ws.state.ensure((size_t)ntiles + 1);
+    if (ws.state.cap != ws.state_cap || ws.epoch >= (1u << 30) - 1) {   // new block (or epoch wrap): clear words + ticket once
+        DSA_CUDA(cudaMemsetAsync(ws.state.p, 0, ws.state.cap * sizeof(unsigned long long), st));
+        ws.state_cap = ws.state.cap;
+        ws.epoch = 0;
     }
-    int32_t* sums = ws.tile_sums.ensure((size_t)ntiles);
-    DSA_LAUNCH("scan_tile_reduce", (k_scan_tile_reduce<InT>), (unsigned)ntiles, SCAN_THREADS, 0, st, d_in, n, sums);
-    DSA_LAUNCH("scan_tile_sums", k_scan_tile_sums, 1, 1024, 0, st, sums, ntiles, d_total);
-    DSA_LAUNCH("scan_tile_apply", (k_scan_tile_apply<InT>), (unsigned)ntiles, SCAN_THREADS, 0, st, d_in, d_out, n, sums);
+    ws.epoch += 1;
+    uint32_t* ticket = reinterpret_cast<uint32_t*>(ws.state.p + (ws.state.cap - 1));
+    DSA_LAUNCH("scan_onepass", (k_scan_onepass<InT>), (unsigned)ntiles, SCAN_THREADS, 0, st, d_in, d_out, n, ntiles, ws.state.p, ticket,
+               ws.epoch, d_total);
 }
 
 // ---------------------------------------------------------------------------------------------

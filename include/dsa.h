@@ -139,22 +139,6 @@ int dsa_matrix_info(const dsa_matrix_t* A, int which, int64_t* out10);
 int dsa_matrix_export(dsa_matrix_t* A, int which, uint8_t* occupied, int64_t* keys, double* vals, int64_t* semaphores,
                       int64_t* col_keys, uint8_t* col_live);
 
-/* ---------------------------------------------------------------- sharded use (one orientation at a time) ---- */
-/* A rank of a column-range-sharded matrix owns the col-major structure of ITS columns and the row-major structure of ITS rows
- * (SURVEY.md §8e), so the two orientations of its handle receive different op sets.  in-array keys / partition keys are
- * (rows, cols) for DSA_COLMAJOR and (cols, rows) for DSA_ROWMAJOR. */
-int dsa_matrix_build_one(dsa_matrix_t* A, int which, const int64_t* inkeys, const int64_t* partkeys, const double* vals, int64_t n,
-                         int combine);
-int dsa_matrix_set_batch_one_d(dsa_matrix_t* A, int which, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals,
-                               int64_t n);
-/* both orientations in one call (they share the two host synchronisations of a batch): the col-major structure receives
- * (rows_c, cols_c, vals_c), the row-major one (rows_r, cols_r, vals_r) */
-int dsa_matrix_set_batch_two_d(dsa_matrix_t* A, const int64_t* d_rows_c, const int64_t* d_cols_c, const double* d_vals_c, int64_t nc,
-                               const int64_t* d_rows_r, const int64_t* d_cols_r, const double* d_vals_r, int64_t nr);
-/* y[k - key_lo] = (row-major if trans == 0, else col-major) partition k times x, for key_lo <= k < key_hi; other entries 0 */
-int dsa_matrix_spmv_dense_range_d(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t key_lo,
-                                  int64_t key_hi);
-
 /* ---------------------------------------------------------------- multi-GPU (SURVEY.md §8e) ---- */
 /* One process per GPU.  A dsa_dist_t is this rank's seat in a group of `world` ranks on one NVLink box; a dsa_dmatrix_t is a
  * DynamicSparseMatrix sharded by key range over the group: rank r owns the column-major PCSR of the columns in
