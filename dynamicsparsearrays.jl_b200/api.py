@@ -21,6 +21,7 @@ same names, same argument meaning, same error behaviour; the structures themselv
 """
 import ctypes as C
 import os
+import sys
 
 import numpy as np
 
@@ -661,13 +662,53 @@ class DynamicSparseMatrix:
         return self._mul(x, trans=False, n=self._dims()[0])
 
     def mul_dense(self, x, trans=False):
-        """Dense-x product: x[j-1] for every j in 1..len(x); returns dense y of length size[0] (or size[1] if trans)."""
+        """Dense-x product: x[j-1] for every j in 1..len(x); returns dense y of length size[0] (or size[1] if trans).
+        A 2-D x of shape (nx, k) holds k right-hand sides, multiplied in one pass over the matrix per 32 columns: the result
+        is (ny, k), and its column c equals mul_dense(x[:, c]) bit for bit.  A torch CUDA tensor (1-D or 2-D) stays on the
+        device: the product runs after the work already queued on torch's current stream, and the float64 result tensor is
+        ready on that stream."""
         self._not_fillmode("Matrix is in fill mode")
         self.flush()
+        torch = sys.modules.get("torch")
+        if torch is not None and isinstance(x, torch.Tensor) and x.is_cuda:
+            return self._mul_dense_cuda(torch, x, trans)
         x = _f64(x)
+        if x.ndim > 2:
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, f"mul_dense takes a vector or an (nx, k) matrix, not a {x.ndim}-D array")
         ny = self._dims()[1] if trans else self._dims()[0]
+        if x.ndim == 2:
+            nx, k = x.shape
+            y = np.zeros((max(ny, 1), k), np.float64)
+            check(lib().dsa_matrix_spmm_dense(self._h, C.c_int(1 if trans else 0), _p(x), C.c_int64(nx), C.c_int64(k), C.c_int64(k),
+                                              _p(y), C.c_int64(ny), C.c_int64(k)))
+            return y[:ny]
         y = np.zeros(max(ny, 1), np.float64)
         check(lib().dsa_matrix_spmv_dense(self._h, C.c_int(1 if trans else 0), _p(x), C.c_int64(len(x)), _p(y), C.c_int64(ny)))
+        return y[:ny]
+
+    def _mul_dense_cuda(self, torch, x, trans):
+        if x.dim() not in (1, 2):
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, f"mul_dense takes a vector or an (nx, k) matrix, not a {x.dim()}-D tensor")
+        ny = self._dims()[1] if trans else self._dims()[0]
+        x = x.to(torch.float64)
+        if x.dim() == 1 or x.stride(1) != 1 or x.stride(0) < x.shape[1]:   # a row-major view (any row stride) is read in place
+            x = x.contiguous()
+        y = torch.empty((max(ny, 1),) + tuple(x.shape[1:]), dtype=torch.float64, device=x.device)
+        st = C.c_void_p()
+        check(lib().dsa_matrix_get_stream(self._h, C.byref(st)))
+        # the handle keeps its own stream (its priority orders the update pipeline): order it against torch's both ways
+        cur = torch.cuda.current_stream(x.device)
+        hs = torch.cuda.ExternalStream(st.value or 0, device=x.device)
+        hs.wait_stream(cur)
+        t = C.c_int(1 if trans else 0)
+        xp, yp = C.c_void_p(x.data_ptr()), C.c_void_p(y.data_ptr())
+        if x.dim() == 1:
+            check(lib().dsa_matrix_spmv_dense_d(self._h, t, xp, C.c_int64(x.shape[0]), yp, C.c_int64(ny)))
+        else:
+            nx, k = x.shape
+            check(lib().dsa_matrix_spmm_dense_d(self._h, t, xp, C.c_int64(nx), C.c_int64(k), C.c_int64(x.stride(0)), yp, C.c_int64(ny),
+                                                C.c_int64(k)))
+        cur.wait_stream(hs)
         return y[:ny]
 
 

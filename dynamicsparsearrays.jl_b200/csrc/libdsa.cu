@@ -1059,6 +1059,71 @@ int dsa_matrix_spmv_dense_d(dsa_matrix_t* A, int trans, const double* d_x, int64
     return DSA_OK;
     DSA_CATCH
 }
+// Columns per pass over the matrix: the pass's partials take (slots + chunks) x 8 B per column of workspace
+static constexpr int64_t SPMM_COLS_PER_PASS = 32;
+static void check_spmm_args(int64_t nx, int64_t k, int64_t ldx, int64_t ny, int64_t ldy) {
+    if (nx < 0 || ny < 0 || k < 0 || ldx < k || ldy < k)
+        throw DsaError{DSA_ERR_ARGUMENT, "spmm_dense: need nx >= 0, ny >= 0, k >= 0, ldx >= k and ldy >= k"};
+}
+// X row-major with ld % 4 == 0, 32-byte aligned, every row readable up to column k rounded up to 4
+static void spmm_dense_run(dsa_matrix_t* A, int trans, const double* X, int64_t nx, int64_t k, int64_t ld, double* d_Y, int64_t ny,
+                           int64_t ldy) {
+    cudaStream_t st = A->sh.st;
+    Pcsr& P = trans ? A->colmajor : A->rowmajor;
+    if (ny > 0) DSA_CUDA(cudaMemset2DAsync(d_Y, (size_t)ldy * 8, 0, (size_t)k * 8, (size_t)ny, st));
+    for (int64_t c0 = 0; c0 < k; c0 += SPMM_COLS_PER_PASS)
+        P.spmm_dense_pass(A->ws, nx > 0 ? X + c0 : X, nx, ld, (int)std::min(SPMM_COLS_PER_PASS, k - c0), d_Y + c0, ldy, 1, ny + 1, st);
+}
+static void spmm_dense_dev(dsa_matrix_t* A, int trans, const double* d_X, int64_t nx, int64_t k, int64_t ldx, double* d_Y, int64_t ny,
+                           int64_t ldy) {
+    if (k == 1 && ldx == 1 && ldy == 1) {   // one contiguous vector: the single-vector product itself
+        spmv_dense_dev(A, trans, d_X, nx, d_Y, ny);
+        return;
+    }
+    // a cell reads 4 consecutive entries of its row of X with one 256-bit load: other layouts are re-laid with ld = k rounded up
+    // to 4 (the padding columns are read, their results dropped)
+    if (nx > 0 && (k % 4 != 0 || ldx % 4 != 0 || (uintptr_t)d_X % 32 != 0)) {
+        const int64_t ld = (k + 3) / 4 * 4;
+        double* xp = A->ws.xpad.ensure((size_t)(nx * ld));
+        DSA_CUDA(cudaMemcpy2DAsync(xp, (size_t)ld * 8, d_X, (size_t)ldx * 8, (size_t)k * 8, (size_t)nx, cudaMemcpyDeviceToDevice,
+                                   A->sh.st));
+        spmm_dense_run(A, trans, xp, nx, k, ld, d_Y, ny, ldy);
+    } else {
+        spmm_dense_run(A, trans, d_X, nx, k, ldx, d_Y, ny, ldy);
+    }
+}
+int dsa_matrix_spmm_dense(dsa_matrix_t* A, int trans, const double* X, int64_t nx, int64_t k, int64_t ldx, double* Y, int64_t ny,
+                          int64_t ldy) {
+    DSA_TRY
+    check_spmm_args(nx, k, ldx, ny, ldy);
+    if (k == 0) return DSA_OK;
+    cudaStream_t st = A->sh.st;
+    // staged in the layout the kernel reads in place: ld = k rounded up to 4 (a single column stays a contiguous vector)
+    const int64_t lds = k == 1 ? 1 : (k + 3) / 4 * 4;
+    double* dx = A->stg.v.ensure((size_t)std::max<int64_t>(nx * lds, 1));
+    if (nx > 0)
+        DSA_CUDA(cudaMemcpy2DAsync(dx, (size_t)lds * 8, X, (size_t)ldx * 8, (size_t)k * 8, (size_t)nx, cudaMemcpyHostToDevice, st));
+    double* dy = A->stg.out.ensure((size_t)std::max<int64_t>(ny * k, 1));
+    if (k == 1) spmv_dense_dev(A, trans, dx, nx, dy, ny);
+    else spmm_dense_run(A, trans, dx, nx, k, lds, dy, ny, k);
+    if (ny > 0)
+        DSA_CUDA(cudaMemcpy2DAsync(Y, (size_t)ldy * 8, dy, (size_t)k * 8, (size_t)k * 8, (size_t)ny, cudaMemcpyDeviceToHost, st));
+    DSA_CUDA(cudaStreamSynchronize(st));
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_spmm_dense_d(dsa_matrix_t* A, int trans, const double* d_X, int64_t nx, int64_t k, int64_t ldx, double* d_Y, int64_t ny,
+                            int64_t ldy) {
+    DSA_TRY
+    check_spmm_args(nx, k, ldx, ny, ldy);
+    if (k > 0) spmm_dense_dev(A, trans, d_X, nx, k, ldx, d_Y, ny, ldy);
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_get_stream(const dsa_matrix_t* A, void** cuda_stream_out) {
+    *cuda_stream_out = (void*)A->sh.st;
+    return DSA_OK;
+}
 int dsa_matrix_info(const dsa_matrix_t* A, int which, int64_t* out10) {
     const Pcsr& P = which == DSA_COLMAJOR ? A->colmajor : A->rowmajor;
     out10[0] = P.pma.g.capacity; out10[1] = P.pma.g.segment_capacity; out10[2] = P.pma.g.nb_segments; out10[3] = P.pma.nnz;

@@ -602,6 +602,158 @@ __global__ void __launch_bounds__(256) k_spmv_fix_to_dense(const double* __restr
     y[k - key_lo] = a;
 }
 
+// ---------------------------------------------------------------------------------------------
+// K7b multi-vector product Y = A * X over the gapped array, for one pass of 4 * ngroups columns of a row-major X (row stride
+// ldx % 4 == 0, 32-byte aligned base).  Bit for bit, column c is k_spmv_blocked<0, C> + k_spmv_fix_to_dense on column c alone:
+// the same 32 * C-cell chunk per warp, the same C contiguous cells per lane summed sequentially, the same segmented scan over
+// the lane aggregates (same shuffle order), the same carries added in chunk order by the epilogue, mul and add rounded
+// separately.  What is shared: the keys / values are streamed once for all columns, and a cell's x becomes one 256-bit load of
+// 4 consecutive entries of its row of X per column group instead of one 8-byte gather per vector.  Column groups run one after
+// the other inside the warp, so the registers a group needs do not grow with the pass width.
+// Partials: yslot[slot * W + col], carry[chunk * W + col] with W = 4 * ngroups; chunk_last_slot as in k_spmv_blocked.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ void ldg_x4(const double* p, double& a, double& b, double& c, double& d) {
+    asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(a), "=d"(b), "=d"(c), "=d"(d) : "l"(p));
+}
+
+template <int C>
+__global__ void __launch_bounds__(256) k_spmm_blocked(const int64_t* __restrict__ keys, const double* __restrict__ vals, int64_t cap,
+                                                       const double* __restrict__ X, int64_t nx, int64_t ldx, int ngroups,
+                                                       double* __restrict__ yslot, double* __restrict__ carry,
+                                                       int32_t* __restrict__ chunk_last_slot, int64_t nchunks) {
+    static_assert(C % 4 == 0, "a lane loads its cells in groups of 4 (256 bits)");
+    const int64_t chunk = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (chunk >= nchunks) return;
+    const unsigned lt = lanemask_lt();
+    const uint64_t l2pol = l2_evict_first_policy();
+    const int64_t p0 = chunk * (32 * C) + (int64_t)lane * C;
+    int64_t k[C];
+    double t[C];
+#pragma unroll
+    for (int c = 0; c < C; c += 4) {
+        if (p0 + c + 4 <= cap) {
+            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], l2pol);
+            ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], l2pol);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const int64_t p = p0 + c + e;
+                k[c + e] = p < cap ? keys[p] : GAP_KEY;
+                t[c + e] = p < cap ? vals[p] : 0.0;
+            }
+        }
+    }
+    // the segment structure of the chunk is the same for every column
+    bool has_head = false;
+    int32_t lastslot = -1;
+#pragma unroll
+    for (int c = 0; c < C; ++c)
+        if (k[c] == 0) {
+            has_head = true;
+            lastslot = (int32_t)t[c] - 1;
+        }
+    const unsigned hb = __ballot_sync(0xffffffffu, has_head);
+    const unsigned hle = hb & (lt | (1u << lane));
+    const int seg_lo = hle ? 31 - __clz(hle) : 0;
+    const unsigned hlt = hb & lt;
+    const int32_t prev_slot = __shfl_sync(0xffffffffu, lastslot, hlt ? 31 - __clz(hlt) : 0);
+    const int32_t end_slot = __shfl_sync(0xffffffffu, lastslot, hb ? 31 - __clz(hb) : 0);
+    if (lane == 31) chunk_last_slot[chunk] = hb ? end_slot : -1;
+    const int64_t W = 4 * (int64_t)ngroups;
+#pragma unroll 1
+    for (int g = 0; g < ngroups; ++g) {
+        // the C row loads of x: independent, branch-free, all in flight together (gap / head lanes read row 0)
+        double xv[C][4];
+#pragma unroll
+        for (int c = 0; c < C; ++c)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) xv[c][j] = 0.0;
+        if (nx > 0) {   // warp-uniform
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const int64_t kk = k[c];
+                const int64_t idx = (kk > 0 && kk <= nx) ? kk - 1 : 0;
+                ldg_x4(X + idx * ldx + 4 * g, xv[c][0], xv[c][1], xv[c][2], xv[c][3]);
+            }
+        }
+        // sequential reduction of the lane's cells, per column
+        double run[4] = {0.0, 0.0, 0.0, 0.0}, pre[4] = {0.0, 0.0, 0.0, 0.0};
+        bool seen = false;
+        int32_t open = -1;
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            const int64_t kk = k[c];
+            if (kk == 0) {
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (!seen) pre[j] = run[j];
+                    else yslot[open * W + 4 * g + j] = run[j];   // a whole partition inside this lane
+                    run[j] = 0.0;
+                }
+                seen = true;
+                open = (int32_t)t[c] - 1;
+            } else if (kk > 0) {
+                const bool present = kk <= nx;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) run[j] = __dadd_rn(run[j], present ? __dmul_rn(xv[c][j], t[c]) : 0.0);
+            }
+        }
+        // segmented inclusive scan over the lanes, per column
+        double inc[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) inc[j] = run[j];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const double u = __shfl_up_sync(0xffffffffu, inc[j], o);
+                if (lane >= o && lane - o >= seg_lo) inc[j] = __dadd_rn(u, inc[j]);
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            double cin = __shfl_up_sync(0xffffffffu, inc[j], 1);
+            if (lane == 0) cin = 0.0;
+            const int64_t col = 4 * g + j;
+            if (has_head) {   // this lane's first head closes the partition that was open before it
+                const double tot = __dadd_rn(cin, pre[j]);
+                if (hlt) yslot[prev_slot * W + col] = tot;
+                else carry[chunk * W + col] = tot;   // it started in an earlier chunk: the epilogue adds this prefix
+            }
+            if (lane == 31) {
+                if (hb) yslot[end_slot * W + col] = inc[j];   // open partition at the end of the chunk: completed by the epilogue
+                else carry[chunk * W + col] = inc[j];         // no head in the whole chunk
+            }
+        }
+    }
+}
+
+// k_spmv_fix_to_dense per column: thread (slot, col) of one pass; Y[(key - key_lo) * ldy + col] for col < ncols
+__global__ void __launch_bounds__(256) k_spmm_fix_to_dense(const double* __restrict__ yslot, const double* __restrict__ carry,
+                                                            const int32_t* __restrict__ chunk_last_slot, const int64_t* __restrict__ sem,
+                                                            const int32_t* __restrict__ next_slot, const int64_t* __restrict__ slot_key,
+                                                            int64_t nslots, int64_t cap, int64_t nchunks, int lg_chunk, int W, int ncols,
+                                                            double* __restrict__ Y, int64_t ldy, int64_t key_lo, int64_t key_hi) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t s = i / W;
+    const int col = (int)(i - s * W);
+    if (s >= nslots || col >= ncols) return;
+    const int64_t ps = sem[s];
+    if (ps < 0) return;
+    const int64_t k = slot_key[s];
+    if (k < key_lo || k >= key_hi) return;
+    double a = yslot[s * W + col];
+    const int64_t c0 = ps >> lg_chunk;
+    if (span_end(sem, next_slot, (int32_t)s, cap) >= ((c0 + 1) << lg_chunk)) {
+        for (int64_t d = c0 + 1; d < nchunks; ++d) {
+            a = __dadd_rn(a, carry[d * W + col]);
+            if (chunk_last_slot[d] >= 0) break;
+        }
+    }
+    Y[(k - key_lo) * ldy + col] = a;
+}
+
 // touched partitions (at least one product) for the sparse output (operations.jl:11-12, sparsevec(::Dict, n))
 __global__ void __launch_bounds__(256) k_flag_touched(const int32_t* __restrict__ ycnt, const int64_t* __restrict__ sem, int64_t nslots,
                                                        int32_t* __restrict__ flag) {
@@ -664,6 +816,7 @@ struct PcsrWorkspace {
     DBuf<TileRec> trec;          // tile buckets of a tile-streamed batch: TILE_CAP records per tile
     DBuf<int64_t> miss_keys, cs, u_key, live_pos, nuniq, tmp_k, tmp_owner, del_keys;
     DBuf<double> u_val, tmp_v, yslot, carry, xdense;
+    DBuf<double> yslot_mv, carry_mv, xpad;   // multi-vector product: partials of a pass (W per slot / chunk), X re-laid to ld % 4 == 0
     DBuf<uint64_t> sk;
     DBuf<uint32_t> perm;
     DBuf<uint8_t> xmask;
@@ -852,6 +1005,26 @@ struct Pcsr {
         if (ns > 0)
             DSA_LAUNCH("spmv_fix_to_dense", k_spmv_fix_to_dense, grid_for(ns, 256), 256, 0, st, ws.yslot.p, ws.carry.p, ws.chunk_last.p, d_sem.p,
                        d_next_slot.p, d_slot_key.p, ns, cap, nchunks, SPMV_LG_CHUNK, d_y, key_lo, key_hi);
+    }
+
+    // mat * X -> Y for one pass of ncols (<= 4 * ngroups) columns, over the partition keys [key_lo, key_hi) (Y zeroed by the
+    // caller; columns >= ncols of Y untouched): X row-major, ldx % 4 == 0, 32-byte aligned; columns ncols .. W-1 of X are read
+    // and their results dropped
+    void spmm_dense_pass(PcsrWorkspace& ws, const double* d_X, int64_t nx, int64_t ldx, int ncols, double* d_Y, int64_t ldy,
+                         int64_t key_lo, int64_t key_hi, cudaStream_t st) {
+        constexpr int C = SPMV_CELLS_PER_LANE;
+        const int ngroups = (ncols + 3) / 4, W = 4 * ngroups;
+        const int64_t cap = pma.g.capacity, ns = nslots();
+        const int64_t nchunks = (cap + (1 << SPMV_LG_CHUNK) - 1) >> SPMV_LG_CHUNK;
+        static_assert(32 * C == 1 << SPMV_LG_CHUNK, "a warp's chunk");
+        double* yslot = ws.yslot_mv.ensure((size_t)(ns + 1) * W);
+        double* carry = ws.carry_mv.ensure((size_t)nchunks * W);
+        int32_t* clast = ws.chunk_last.ensure((size_t)nchunks);
+        DSA_LAUNCH("spmm_blocked", k_spmm_blocked<C>, grid_for(nchunks * 32, 256), 256, 0, st, pma.keys.p, pma.vals.p, cap, d_X, nx, ldx,
+                   ngroups, yslot, carry, clast, nchunks);
+        if (ns > 0)
+            DSA_LAUNCH("spmm_fix_to_dense", k_spmm_fix_to_dense, grid_for(ns * W, 256), 256, 0, st, yslot, carry, clast, d_sem.p,
+                       d_next_slot.p, d_slot_key.p, ns, cap, nchunks, SPMV_LG_CHUNK, W, ncols, d_Y, ldy, key_lo, key_hi);
     }
 
     void clone_from(const Pcsr& o, cudaStream_t st) {

@@ -132,6 +132,17 @@ int dsa_matrix_spmv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const dou
 /* dense-x variant: x_j = x[j-1] for j in 1..nx (every entry stored); y[i-1] for i in 1..ny, 0.0 where no entry */
 int dsa_matrix_spmv_dense(dsa_matrix_t* A, int trans, const double* x, int64_t nx, double* y, int64_t ny);
 int dsa_matrix_spmv_dense_d(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t ny);
+/* mat * X (trans = 0) / transpose(mat) * X (trans = 1) for a dense row-major X (nx rows, k columns, row stride ldx >= k):
+ * Y[i-1, c] for i in 1..ny, c < k (row stride ldy >= k), 0.0 where no entry; columns k..ldy-1 of Y are not written.
+ * Column c equals dsa_matrix_spmv_dense of column c bit for bit.  k == 0: nothing is written.  nx, ny or k < 0, ldx < k or
+ * ldy < k: DSA_ERR_ARGUMENT, nothing is launched.  One pass over the matrix carries up to 32 columns; X is read in place when
+ * ldx and k are multiples of 4 and X is 32-byte aligned, otherwise re-laid on the device first. */
+int dsa_matrix_spmm_dense(dsa_matrix_t* A, int trans, const double* X, int64_t nx, int64_t k, int64_t ldx, double* Y, int64_t ny,
+                          int64_t ldy);
+int dsa_matrix_spmm_dense_d(dsa_matrix_t* A, int trans, const double* d_X, int64_t nx, int64_t k, int64_t ldx, double* d_Y,
+                            int64_t ny, int64_t ldy);
+/* the CUDA stream the handle's work is enqueued on (so that a caller can order its own streams against it) */
+int dsa_matrix_get_stream(const dsa_matrix_t* A, void** cuda_stream_out);
 /* which = DSA_COLMAJOR | DSA_ROWMAJOR; out = {capacity, segment_capacity, nb_segments, nb_elements, height, nb_partitions,
  * len(semaphores), m, n, nnz} (pma.jl:8-24, pcsr.jl:4-21, matrix.jl:1-8,91) */
 int dsa_matrix_info(const dsa_matrix_t* A, int which, int64_t* out10);

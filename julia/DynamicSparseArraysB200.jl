@@ -307,6 +307,23 @@ Base.:(*)(t::Transposed, v::VecLike) = _mul(t.array, true, _xs(v)..., size(t.arr
 Base.:(*)(v::VecLike, t::Transposed) = _mul(t.array, false, _xs(v)..., size(t.array, 1))                  # operations.jl:38-48
 Base.:(*)(v::VecLike, A::DynamicSparseMatrix) = _mul(A, true, _xs(v)..., size(A, 2))                      # operations.jl:50-60
 
+# k dense right-hand sides in one call (one pass over the matrix per 32 columns); column c of the result equals the product
+# with X[:, c] bit for bit.  The library takes row-major buffers: permutedims turns the column-major X into one (ldx = k).
+function _mul_dense(A::DynamicSparseMatrix, trans::Bool, X::Matrix{Float64})
+    A.fillmode && error("Matrix is in fill mode")
+    flush!(A)
+    nx, k = size(X)
+    ny = size(A, trans ? 2 : 1)
+    Xr = permutedims(X)
+    Yr = Matrix{Float64}(undef, k, ny)
+    _check(ccall((:dsa_matrix_spmm_dense, libdsa), Cint,
+                 (Ptr{Cvoid}, Cint, Ptr{Float64}, Int64, Int64, Int64, Ptr{Float64}, Int64, Int64),
+                 A.h, trans ? 1 : 0, Xr, nx, k, k, Yr, ny, k))
+    return permutedims(Yr)
+end
+Base.:(*)(A::DynamicSparseMatrix, X::Matrix{Float64}) = _mul_dense(A, false, X)                           # size (size(A, 1), k)
+Base.:(*)(t::Transposed, X::Matrix{Float64}) = _mul_dense(t.array, true, X)                               # size (size(A, 2), k)
+
 
 # ------------------------------------------------------------------------------------------ multi-GPU (include/dsa.h "multi-GPU")
 # One Julia process per GPU (e.g. under MPI.jl or Distributed).  A ShardedDynamicSparseMatrix is the same DynamicSparseMatrix
