@@ -13,10 +13,10 @@
 //                   (the result of find — hit or predecessor — by a leaf-first search), hits overwrite their value in place or
 //                   set their leaf's delete bit (last writer wins by arrival), misses with a value are the leaf's inserts, and
 //                   every leaf whose post-batch count stays inside its own density bounds (pma.jl:119-123 with h = 0) is re-laid
-//                   at its spread! positions on the spot (pack! + spread!, moves.jl:94-172): one thread per leaf writes down what
-//                   lands in each cell, one thread per cell fetches and stores it.  Leaves that fail their bounds hand their
-//                   inserts, in order, to the density tree / window kernels of pma.cuh, exactly as the random-access pipeline
-//                   does.  Only modified leaves are written back.
+//                   at its spread! positions on the spot (pack! + spread!, moves.jl:94-172): these leaves are shared out
+//                   over all warps, one lane per cell, and each lane fetches and stores what lands in its own cell.  Leaves
+//                   that fail their bounds hand their inserts, in order, to the density tree / window kernels of pma.cuh,
+//                   exactly as the random-access pipeline does.  Only modified leaves are written back.
 //
 // The result is the batch policy's layout (DESIGN.md §4), bit for bit: a leaf accepted at its own level and later covered by a
 // larger window is simply re-laid twice (the window kernel reads the merged leaf with no pending inserts).
@@ -206,10 +206,11 @@ struct TileSmem {
             uint32_t rarr[TILE_CAP];
             int32_t rslot[TILE_CAP];
         } op;
-        struct {                      // phases D2, E: what lands in each cell of a re-laid leaf; S + 1 entries per leaf
-            uint16_t code[TILE_CELLS + TILE_MAX_LEAVES];
-            uint8_t leaf[TILE_MAX_LEAVES];
-        } work;
+        struct {                      // phases D, R: the leaves re-laid here, and the survivors of each by number
+            uint2 leaf[TILE_MAX_LEAVES];   // {survivor mask, spread! mask}, nrelay entries
+            uint8_t lid[TILE_MAX_LEAVES];  // ... and the leaf
+            uint8_t sidx[TILE_CELLS];      // sidx[leaf cell 0 + i] = the leaf cell of survivor number i
+        } lay;
     } u;
     // per leaf
     uint32_t live[TILE_MAX_LEAVES];   // cells stored before the batch
@@ -223,7 +224,7 @@ struct TileSmem {
     int16_t rnext[TILE_CAP];          // next op of the same leaf (-1 = end)
     uint8_t rstat[TILE_CAP];          // 1 = live insert
     uint8_t rop[TILE_CELLS];          // per re-laid leaf: rop[leaf cell 0 + R] = the op that takes merged rank R
-    int nwork;                        // re-laid leaves so far
+    int nrelay;                       // leaves re-laid here (entries of u.lay.leaf)
 };
 
 struct TileArgs {
@@ -256,11 +257,11 @@ __device__ __forceinline__ int tile_insert_rank(const TileSmem& s, int head, int
 }
 
 // Control flow is data-parallel and kept short (the kernel is bound by instruction issue, not by HBM): op phases run one thread
-// per op and only ever walk the list of the ops of the op's own leaf (one or two entries on a uniform batch); one thread per
-// modified leaf writes down, cell by cell, what lands where (a work list); the cells of the work list are then fetched and stored
-// by one thread each.  Only the keys are staged (the searches read them); values are touched where something changes: an
-// overwrite stores its value in place, a re-laid leaf is written destination-driven (the r-th survivor, an insert, or a gap per
-// cell), so every cell has exactly one writer and a re-laid leaf goes back as full lines.
+// per op and only ever walk the list of the ops of the op's own leaf (one or two entries on a uniform batch); the re-laid
+// leaves are then shared out over all warps with one lane per cell, and each lane works out what lands in its own cell.
+// Only the keys are staged (the searches read them); values are touched where something changes: an overwrite stores its value
+// in place, a re-laid leaf is written destination-driven (the r-th survivor, an insert, or a gap per cell), so every cell has
+// exactly one writer and a re-laid leaf goes back as full lines.
 template <int LGS>
 __global__ void __launch_bounds__(TILE_THREADS, TILE_CTAS_PER_SM) k_tile_merge(TileArgs A, Levels L) {
     extern __shared__ __align__(16) unsigned char tile_smem_raw[];
@@ -310,7 +311,7 @@ __global__ void __launch_bounds__(TILE_THREADS, TILE_CTAS_PER_SM) k_tile_merge(T
             s.nins[l] = 0;
             s.lhead[l] = -1;
         }
-        if (tid == 0) s.nwork = 0;
+        if (tid == 0) s.nrelay = 0;
     }
     __syncthreads();
     {   // live masks: a warp reads a row of 32 cells, the first 32/S lanes store the masks of its leaves
@@ -368,70 +369,42 @@ __global__ void __launch_bounds__(TILE_THREADS, TILE_CTAS_PER_SM) k_tile_merge(T
         uint8_t st = 0;
         if (!dead) {
             if (pp & 0x8000) {
-                if (v != 0.0) A.vals[tbase + pos] = v;   // in place; a re-laid leaf reads it back from there in phase E
+                if (v != 0.0) A.vals[tbase + pos] = v;   // in place; a re-laid leaf reads it back from there in phase R
                 else atomicOr(&s.del[l], 1u << (pos & (S - 1)));
             } else if (v != 0.0) {
                 st = 1;
                 atomicAdd(&s.nins[l], 1);
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(A.vals + tbase + (l << lgS)));   // phase E reads the leaf's values
+                asm volatile("prefetch.global.L2 [%0];" ::"l"(A.vals + tbase + (l << lgS)));   // phase R reads the leaf's values
             }
         }
         s.rstat[j] = st;
     }
     __syncthreads();
 
-    // ---- D1: inserts of the leaves that are re-laid here (post-batch count inside the leaf's own bounds, pma.jl:119-123 with
-    //          h = 0): merged rank = survivors up to the predecessor cell + inserts ordered before ----------------------------
-    for (int j = tid; j < nrec; j += TILE_THREADS) {
-        if (!s.rstat[j]) continue;
-        const int pp = s.rpos[j] & 0x7fff, l = pp >> lgS;
-        const unsigned surv = s.live[l] & ~s.del[l];
-        const int m = __popc(surv) + s.nins[l];
-        if (m < mn0 || m > mx0) continue;
-        const int R = __popc(surv & mask_le(pp & (S - 1))) + tile_insert_rank(s, s.lhead[l], pp, s.rkey[j]);
-        s.rop[(l << lgS) + R] = (uint8_t)j;
-        atomicOr(&s.insm[l], 1u << R);
-    }
-    __syncthreads();
-
-    // ---- D2: one thread per modified leaf.  Re-laid leaf (pack! + spread!, moves.jl:94-172): cell q is occupied iff the
-    //          spread! mask of m elements says so; rank r is an insert's or the next survivor's.  A leaf outside its bounds hands
-    //          its inserts, in order, to the density tree / window kernels; blanked cells are stored at once. -----------------
-    constexpr uint32_t CODE_GAP = 0xffffu, CODE_OP = 0x8000u;
-    for (int l = tid; l < NL; l += TILE_THREADS) {
+    // ---- D: one thread per leaf.  A modified leaf (inserts or deletes) is re-laid here if it has inserts and its post-batch
+    //         count m stays inside its own bounds (pma.jl:119-123 with h = 0): it goes on the list of phase R with its
+    //         survivors and its spread! mask.  Any other modified leaf is finished here: its deleted cells are blanked, and if
+    //         it has inserts they are handed, in order, to the density tree / window kernels. --------------------------------
+    for (int l = tid; l < NL; l += TILE_THREADS) {   // NL is a multiple of 32: whole warps
         const int ni = s.nins[l];
-        const unsigned dl = s.del[l];
-        if (ni == 0 && dl == 0) continue;
-        unsigned surv = s.live[l] & ~dl;
-        const int cnt = __popc(surv);
-        const int m = cnt + ni;
+        const unsigned dl = s.del[l], surv = s.live[l] & ~dl;
+        const int cnt = __popc(surv), m = cnt + ni;
         const bool relay = ni > 0 && m >= mn0 && m <= mx0;
+        const unsigned b = __ballot_sync(FULL, relay);
+        int base = 0;
+        if (lane == 0 && b) base = atomicAdd(&s.nrelay, __popc(b));
+        base = __shfl_sync(FULL, base, 0);
+        if (ni == 0 && dl == 0) continue;
         const int64_t lg = (int64_t)t * NL + l;
-        const int lcell = l << lgS;
         A.touched[lg] = 1;
         if (relay) {
             A.leafcnt[lg] = m;
-            const int slot = atomicAdd(&s.nwork, 1);
-            uint16_t* w = s.u.work.code + slot * (S + 1);   // S + 1 entries per leaf: the threads of a warp write different banks
-            s.u.work.leaf[slot] = (uint8_t)l;
-            const unsigned mask = L.leafmask[m], insm = s.insm[l];
-            int r = 0;
-#pragma unroll
-            for (int q = 0; q < S; ++q) {
-                uint32_t code = CODE_GAP;
-                if ((mask >> q) & 1u) {
-                    if ((insm >> r) & 1u) {
-                        code = CODE_OP | s.rop[lcell + r];
-                    } else {
-                        code = (uint32_t)(__ffs(surv) - 1);
-                        surv &= surv - 1;
-                    }
-                    ++r;
-                }
-                w[q] = (uint16_t)code;
-            }
+            const int i = base + __popc(b & ((1u << lane) - 1u));
+            s.u.lay.leaf[i] = make_uint2(surv, L.leafmask[m]);
+            s.u.lay.lid[i] = (uint8_t)l;
             continue;
         }
+        const int lcell = l << lgS;
         if (dl) {
             A.leafcnt[lg] = cnt;
             for (unsigned d = dl; d; d &= d - 1) A.keys[tbase + lcell + (__ffs(d) - 1)] = GAP_KEY;
@@ -451,44 +424,66 @@ __global__ void __launch_bounds__(TILE_THREADS, TILE_CTAS_PER_SM) k_tile_merge(T
             A.ins_first[lg] = (int32_t)gb;
         }
     }
+    //      and the inserts of the leaves re-laid here: merged rank = survivors up to the predecessor cell + inserts ordered before
+    for (int j = tid; j < nrec; j += TILE_THREADS) {
+        if (!s.rstat[j]) continue;
+        const int pp = s.rpos[j] & 0x7fff, l = pp >> lgS;
+        const unsigned surv = s.live[l] & ~s.del[l];
+        const int m = __popc(surv) + s.nins[l];
+        if (m < mn0 || m > mx0) continue;
+        const int R = __popc(surv & mask_le(pp & (S - 1))) + tile_insert_rank(s, s.lhead[l], pp, s.rkey[j]);
+        s.rop[(l << lgS) + R] = (uint8_t)j;
+        atomicOr(&s.insm[l], 1u << R);
+    }
     __syncthreads();
 
-    // ---- E: the cells of the re-laid leaves, one thread each: fetch (survivor values from global memory, all loads of a
-    //         chunk in flight together), then store.  A leaf's cells sit in one warp, in one chunk. ---------------------------
-    const int nwork = s.nwork << lgS;
-    constexpr int EU = 4;
-    for (int w0 = 0; w0 < nwork; w0 += EU * TILE_THREADS) {
-        int64_t k[EU];
-        double v[EU];
-        int cell[EU];
-#pragma unroll
-        for (int u = 0; u < EU; ++u) {
-            const int w = w0 + u * TILE_THREADS + tid;
-            cell[u] = -1;
-            k[u] = GAP_KEY;
-            v[u] = 0.0;
-            if (w < nwork) {
-                const int slot = w >> lgS, q = w & (S - 1);
-                const uint32_t code = s.u.work.code[slot * (S + 1) + q];
-                const int lcell = (int)s.u.work.leaf[slot] << lgS;
-                cell[u] = lcell + q;
-                if (code < 32u) {
-                    k[u] = s.sk[lcell + (int)code];
-                    v[u] = A.vals[tbase + lcell + (int)code];
-                } else if (code != CODE_GAP) {
-                    k[u] = s.rkey[code & 0xffu];
-                    v[u] = s.rval[code & 0xffu];
+    // ---- R: the re-laid leaves (pack! + spread!, moves.jl:94-172), shared out over all warps, 32/S leaves per warp step and
+    //         one lane per cell.  Cell q is occupied iff bit q of the spread! mask M is set; it then takes merged rank
+    //         r = popc(M below q), which is an insert's (bit r of insm) or else survivor number r - popc(insm below r).  Every
+    //         lane loads and stores only its own cell: a survivor's value comes by shuffle from the lane of its old cell (phase
+    //         C's in-place overwrites are in global memory), its key from the staged keys. ---------------------------------
+    {
+        constexpr int G = 32 >> lgS;                       // leaves per warp step
+        const int nrelay = s.nrelay;
+        const int q = lane & (S - 1), g0 = lane & ~(S - 1);   // this lane's cell in its leaf; the group's first lane
+        const unsigned below = (1u << q) - 1u;
+        int64_t* const kq = A.keys + tbase + q;
+        double* const vq = A.vals + tbase + q;
+        for (int i0 = warp * G; i0 < nrelay; i0 += WARPS * G) {   // whole warps: the shuffle and __syncwarp see every lane
+            const int i = i0 + (lane >> lgS);
+            const bool on = i < nrelay;
+            uint2 e = make_uint2(0u, 0u);   // {survivors, spread! mask}
+            int lcell = 0;
+            double vold = 0.0;              // the cell's value before the re-lay
+            if (on) {
+                e = s.u.lay.leaf[i];
+                lcell = (int)s.u.lay.lid[i] << lgS;
+                vold = vq[lcell];
+                if ((e.x >> q) & 1u) s.u.lay.sidx[lcell + __popc(e.x & below)] = (uint8_t)q;
+            }
+            __syncwarp();   // the leaf's survivor numbers are written
+            int64_t k = GAP_KEY;
+            double v = 0.0;
+            int src = -1;   // lane of the survivor that lands here
+            if ((e.y >> q) & 1u) {
+                const int r = __popc(e.y & below);
+                const unsigned insm = s.insm[lcell >> lgS];
+                if ((insm >> r) & 1u) {
+                    const int o = s.rop[lcell + r];
+                    k = s.rkey[o];
+                    v = s.rval[o];
+                } else {
+                    const int c = s.u.lay.sidx[lcell + r - __popc(insm & ((1u << r) - 1u))];
+                    k = s.sk[lcell + c];
+                    src = g0 + c;
                 }
             }
-        }
-        __syncwarp();   // every value of the warp's leaves is read before any of their cells is written
-#pragma unroll
-        for (int u = 0; u < EU; ++u) {
-            if (cell[u] >= 0) {
-                const int64_t p = tbase + cell[u];
-                A.keys[p] = k[u];
-                A.vals[p] = v[u];
-                if (k[u] == 0) A.sem[(int64_t)v[u] - 1] = p;   // moves.jl:160-166
+            const double vs = __shfl_sync(FULL, vold, src & 31);   // src < 0: no survivor lands here, vs is not used
+            if (on) {
+                if (src >= 0) v = vs;
+                kq[lcell] = k;
+                vq[lcell] = v;
+                if (k == 0) A.sem[(int64_t)v - 1] = tbase + lcell + q;   // moves.jl:160-166
             }
         }
     }
