@@ -35,6 +35,10 @@ __device__ __forceinline__ unsigned lanemask_lt() {
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
     return m;
 }
+// bits 0..x (x >= 31: all 32)
+__device__ __forceinline__ unsigned mask_le(int x) { return x >= 31 ? 0xffffffffu : ((2u << x) - 1u); }
+// bits 0..n-1, n <= 32 (the cells of a leaf of n cells)
+__host__ __device__ __forceinline__ constexpr unsigned low_bits(int n) { return n >= 32 ? 0xffffffffu : ((1u << n) - 1u); }
 __device__ __forceinline__ int64_t warp_sum_i64(int64_t v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -75,10 +79,7 @@ __global__ void __launch_bounds__(256) k_layout(int64_t* __restrict__ keys, doub
     }
     const unsigned b = __ballot_sync(0xffffffffu, live);
     const int S = 1 << lgS;
-    if (p < cap && (p & (S - 1)) == 0) {
-        unsigned m = S >= 32 ? 0xffffffffu : ((1u << S) - 1u);
-        leafcnt[p >> lgS] = __popc((b >> lane) & m);
-    }
+    if (p < cap && (p & (S - 1)) == 0) leafcnt[p >> lgS] = __popc((b >> lane) & low_bits(S));
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -483,26 +484,13 @@ __global__ void __launch_bounds__(256) k_select_pending(const int32_t* __restric
     if (blockIdx.x == 0 && threadIdx.x == 0) status[ST_ROOT] = post[L.off[L.H]];   // element count after the batch
 }
 
-__device__ __forceinline__ int nth_set_bit(unsigned m, int n) {   // position of the n-th (0-based) set bit of m
-    int pos = 0;
-#pragma unroll
-    for (int s = 16; s >= 1; s >>= 1) {
-        const unsigned low = (m >> pos) & ((1u << s) - 1u);
-        const int c = __popc(low);
-        if (n >= c) {
-            n -= c;
-            pos += s;
-        }
-    }
-    return pos;
-}
-
 // ---------------------------------------------------------------------------------------------
-// K2 + K4 merge / redistribute.  One warp per leaf (lane = cell).  The leaf's final window is its outermost marked
-// ancestor (lane h probes level h, one ballot).  Rank of an item inside its window = prefix of post counts over the
-// preceding leaves (read off the implicit tree, <= h loads) + position inside the leaf's merged run; destination =
-// window start + closed-form spread! offset.  h == 0: rewritten in place from registers; h >= 1: scattered into the
-// shadow array and copied back by k_copyback; root mode: scattered into the freshly allocated (resized) array.
+// K2 + K4 merge / redistribute.  Rank of an item inside its window = prefix of post counts over the window's preceding leaves
+// (read off the implicit tree, <= h loads) + position inside the leaf's merged run: the survivors before it + the leaf's
+// inserts whose predecessor lies before it.  Destination = window start + closed-form spread! offset.  Leaves accepted at
+// their own level are rewritten in place (k_leaf_merge), windows of at most SMALL_CELLS cells through shared memory
+// (k_window_small); bigger windows are scattered into the shadow array and copied back (k_merge_scatter_big,
+// k_scatter_inserts, k_copyback_big).  Root mode (resize): the same scatter over the root window, into the new arrays.
 // ---------------------------------------------------------------------------------------------
 struct MergeArgs {
     const int64_t* src_k;
@@ -520,98 +508,82 @@ struct MergeArgs {
     const int64_t* ins_pos;
     int32_t* leafcnt;
     int64_t* sem;   // nullable; 0-based positions per partition id
-    int root_mode;
+    int root_mode;  // resize: one window of height L.H, root_c cells, root_m elements, scattered into dst
     int64_t root_c, root_m;
-    int min_h;                 // dense path: only windows with outermost height >= min_h (the big ones)
-    const uint8_t* cover;      // per leaf: 0 = not inside a window above leaf level
+    const uint8_t* cover;      // per leaf: 0 = not inside a window above leaf level, else 1 + height of the outermost one
     const uint8_t* destpos;    // [33][32] spread! offset of rank r in a leaf holding m elements
     const ActiveLeaf* act;     // leaves that receive inserts
     const int64_t* nact_dev;
     const int32_t* hi_h;       // work list of windows above leaf level
     const int64_t* hi_w;
-    const int32_t* big_h;      // work list of the windows above SMALL_CELLS (list-driven big path)
+    const int32_t* big_h;      // work list of the windows above SMALL_CELLS
     const int64_t* big_w;
 };
 
-__device__ __forceinline__ int window_height(const uint8_t* __restrict__ mark, const Levels& L, int64_t l, int lane) {
-    bool mk = false;
-    if (lane <= L.H) mk = mark[L.off[lane] + (l >> lane)] != 0;
-    const unsigned b = __ballot_sync(0xffffffffu, mk);
-    return b ? 31 - __clz(b) : -1;
+// post count of the left sibling of leaf l's ancestor at level k.  The elements of a window of height h that lie before leaf l
+// are the sum of these over the levels k < h at which that ancestor is a right child (bit k of l set).
+__device__ __forceinline__ int32_t left_sibling_post(const int32_t* __restrict__ post, const Levels& L, int64_t l, int k) {
+    return post[L.off[k] + ((l >> k) - 1)];
+}
+// the same sum by one warp: lane k adds level k
+__device__ __forceinline__ int64_t window_prefix(const int32_t* __restrict__ post, const Levels& L, int64_t l, int h, int lane) {
+    int64_t term = 0;
+    if (lane < h && ((l >> lane) & 1)) term = left_sibling_post(post, L, l, lane);
+    return warp_sum_i64(term);
+}
+// one warp over a leaf, lane = cell p (in = the lane holds a cell): the cell's key and value; returns the leaf's survivors
+__device__ __forceinline__ unsigned load_leaf_cell(const int64_t* src_k, const double* src_v, int64_t p, bool in, int64_t& key,
+                                                   double& val) {
+    key = GAP_KEY;
+    val = 0.0;
+    if (in) {
+        key = src_k[p];
+        val = src_v[p];
+    }
+    return __ballot_sync(0xffffffffu, key != GAP_KEY);
+}
+// inserts of a leaf (predecessor cells ins_pos[0..nins), sorted) whose predecessor lies before cell p
+__device__ __forceinline__ int inserts_before(const int64_t* ins_pos, int nins, int64_t p) {
+    int lo = 0, hi = nins;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (ins_pos[mid] < p) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+// survivors of a leaf (mask lm) up to its cell qq (-1 = before the first cell): they precede an insert whose predecessor is qq
+__device__ __forceinline__ int survivors_le(unsigned lm, int qq) { return qq < 0 ? 0 : __popc(lm & mask_le(qq)); }
+// the window of height h that holds leaf l: first cell, cells, elements after the batch (root: the resized array)
+struct Window {
+    int64_t cell0, c, m;
+};
+__device__ __forceinline__ Window window_of(const MergeArgs& A, const Levels& L, int64_t l, int h, bool root) {
+    if (root) return Window{0, A.root_c, A.root_m};
+    return Window{((l >> h) << h) << L.lgS, (int64_t)(1 << L.lgS) << h, A.post[L.off[h] + (l >> h)]};
 }
 
-// one leaf of a window of height h (lane = cell): survivors ranked and scattered to their spread! positions
+// one leaf of a big window (one warp, lane = cell): survivors ranked and scattered to their spread! positions in dst.  The
+// leaf's inserts are placed by k_scatter_inserts (one thread per insert: a hot leaf may receive millions).
 __device__ __forceinline__ void merge_scatter_leaf(const MergeArgs& A, const Levels& L, int64_t l, int h, int lane) {
     const int nins = A.inscnt[l];
-    if (!A.root_mode && h == 0 && nins == 0) return;   // leaf accepted, nothing inserted: nothing moves (pma.jl:96-99)
-    const int S = 1 << L.lgS;
-    const int64_t first_leaf = (l >> h) << h;
-    const int64_t c = A.root_mode ? A.root_c : ((int64_t)S << h);
-    const int64_t m = A.root_mode ? A.root_m : (int64_t)A.post[L.off[h] + (l >> h)];
-    int64_t term = 0;
-    if (lane < h && ((l >> lane) & 1)) term = A.post[L.off[lane] + ((l >> lane) - 1)];
-    const int64_t base = warp_sum_i64(term);
-    const int64_t p0 = l << L.lgS;
-    const int64_t p = p0 + lane;
-    int64_t key = GAP_KEY;
-    double val = 0.0;
-    if (lane < S) {
-        key = A.src_k[p];
-        val = A.src_v[p];
-    }
-    const bool live = key != GAP_KEY;
-    const unsigned lm = __ballot_sync(0xffffffffu, live);
-    const int srank = __popc(lm & lanemask_lt());
     const int64_t i0 = nins ? A.ins_first[l] : 0;
-    int cntb = 0;
-    if (live && nins) {   // inserts whose predecessor lies before this cell
-        int lo = 0, hi = nins;
-        while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (A.ins_pos[i0 + mid] < p) lo = mid + 1;
-            else hi = mid;
-        }
-        cntb = lo;
-    }
-    const Spread sp = spread_make(c, m);
-    const int64_t wbase = A.root_mode ? 0 : (first_leaf << L.lgS);
-    int64_t* dk;
-    double* dv;
-    if (!A.root_mode && h == 0) {
-        dk = A.cur_k;
-        dv = A.cur_v;
-        __syncwarp();
-        if (lane < S) {
-            dk[p] = GAP_KEY;
-            dv[p] = 0.0;
-        }
-        __syncwarp();
-    } else {
-        dk = A.dst_k;
-        dv = A.dst_v;
-    }
+    const Window W = window_of(A, L, l, h, A.root_mode);
+    const int64_t base = window_prefix(A.post, L, l, h, lane);
+    const int64_t p = (l << L.lgS) + lane;
+    int64_t key;
+    double val;
+    const unsigned lm = load_leaf_cell(A.src_k, A.src_v, p, lane < (1 << L.lgS), key, val);
+    const bool live = key != GAP_KEY;
+    const int srank = __popc(lm & lanemask_lt());
+    const int cntb = live ? inserts_before(A.ins_pos + i0, nins, p) : 0;
+    const Spread sp = spread_make(W.c, W.m);
     if (live) {
-        const int64_t d = wbase + spread_dest(sp, base + srank + cntb);
-        dk[d] = key;
-        dv[d] = val;
+        const int64_t d = W.cell0 + spread_dest(sp, base + srank + cntb);
+        A.dst_k[d] = key;
+        A.dst_v[d] = val;
         if (A.sem && key == 0) A.sem[(int64_t)val - 1] = d;   // moves.jl:160-166
     }
-    // the leaf's inserts are placed by k_scatter_inserts (one thread per insert: a hot leaf may receive millions)
-    if (!A.root_mode && h == 0 && lane == 0) A.leafcnt[l] = (int32_t)m;
-}
-
-// dense: one warp per leaf of the whole array (resize: every leaf belongs to the root window)
-__global__ void __launch_bounds__(256) k_merge_scatter(MergeArgs A, Levels L) {
-    const int64_t l = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (l >= L.nsegs) return;
-    int h;
-    if (A.root_mode) h = L.H;
-    else {
-        h = window_height(A.mark, L, l, lane);
-        if (h < A.min_h) return;
-    }
-    merge_scatter_leaf(A, L, l, h, lane);
 }
 
 // outermost = no marked ancestor (a window nested in a larger marked one is re-laid by that one)
@@ -621,20 +593,30 @@ __device__ __forceinline__ bool window_is_outermost(const uint8_t* __restrict__ 
     return true;
 }
 
-// list-driven: grid = (chunks, big windows).  Only the leaves of the listed windows are visited — a skewed batch marks a few
-// hundred windows of a few thousand cells in an array of tens of millions (the dense sweep cost 2 ms per batch at 2^25 cells).
-__global__ void __launch_bounds__(256) k_merge_scatter_big(MergeArgs A, Levels L) {
+// grid = (chunks, windows): the blocks of window blockIdx.z * gridDim.y + blockIdx.y (grid.y stops at 65535) share out its
+// leaves, one warp per leaf calls leaf_fn(leaf, h, lane).  Only the leaves of the listed windows are visited — a skewed batch
+// marks a few hundred windows of a few thousand cells in an array of tens of millions.  Root mode: the one window of height
+// L.H, which is every leaf.
+template <class LeafFn>
+__device__ __forceinline__ void for_each_big_window_leaf(const MergeArgs& A, const Levels& L, int64_t nbig, LeafFn leaf_fn) {
     __shared__ int ok;
-    const int64_t i = blockIdx.y;
-    const int h = A.big_h[i];
-    const int64_t w = A.big_w[i];
-    if (threadIdx.x == 0) ok = window_is_outermost(A.mark, L, h, w);
-    __syncthreads();
-    if (!ok) return;
+    const int64_t i = (int64_t)blockIdx.z * gridDim.y + blockIdx.y;
+    if (i >= nbig) return;
+    const int h = A.root_mode ? L.H : A.big_h[i];
+    const int64_t w = A.root_mode ? 0 : A.big_w[i];
+    if (!A.root_mode) {   // (the root has no ancestor: a resize's many short blocks skip the barrier)
+        if (threadIdx.x == 0) ok = window_is_outermost(A.mark, L, h, w);
+        __syncthreads();
+        if (!ok) return;
+    }
     const int lane = threadIdx.x & 31;
     const int64_t nleaves = (int64_t)1 << h, first = w << h;
     for (int64_t j = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < nleaves; j += (int64_t)gridDim.x * (blockDim.x >> 5))
-        merge_scatter_leaf(A, L, first + j, h, lane);
+        leaf_fn(first + j, h, lane);
+}
+
+__global__ void __launch_bounds__(256) k_merge_scatter_big(MergeArgs A, Levels L, int64_t nbig) {
+    for_each_big_window_leaf(A, L, nbig, [&](int64_t l, int h, int lane) { merge_scatter_leaf(A, L, l, h, lane); });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -648,7 +630,7 @@ __global__ void __launch_bounds__(256) k_leaf_merge(MergeArgs A, Levels L) {
     const int lane = threadIdx.x & 31;
     const int lgS = L.lgS, S = 1 << lgS;
     const int grp = lane >> lgS, q = lane & (S - 1), gshift = grp << lgS;
-    const unsigned gmask = S >= 32 ? 0xffffffffu : ((1u << S) - 1u);
+    const unsigned gmask = low_bits(S);
     const int64_t e = gw * (32 >> lgS) + grp;
     const int64_t nact = *A.nact_dev;
     if (gw * (32 >> lgS) >= nact) return;
@@ -683,7 +665,7 @@ __global__ void __launch_bounds__(256) k_leaf_merge(MergeArgs A, Levels L) {
     int rj = 0;
     unsigned insbit = 0;
     if (has_ins) {
-        rj = (qq < 0 ? 0 : __popc(lm & (qq >= 31 ? 0xffffffffu : ((2u << qq) - 1u)))) + q;
+        rj = survivors_le(lm, qq) + q;
         insbit = 1u << rj;
     }
     const unsigned insmask = __reduce_or_sync(gmask << gshift, insbit);   // merged ranks taken by the inserts
@@ -700,7 +682,7 @@ __global__ void __launch_bounds__(256) k_leaf_merge(MergeArgs A, Levels L) {
             // the srank-th rank not taken by an insert: least fixed point of R = srank + #inserts at ranks <= R
             int R = srank;
             while (true) {
-                const int Rn = srank + __popc(insmask & (R >= 31 ? 0xffffffffu : ((2u << R) - 1u)));
+                const int Rn = srank + __popc(insmask & mask_le(R));
                 if (Rn == R) break;
                 R = Rn;
             }
@@ -763,41 +745,23 @@ __global__ void __launch_bounds__(256) k_window_small(MergeArgs A, Levels L, uin
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
     for (int64_t j = wid; j < ((int64_t)1 << h); j += nw) {
         const int64_t l = first_leaf + j;
-        int64_t term = 0;
-        if (lane < h && ((l >> lane) & 1)) term = A.post[L.off[lane] + ((l >> lane) - 1)];
-        const int64_t base = warp_sum_i64(term);
+        const int64_t base = window_prefix(A.post, L, l, h, lane);
         const int nins = A.inscnt[l];
         const int64_t i0 = nins ? A.ins_first[l] : 0;
         const int64_t p0 = l << lgS, p = p0 + lane;
-        int64_t key = GAP_KEY;
-        double val = 0.0;
-        if (lane < S) {
-            key = A.src_k[p];
-            val = A.src_v[p];
-        }
+        int64_t key;
+        double val;
+        const unsigned lm = load_leaf_cell(A.src_k, A.src_v, p, lane < S, key, val);
         const bool live = key != GAP_KEY;
-        const unsigned lm = __ballot_sync(0xffffffffu, live);
         const int srank = __popc(lm & lanemask_lt());
-        int cntb = 0;
-        if (live && nins) {
-            int lo = 0, hi = nins;
-            while (lo < hi) {
-                const int mid = (lo + hi) >> 1;
-                if (A.ins_pos[i0 + mid] < p) lo = mid + 1;
-                else hi = mid;
-            }
-            cntb = lo;
-        }
+        const int cntb = live ? inserts_before(A.ins_pos + i0, nins, p) : 0;
         if (live) {
             const int64_t d = spread_dest(sp, base + srank + cntb);
             sk[d] = key;
             sv[d] = val;
         }
         for (int jj = lane; jj < nins; jj += 32) {
-            const int64_t ipos = A.ins_pos[i0 + jj];
-            const int qq = (int)(ipos - p0);
-            const int surv_le = qq < 0 ? 0 : __popc(lm & (qq >= 31 ? 0xffffffffu : ((2u << qq) - 1u)));
-            const int64_t d = spread_dest(sp, base + surv_le + jj);
+            const int64_t d = spread_dest(sp, base + survivors_le(lm, (int)(A.ins_pos[i0 + jj] - p0)) + jj);
             sk[d] = A.ins_key[i0 + jj];
             sv[d] = A.ins_val[i0 + jj];
         }
@@ -816,10 +780,7 @@ __global__ void __launch_bounds__(256) k_window_small(MergeArgs A, Levels L, uin
             if (A.sem && k == 0) A.sem[(int64_t)v - 1] = p;
         }
         const unsigned b = __ballot_sync(0xffffffffu, in && k != GAP_KEY);
-        if (in && (t & (S - 1)) == 0) {
-            const unsigned mm = S >= 32 ? 0xffffffffu : ((1u << S) - 1u);
-            A.leafcnt[(ws_cell + t) >> lgS] = __popc((b >> lane) & mm);
-        }
+        if (in && (t & (S - 1)) == 0) A.leafcnt[(ws_cell + t) >> lgS] = __popc((b >> lane) & low_bits(S));
     }
 }
 
@@ -834,22 +795,17 @@ __global__ void __launch_bounds__(256) k_scatter_inserts(MergeArgs A, Levels L, 
     int h;
     if (A.root_mode) h = L.H;
     else {
-        h = (int)A.cover[l] - 1;          // height of the outermost window covering the leaf (k_cover_windows)
-        if (h < A.min_h) return;          // leaf-level or small window: placed by k_leaf_merge / k_window_small
+        h = (int)A.cover[l] - 1;          // height of the outermost window covering the leaf (k_window_small)
+        if (h <= L.hsmall) return;        // leaf-level or small window: placed by k_leaf_merge / k_window_small
     }
-    const int S = 1 << L.lgS;
-    const int64_t first_leaf = (l >> h) << h;
-    const int64_t c = A.root_mode ? A.root_c : ((int64_t)S << h);
-    const int64_t m = A.root_mode ? A.root_m : (int64_t)A.post[L.off[h] + (l >> h)];
+    const Window W = window_of(A, L, l, h, A.root_mode);
     int64_t base = 0;
     for (int k = 0; k < h; ++k)
-        if ((l >> k) & 1) base += A.post[L.off[k] + ((l >> k) - 1)];
-    const int64_t p0 = l << L.lgS;
+        if ((l >> k) & 1) base += left_sibling_post(A.post, L, l, k);
     int surv_le = 0;
-    for (int64_t p = p0; p <= ipos; ++p) surv_le += A.src_k[p] != GAP_KEY;
+    for (int64_t p = l << L.lgS; p <= ipos; ++p) surv_le += A.src_k[p] != GAP_KEY;
     const int64_t r = base + surv_le + (j - A.ins_first[l]);
-    const int64_t wbase = A.root_mode ? 0 : (first_leaf << L.lgS);
-    const int64_t d = wbase + spread_dest(spread_make(c, m), r);
+    const int64_t d = W.cell0 + spread_dest(spread_make(W.c, W.m), r);
     const int64_t ik = A.ins_key[j];
     const double iv = A.ins_val[j];
     A.dst_k[d] = ik;
@@ -857,63 +813,27 @@ __global__ void __launch_bounds__(256) k_scatter_inserts(MergeArgs A, Levels L, 
     if (A.sem && ik == 0) A.sem[(int64_t)iv - 1] = d;
 }
 
-// windows of height >= 1: copy the shadow back, writing the analytic gaps and the new leaf counts
-__device__ __forceinline__ void copyback_leaf(int64_t* __restrict__ keys, double* __restrict__ vals, const int64_t* __restrict__ scr_k,
-                                              const double* __restrict__ scr_v, const int32_t* __restrict__ post,
-                                              int32_t* __restrict__ leafcnt, const Levels& L, int64_t l, int h, int lane) {
-    const int S = 1 << L.lgS;
-    const int64_t first_leaf = (l >> h) << h;
-    const Spread sp = spread_make((int64_t)S << h, (int64_t)post[L.off[h] + (l >> h)]);
-    const int64_t p = (l << L.lgS) + lane;
-    bool live = false;
-    if (lane < S) {
-        live = spread_rank_at(sp, p - (first_leaf << L.lgS)) >= 0;
-        keys[p] = live ? scr_k[p] : GAP_KEY;
-        vals[p] = live ? scr_v[p] : 0.0;
-    }
-    const unsigned b = __ballot_sync(0xffffffffu, live);
-    if (lane == 0) leafcnt[l] = __popc(b);
-}
-__global__ void __launch_bounds__(256) k_copyback(int64_t* __restrict__ keys, double* __restrict__ vals,
-                                                   const int64_t* __restrict__ scr_k, const double* __restrict__ scr_v,
-                                                   const int32_t* __restrict__ post, const uint8_t* __restrict__ mark,
-                                                   int32_t* __restrict__ leafcnt, Levels L, int min_h) {
-    const int64_t l = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (l >= L.nsegs) return;
-    const int h = window_height(mark, L, l, lane);
-    if (h < 1 || h < min_h) return;
-    copyback_leaf(keys, vals, scr_k, scr_v, post, leafcnt, L, l, h, lane);
-}
-__global__ void __launch_bounds__(256) k_copyback_big(int64_t* __restrict__ keys, double* __restrict__ vals,
-                                                       const int64_t* __restrict__ scr_k, const double* __restrict__ scr_v,
-                                                       const int32_t* __restrict__ post, const uint8_t* __restrict__ mark,
-                                                       int32_t* __restrict__ leafcnt, Levels L, const int32_t* __restrict__ big_h,
-                                                       const int64_t* __restrict__ big_w) {
-    __shared__ int ok;
-    const int64_t i = blockIdx.y;
-    const int h = big_h[i];
-    const int64_t w = big_w[i];
-    if (threadIdx.x == 0) ok = window_is_outermost(mark, L, h, w);
-    __syncthreads();
-    if (!ok) return;
-    const int lane = threadIdx.x & 31;
-    const int64_t nleaves = (int64_t)1 << h, first = w << h;
-    for (int64_t j = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < nleaves; j += (int64_t)gridDim.x * (blockDim.x >> 5))
-        copyback_leaf(keys, vals, scr_k, scr_v, post, leafcnt, L, first + j, h, lane);
-}
-
-// recount (used after clone/import and by tests)
-__global__ void __launch_bounds__(256) k_count_leaves(const int64_t* __restrict__ keys, int64_t cap, int32_t* __restrict__ leafcnt, int lgS) {
-    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int lane = threadIdx.x & 31;
-    const bool live = p < cap && keys[p] != GAP_KEY;
-    const unsigned b = __ballot_sync(0xffffffffu, live);
-    const int S = 1 << lgS;
-    if (p < cap && (p & (S - 1)) == 0) {
-        unsigned m = S >= 32 ? 0xffffffffu : ((1u << S) - 1u);
-        leafcnt[p >> lgS] = __popc((b >> lane) & m);
-    }
+// big windows: copy the shadow back, writing the analytic gaps and the new leaf counts
+__global__ void __launch_bounds__(256) k_copyback_big(MergeArgs A, Levels L, int64_t nbig) {
+    for_each_big_window_leaf(A, L, nbig, [&](int64_t l, int h, int lane) {
+        const Window W = window_of(A, L, l, h, false);   // a resize scatters straight into the new arrays: no copy back
+        const Spread sp = spread_make(W.c, W.m);
+        const int64_t p = (l << L.lgS) + lane;
+        bool live = false;
+        if (lane < (1 << L.lgS)) {
+            live = spread_rank_at(sp, p - W.cell0) >= 0;
+            int64_t k = GAP_KEY;
+            double v = 0.0;
+            if (live) {
+                k = A.dst_k[p];
+                v = A.dst_v[p];
+            }
+            A.cur_k[p] = k;
+            A.cur_v[p] = v;
+        }
+        const unsigned b = __ballot_sync(0xffffffffu, live);
+        if (lane == 0) A.leafcnt[l] = __popc(b);
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1103,7 +1023,6 @@ struct PmaCore {
         A.destpos = destpos.p;
         A.act = ws.act.p;
         A.nact_dev = ws.status + ST_NACT;
-        const unsigned warp_grid = grid_for(nsegs * 32, 256);
         if (hs[ST_OVER] || hs[ST_UNDER]) {
             // root failed: _extend!/_shrink! (pma.jl:132-139) until the root accepts, then one full spread into the new array
             Geometry ng = geometry_after_root_failure(g, N, ws.single_op);
@@ -1112,7 +1031,9 @@ struct PmaCore {
             nk.ensure((size_t)ng.capacity);
             nv.ensure((size_t)ng.capacity);
             A.dst_k = nk.p; A.dst_v = nv.p; A.root_mode = 1; A.root_c = ng.capacity; A.root_m = N;
-            DSA_LAUNCH("merge_scatter_root", k_merge_scatter, warp_grid, 256, 0, st, A, L);
+            // the root window is every leaf (geometries are built with 2^height segments, and resizes keep that)
+            if (nsegs != (int64_t)1 << L.H) throw DsaError{DSA_ERR_INTERNAL, "nb_segments is not 2^height"};
+            DSA_LAUNCH("merge_scatter_root", k_merge_scatter_big, dim3(grid_for(nsegs * 32, 256), 1), 256, 0, st, A, L, (int64_t)1);
             if (hs[ST_NINS] > 0)
                 DSA_LAUNCH("scatter_inserts_root", k_scatter_inserts, grid_for(hs[ST_NINS], 256), 256, 0, st, A, L, ws.status + ST_NINS);
             g = ng;
@@ -1139,29 +1060,23 @@ struct PmaCore {
                 const int64_t lm_warps = (nact + leaves_per_warp - 1) / leaves_per_warp;
                 DSA_LAUNCH("leaf_merge", k_leaf_merge, grid_for(lm_warps * 32, 256), 256, 0, st, A, L);
             }
-            // bigger windows (rare: cascades): dense warp-per-leaf scatter into the shadow array + copy back
+            // bigger windows (rare: cascades): warp-per-leaf scatter into the shadow array + copy back
             if (hs[ST_ANYBIG]) {
                 A.dst_k = ws.shadow_k.ensure((size_t)g.capacity);
                 A.dst_v = ws.shadow_v.ensure((size_t)g.capacity);
-                A.min_h = L.hsmall + 1;
                 A.big_h = ws.big_h.p;
                 A.big_w = ws.big_w.p;
                 const int64_t nbig = hs[ST_NBIG];
-                const bool listed = nbig > 0 && nbig <= 65535;   // grid.y limit; beyond it (never seen) the dense sweep still works
                 // chunks per window: ~2 leaves per warp for the largest window of the batch
                 // (and at most ~128k CTAs in all: many listed windows share the chunks of the largest one)
                 const int64_t want_chunks = std::min<int64_t>(2048, std::max<int64_t>(1, (int64_t(1) << hs[ST_MAXBIGH]) / 16));
-                const unsigned ychunks = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want_chunks, (int64_t(1) << 17) / std::max<int64_t>(nbig, 1)));
-                if (listed) DSA_LAUNCH("merge_scatter_big", k_merge_scatter_big, dim3(ychunks, (unsigned)nbig), 256, 0, st, A, L);
-                else DSA_LAUNCH("merge_scatter_big", k_merge_scatter, warp_grid, 256, 0, st, A, L);
+                const unsigned ychunks = (unsigned)std::max<int64_t>(1, std::min<int64_t>(want_chunks, (int64_t(1) << 17) / nbig));
+                const int64_t wy = std::min<int64_t>(nbig, 65535);   // grid.y limit: the windows go on in grid.z
+                const dim3 grid(ychunks, (unsigned)wy, (unsigned)((nbig + wy - 1) / wy));
+                DSA_LAUNCH("merge_scatter_big", k_merge_scatter_big, grid, 256, 0, st, A, L, nbig);
                 if (hs[ST_NINS] > 0)
                     DSA_LAUNCH("scatter_inserts_big", k_scatter_inserts, grid_for(hs[ST_NINS], 256), 256, 0, st, A, L, ws.status + ST_NINS);
-                if (listed)
-                    DSA_LAUNCH("copyback_big", k_copyback_big, dim3(ychunks, (unsigned)nbig), 256, 0, st, keys.p, vals.p, A.dst_k, A.dst_v, post, mark,
-                               leafcnt.p, L, (const int32_t*)ws.big_h.p, (const int64_t*)ws.big_w.p);
-                else
-                    DSA_LAUNCH("copyback_big", k_copyback, warp_grid, 256, 0, st, keys.p, vals.p, A.dst_k, A.dst_v, post, mark, leafcnt.p, L,
-                               L.hsmall + 1);
+                DSA_LAUNCH("copyback_big", k_copyback_big, grid, 256, 0, st, A, L, nbig);
             }
         }
         nnz = N;

@@ -147,8 +147,6 @@ __global__ void __launch_bounds__(256, 6) k_tile_assign(const int64_t* __restric
     }
 }
 
-__device__ __forceinline__ unsigned mask_le_c(int x) { return x >= 31 ? 0xffffffffu : ((2u << x) - 1u); }
-
 // find (finds.jl:29-57) on the tile in shared memory: position of the hit or of the predecessor of `key` among the stored cells
 // of [lo, hi] (all of one partition), else the nearest stored cell to the left of lo (an insert's partition semaphore).
 // The reference's gapped binary search probes cells and walks over gaps; here the search first picks the LEAF — fpos[l] is the
@@ -177,7 +175,7 @@ __device__ __forceinline__ int tile_find(const int64_t* sk, const uint32_t* live
         const int c0 = best << LGS;
         unsigned m = live[best];
         if (lo > c0) m &= ~((1u << (lo - c0)) - 1u);
-        if (hi < c0 + S - 1) m &= mask_le_c(hi - c0);
+        if (hi < c0 + S - 1) m &= mask_le(hi - c0);
         while (m) {
             const int q = 31 - __clz(m);
             const int64_t k = sk[c0 + q];
@@ -193,8 +191,6 @@ __device__ __forceinline__ int tile_find(const int64_t* sk, const uint32_t* live
     while (i > 0 && sk[i] == GAP_KEY) --i;   // finds.jl:49-56 (the predecessor lies in this tile by construction)
     return i < 0 ? 0 : i;
 }
-
-__device__ __forceinline__ unsigned mask_le(int x) { return x >= 31 ? 0xffffffffu : ((2u << x) - 1u); }
 
 static_assert(TILE_CAP <= 256 && TILE_CELLS <= 2048, "op indices are stored in 8 bits, tile-local positions in 15");
 struct TileSmem {
@@ -316,7 +312,7 @@ __global__ void __launch_bounds__(TILE_THREADS, TILE_CTAS_PER_SM) k_tile_merge(T
     __syncthreads();
     {   // live masks: a warp reads a row of 32 cells, the first 32/S lanes store the masks of its leaves
         constexpr int G = 32 >> lgS;
-        constexpr unsigned gmask = S >= 32 ? 0xffffffffu : ((1u << (S & 31)) - 1u);
+        constexpr unsigned gmask = low_bits(S);
 #pragma unroll
         for (int i = 0; i < RPW; ++i) {
             const int row = i * WARPS + warp;

@@ -7,7 +7,7 @@ import pytest
 
 import dsa_b200 as D
 from oracle import oracle as O
-from test_gpu_parity import assert_matrix_equal, assert_vec_equal, _rel_close
+from test_gpu_parity import BIG_WINDOW_KERNELS, RESIZE_KERNELS, _kernels_of, assert_matrix_equal, assert_vec_equal, _rel_close
 
 pytestmark = pytest.mark.gpu
 
@@ -145,11 +145,12 @@ def test_config5_skewed_inserts_cascading_rebalances():
     I, J = rng.integers(1, m + 1, 200_000), rng.integers(1, n + 1, 200_000)
     V = rng.random(200_000) + 0.01
     gm, pol = D.dynamicsparse(I, J, V, m=m, n=n), O.Matrix(I, J, V, m=m, n=n)
+    names = set()
     for rnd in range(3):
         nb = 60_000
         I2, J2 = _zipf(rng, m, nb), _zipf(rng, n, nb)
         V2 = rng.random(nb) + 0.01
-        gm.set_batch(I2, J2, V2)
+        names |= _kernels_of(lambda: gm.set_batch(I2, J2, V2))
         pol.set_batch_policy(I2, J2, V2)
         assert_matrix_equal(gm, pol)
     # monotone: 100 hot columns receive long runs of consecutive new row ids
@@ -160,9 +161,10 @@ def test_config5_skewed_inserts_cascading_rebalances():
         J2 = np.repeat(hot, 400)
         V2 = rng.random(len(I2)) + 0.01
         base += 400
-        gm.set_batch(I2, J2, V2)
+        names |= _kernels_of(lambda: gm.set_batch(I2, J2, V2))
         pol.set_batch_policy(I2, J2, V2)
         assert_matrix_equal(gm, pol)
+    assert BIG_WINDOW_KERNELS <= names, sorted(names)   # windows above SMALL_CELLS cells
     seq = O.Matrix(I, J, V, m=m, n=n)          # reference semantics on the final contents (one pass is enough: contents are order-free
     # across batches only through LWW, which the policy oracle already matched batch by batch; re-check one skewed batch sequentially)
     I2, J2, V2 = _zipf(rng, m, 20_000), _zipf(rng, n, 20_000), rng.random(20_000) + 0.01
@@ -178,12 +180,14 @@ def test_growth_from_empty_matches_reference_structure():
     """a matrix that starts empty keeps segment capacity 8 and doubles through _extend! (pma.jl:143-151)"""
     rng = np.random.default_rng(8)
     gm, pol, seq = D.dynamicsparse(fill_mode=False), O.Matrix(fill_mode=False), O.Matrix(fill_mode=False)
+    names = set()
     for rnd in range(4):
         nb = 30_000
         I2, J2, V2 = rng.integers(1, 3000, nb), rng.integers(1, 2000, nb), rng.random(nb) + 0.01
-        gm.set_batch(I2, J2, V2)
+        names |= _kernels_of(lambda: gm.set_batch(I2, J2, V2))
         pol.set_batch_policy(I2, J2, V2)
         seq.set_many(I2, J2, V2)
         assert_matrix_equal(gm, pol)
         assert_matrix_equal(gm, seq, layout=False)
+    assert RESIZE_KERNELS <= names, sorted(names)
     assert gm.info(0)["segment_capacity"] == 8

@@ -11,6 +11,27 @@ from oracle import oracle as O
 pytestmark = pytest.mark.gpu
 
 SPMV_RTOL = 1e-12   # BASELINE.json north_star: "floating-point SpMV outputs within 1e-12 relative (Float64)"
+# launch names of the rebalance tiers that ordinary batches rarely reach: windows above SMALL_CELLS cells, and a resize
+BIG_WINDOW_KERNELS = {"merge_scatter_big", "scatter_inserts_big", "copyback_big"}
+RESIZE_KERNELS = {"merge_scatter_root", "scatter_inserts_root"}
+
+
+def _kernels_of(fn):
+    """names of the kernels fn() launches (per-kernel event profile of the library)"""
+    import ctypes as C
+    L = D.lib()
+    L.dsa_prof_reset()
+    L.dsa_prof_enable(C.c_int(1))
+    try:
+        fn()
+    finally:
+        L.dsa_prof_enable(C.c_int(0))
+    L.dsa_prof_dump.restype = C.c_int64
+    need = L.dsa_prof_dump(None, C.c_int64(0))
+    buf = C.create_string_buffer(int(need) + 16)
+    L.dsa_prof_dump(buf, C.c_int64(len(buf)))
+    L.dsa_prof_reset()
+    return {ln.split(",")[0] for ln in buf.value.decode().strip().splitlines() if ln}
 
 
 def assert_layout_equal(g_occ, g_key, g_val, o_tag, o_key, o_val):
@@ -117,6 +138,7 @@ def test_vec_batches_layout_equals_policy_and_contents_equal_reference(seed):
     vals = rng.random(len(keys)) + 0.5
     gv, pol, seq = D.dynamicsparsevec(keys, vals), O.Vec(keys, vals), O.Vec(keys, vals)
     live = set(keys.tolist())
+    names = set()
     for rnd in range(8):
         nb = int(rng.integers(1, 4000))
         mode = rnd % 4
@@ -134,7 +156,7 @@ def test_vec_batches_layout_equals_policy_and_contents_equal_reference(seed):
         else:
             k = rng.integers(1, 200, nb)
             v = np.where(rng.random(nb) < 0.3, 0.0, rng.random(nb) + 0.5)
-        gv.set_batch(k, v)
+        names |= _kernels_of(lambda: gv.set_batch(k, v))
         pol.set_batch_policy(k, v)
         seq.set_many(k, v)
         for kk, vv in zip(k.tolist(), v.tolist()):
@@ -146,16 +168,20 @@ def test_vec_batches_layout_equals_policy_and_contents_equal_reference(seed):
         assert gv.info()["n"] == seq.info()["n"]
         q = rng.integers(1, 50_000, 500)
         assert np.array_equal(gv.get_batch(q), seq.get_many(q))
+    if seed in (0, 2, 4, 5):   # runs of consecutive keys that no window of SMALL_CELLS cells can hold
+        assert BIG_WINDOW_KERNELS <= names, sorted(names)
 
 
 def test_vec_grow_and_shrink():
     gv, pol = D.dynamicsparsevec([], []), O.Vec([], [])
     k = np.arange(1, 100_001)
-    gv.set_batch(k, np.full(len(k), 2.0))
+    names = _kernels_of(lambda: gv.set_batch(k, np.full(len(k), 2.0)))
+    assert RESIZE_KERNELS <= names, sorted(names)
     pol.set_batch_policy(k, np.full(len(k), 2.0))
     assert_vec_equal(gv, pol)
     assert gv.info()["segment_capacity"] == 8
-    gv.set_batch(k, np.zeros(len(k)))
+    names = _kernels_of(lambda: gv.set_batch(k, np.zeros(len(k))))
+    assert "merge_scatter_root" in names, sorted(names)
     pol.set_batch_policy(k, np.zeros(len(k)))
     assert_vec_equal(gv, pol)
     assert gv.info()["nnz"] == 0 and gv.info()["capacity"] == 16

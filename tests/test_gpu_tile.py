@@ -6,7 +6,7 @@ import pytest
 
 import dsa_b200 as D
 from oracle import oracle as O
-from test_gpu_parity import assert_matrix_equal
+from test_gpu_parity import _kernels_of, assert_matrix_equal
 
 pytestmark = pytest.mark.gpu
 
@@ -16,24 +16,6 @@ def tile_mode():
     prev = D.set_tile_mode(2)
     yield D.set_tile_mode
     D.set_tile_mode(prev)
-
-
-def _kernels_of(fn):
-    """names of the kernels fn() launches (per-kernel event profile of the library)"""
-    import ctypes as C
-    L = D.lib()
-    L.dsa_prof_reset()
-    L.dsa_prof_enable(C.c_int(1))
-    try:
-        fn()
-    finally:
-        L.dsa_prof_enable(C.c_int(0))
-    L.dsa_prof_dump.restype = C.c_int64
-    need = L.dsa_prof_dump(None, C.c_int64(0))
-    buf = C.create_string_buffer(int(need) + 16)
-    L.dsa_prof_dump(buf, C.c_int64(len(buf)))
-    L.dsa_prof_reset()
-    return {ln.split(",")[0] for ln in buf.value.decode().strip().splitlines() if ln}
 
 
 def _coo(rng, m, n, nnz):
