@@ -148,10 +148,10 @@ static void phase1_validate(const Pcsr& P, const BatchCtx& c, const char* what) 
         throw DsaError{DSA_ERR_ARGUMENT, std::string(what) + " must be >= 1 (each is an in-array key of one orientation; key 0 is the semaphore key, pcsr.jl:23)"};
     const int64_t slots_after = P.nslots() + std::max<int64_t>(c.bs.missing, 0);
     if (slots_after >= (int64_t(1) << 31)) throw DsaError{DSA_ERR_ARGUMENT, "too many partitions"};
-    const int kb = std::max(1, bits_for((uint64_t)std::max<int64_t>(c.bs.maxkey, P.max_inkey)));
+    const int kb = std::max(1, bits_for((uint64_t)c.bs.maxkey - (uint64_t)c.bs.minkey + 1));
     const int pb = std::max(1, bits_for((uint64_t)std::max<int64_t>(slots_after - 1, 1)));
     if (!c.tile && (c.bs.missing > 0 || c.bs.maxbucket > BUCKET_MAX) && kb + pb > 64)   // the radix path packs (slot, key) into one 64-bit sort key
-        throw DsaError{DSA_ERR_ARGUMENT, "key range too wide: bits(max in-array key) + bits(#partitions) must be <= 64"};
+        throw DsaError{DSA_ERR_ARGUMENT, "key range too wide: bits(in-array key range + 1) + bits(#partitions) must be <= 64"};
 }
 
 static void phase1_finish(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t st) {
@@ -220,7 +220,7 @@ static void phase2_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
     const int64_t ntot = n + nnew;
     int32_t* d_new = ws.new_slots.ensure((size_t)nnew + 1);
     if (nnew) DSA_CUDA(cudaMemcpyAsync(d_new, c.new_slots_h.data(), (size_t)nnew * 4, cudaMemcpyHostToDevice, st));
-    const int kb = std::max(1, bits_for((uint64_t)c.bs.maxkey));
+    const int kb = std::max(1, bits_for((uint64_t)c.bs.maxkey - (uint64_t)c.bs.minkey + 1));   // k_make_sortkeys packs key - minkey + 1
     const int pb = std::max(1, bits_for((uint64_t)std::max<int64_t>(P.nslots() - 1, 1)));
     if (c.tile) {
         // one CTA per tile: locate, apply, re-lay the accepted leaves; then the shared tail (density tree, window selection)
@@ -251,7 +251,6 @@ static void phase2_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
         P.pma.rebalance_launch(ws.batch, st);
         return;
     }
-    if (kb + pb > 64) throw DsaError{DSA_ERR_ARGUMENT, "key range too wide: bits(max in-array key) + bits(#partitions) must be <= 64"};
     const unsigned grt = grid_for(ntot, 256);
     int32_t* u_pid = ws.u_pid.ensure((size_t)ntot);
     int64_t* u_key = ws.u_key.ensure((size_t)ntot);
@@ -273,9 +272,13 @@ static void phase2_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
         P.pma.rebalance_launch(ws.batch, st);
         return;
     }
+    // only the radix path packs (slot, key) into one 64-bit sort key.  A guard, not the refusal: phase1_validate refuses such a
+    // batch first, with a partition count at least as large (it counts absent ops, not distinct keys), before any column is
+    // created; were this throw ever reached, phase1_finish would already have changed the column map.
+    if (kb + pb > 64) throw DsaError{DSA_ERR_ARGUMENT, "key range too wide: bits(in-array key range + 1) + bits(#partitions) must be <= 64"};
     uint64_t* sk = ws.sk.ensure((size_t)ntot);
     uint32_t* perm = ws.perm.ensure((size_t)ntot);
-    DSA_LAUNCH("make_sortkeys", k_make_sortkeys, grt, 256, 0, st, ws.op_slot.p, c.inkeys, n, d_new, nnew, kb, sk, perm);
+    DSA_LAUNCH("make_sortkeys", k_make_sortkeys, grt, 256, 0, st, ws.op_slot.p, c.inkeys, n, d_new, nnew, c.bs.minkey, kb, sk, perm);
     radix_sort_pairs(ws.sort, sk, perm, ntot, kb + pb, st);
     int32_t* flag = ws.flag32.ensure((size_t)ntot);
     int32_t* uidx = ws.idx32.ensure((size_t)ntot);

@@ -151,14 +151,15 @@ __global__ void __launch_bounds__(256) k_fill_i64(int64_t* a, int64_t n, int64_t
 }
 
 // ---------------------------------------------------------------------------------------------
-// batch assembly: ops + one semaphore insert per new partition; 64-bit sort key = (slot << kb) | in-array key
+// batch assembly: ops + one semaphore insert per new partition; 64-bit sort key = (slot << kb) | (in-array key - kmin + 1), so
+// that kb follows the batch's key range, not its largest key
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_make_sortkeys(const int32_t* __restrict__ op_slot, const int64_t* __restrict__ inkeys, int64_t n,
-                                                        const int32_t* __restrict__ new_slots, int64_t nnew, int kb,
+                                                        const int32_t* __restrict__ new_slots, int64_t nnew, int64_t kmin, int kb,
                                                         uint64_t* __restrict__ sk, uint32_t* __restrict__ idx) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) {
-        sk[i] = ((uint64_t)(uint32_t)op_slot[i] << kb) | (uint64_t)inkeys[i];
+        sk[i] = ((uint64_t)(uint32_t)op_slot[i] << kb) | ((uint64_t)inkeys[i] - (uint64_t)kmin + 1);
         idx[i] = (uint32_t)i;
     } else if (i < n + nnew) {
         sk[i] = ((uint64_t)(uint32_t)new_slots[i - n] << kb);   // key 0 = semaphore key: sorts first in its partition
@@ -260,14 +261,28 @@ __global__ void __launch_bounds__(256) k_gather_unique_ops(const uint64_t* __res
 // builders: duplicate-combine as a left fold in input order (vector.jl:21-31, pcsr.jl:373-398): the head of every run of
 // equal sort keys folds its run sequentially (stable sort => input order)
 // ---------------------------------------------------------------------------------------------
+// min / max are Base.min / Base.max on IEEE floats: NaN if either argument is NaN (the NaN argument itself, as x86 returns it
+// from the `x - y` Base computes), -0.0 orders below 0.0, otherwise the smaller / larger argument
+__device__ __forceinline__ double julia_min(double a, double b) {
+    if (isnan(a)) return a;
+    if (isnan(b)) return b;
+    if (a == b) return signbit(a) ? a : b;
+    return b < a ? b : a;
+}
+__device__ __forceinline__ double julia_max(double a, double b) {
+    if (isnan(a)) return a;
+    if (isnan(b)) return b;
+    if (a == b) return signbit(a) ? b : a;
+    return b > a ? b : a;
+}
 __device__ __forceinline__ double combine_apply(int c, double a, double b) {
     switch (c) {
         case DSA_COMBINE_ADD: return __dadd_rn(a, b);
         case DSA_COMBINE_MUL: return __dmul_rn(a, b);
         case DSA_COMBINE_LAST: return b;
         case DSA_COMBINE_FIRST: return a;
-        case DSA_COMBINE_MIN: return b < a ? b : a;
-        case DSA_COMBINE_MAX: return b > a ? b : a;
+        case DSA_COMBINE_MIN: return julia_min(a, b);
+        case DSA_COMBINE_MAX: return julia_max(a, b);
     }
     return __dadd_rn(a, b);
 }

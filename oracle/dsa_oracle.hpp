@@ -49,14 +49,29 @@ struct Error {
 
 enum Combine : int { COMB_ADD = 0, COMB_MUL = 1, COMB_LAST = 2, COMB_FIRST = 3, COMB_MIN = 4, COMB_MAX = 5 };
 
+// Base.min / Base.max on IEEE floats: NaN if either argument is NaN (the NaN argument itself, as x86 returns it from the
+// `x - y` Base computes), -0.0 orders below 0.0, otherwise the smaller / larger argument
+inline double julia_min(double a, double b) {
+    if (std::isnan(a)) return a;
+    if (std::isnan(b)) return b;
+    if (a == b) return std::signbit(a) ? a : b;
+    return b < a ? b : a;
+}
+inline double julia_max(double a, double b) {
+    if (std::isnan(a)) return a;
+    if (std::isnan(b)) return b;
+    if (a == b) return std::signbit(a) ? b : a;
+    return b > a ? b : a;
+}
+
 inline double combine_apply(int c, double a, double b) {
     switch (c) {
         case COMB_ADD: return a + b;
         case COMB_MUL: return a * b;
         case COMB_LAST: return b;
         case COMB_FIRST: return a;
-        case COMB_MIN: return b < a ? b : a;
-        case COMB_MAX: return b > a ? b : a;
+        case COMB_MIN: return julia_min(a, b);
+        case COMB_MAX: return julia_max(a, b);
     }
     return a + b;
 }
