@@ -711,6 +711,92 @@ class DynamicSparseMatrix:
         cur.wait_stream(hs)
         return y[:ny]
 
+    # -- compressed snapshot ------------------------------------------------------------------
+    def compressed(self, which=_lib.COLMAJOR):
+        """(part_keys, ptr, keys, vals) of one orientation, compacted on the device: the live partitions in ascending key (empty
+        ones included), 0-based offsets ptr[len(part_keys) + 1], then the entries of each partition in ascending in-array key
+        (stored zeros kept, values bit for bit).  COLMAJOR: partitions are columns, keys rows (CSC); ROWMAJOR: the transpose
+        (CSR).  Keys are decoded through the matrix's codecs."""
+        self._not_fillmode("Matrix is in fill mode, cannot take a compressed snapshot.")
+        self.flush()
+        cnt = np.zeros(2, np.int64)
+        check(lib().dsa_matrix_compress(self._h, C.c_int(which), None, None, None, None, C.c_int64(0), C.c_int64(0), _p(cnt)))
+        npart, nnz = int(cnt[0]), int(cnt[1])
+        pk, ptr = np.zeros(max(npart, 1), np.int64), np.zeros(npart + 1, np.int64)
+        k, v = np.zeros(max(nnz, 1), np.int64), np.zeros(max(nnz, 1), np.float64)
+        check(lib().dsa_matrix_compress(self._h, C.c_int(which), _p(pk), _p(ptr), _p(k), _p(v), C.c_int64(npart), C.c_int64(nnz),
+                                        _p(cnt)))
+        pc, kc = (self._cc, self._rc) if which == _lib.COLMAJOR else (self._rc, self._cc)
+        return np.asarray(pc.decode(pk[:npart])), ptr, np.asarray(kc.decode(k[:nnz])), v[:nnz]
+
+    def _dense_form(self, which, what):
+        """checks shared by to_csr / to_csc / to_torch: (m, n, dim, idim) of the orientation"""
+        self._not_fillmode(f"Matrix is in fill mode, cannot convert it {what}.")
+        if not (self._rc.identity and self._cc.identity):
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, f"conversion {what} needs integer row and column keys (this matrix has a key codec): "
+                                                       "use compressed() for the keys themselves")
+        self.flush()
+        m, n = self._dims()
+        return (m, n) + ((n, m) if which == _lib.COLMAJOR else (m, n))
+
+    def _compress_dense_host(self, which, what):
+        m, n, dim, idim = self._dense_form(which, what)
+        cnt = C.c_int64()
+        check(lib().dsa_matrix_compress_dense(self._h, C.c_int(which), C.c_int64(dim), C.c_int64(idim), C.c_int(0), None, None, None,
+                                              C.c_int64(0), C.byref(cnt)))
+        nnz = cnt.value
+        ptr, ind, v = np.zeros(dim + 1, np.int64), np.zeros(max(nnz, 1), np.int64), np.zeros(max(nnz, 1), np.float64)
+        check(lib().dsa_matrix_compress_dense(self._h, C.c_int(which), C.c_int64(dim), C.c_int64(idim), C.c_int(0), _p(ptr), _p(ind),
+                                              _p(v), C.c_int64(nnz), C.byref(cnt)))
+        return (m, n), ptr, ind[:nnz], v[:nnz]
+
+    def to_csr(self):
+        """scipy.sparse.csr_matrix of shape size, from the row-major orientation (canonical: sorted indices, no duplicates,
+        stored zeros kept).  BoundsError if an entry lies outside size (dynamicsparse(I, J, V, m, n) with m < max(I))."""
+        import scipy.sparse as sp
+        shape, ptr, ind, v = self._compress_dense_host(_lib.ROWMAJOR, "to CSR")
+        return sp.csr_matrix((v, ind, ptr), shape=shape)
+
+    def to_csc(self):
+        """scipy.sparse.csc_matrix of shape size, from the column-major orientation (see to_csr)."""
+        import scipy.sparse as sp
+        shape, ptr, ind, v = self._compress_dense_host(_lib.COLMAJOR, "to CSC")
+        return sp.csc_matrix((v, ind, ptr), shape=shape)
+
+    def to_torch(self, layout=None, device=None):
+        """torch sparse CSR (layout=torch.sparse_csr, the default) or CSC (torch.sparse_csc) tensor of shape size with int64
+        indices, filled on the device into tensors torch allocates.  The compaction runs after the work already queued on
+        torch's current stream, and the tensor is ready on that stream (no host synchronisation, unless entries outside size
+        may be stored: then BoundsError is decided before anything is written)."""
+        import torch
+        layout = torch.sparse_csr if layout is None else layout
+        if layout not in (torch.sparse_csr, torch.sparse_csc):
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, f"to_torch: layout must be torch.sparse_csr or torch.sparse_csc, not {layout}")
+        device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if device.type != "cuda":
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, f"to_torch: the matrix lives on a CUDA device, not {device}")
+        which = _lib.ROWMAJOR if layout == torch.sparse_csr else _lib.COLMAJOR
+        m, n, dim, idim = self._dense_form(which, "to torch")
+        cnt = C.c_int64()
+        check(lib().dsa_matrix_compress_dense_d(self._h, C.c_int(which), C.c_int64(dim), C.c_int64(idim), C.c_int(0), None, None, None,
+                                                C.c_int64(0), C.byref(cnt)))
+        nnz = cnt.value
+        ptr = torch.empty(dim + 1, dtype=torch.int64, device=device)
+        ind = torch.empty(nnz, dtype=torch.int64, device=device)
+        v = torch.empty(nnz, dtype=torch.float64, device=device)
+        st = C.c_void_p()
+        check(lib().dsa_matrix_get_stream(self._h, C.byref(st)))
+        # the handle keeps its own stream: order it against torch's both ways (as _mul_dense_cuda does)
+        cur = torch.cuda.current_stream(device)
+        hs = torch.cuda.ExternalStream(st.value or 0, device=device)
+        hs.wait_stream(cur)
+        check(lib().dsa_matrix_compress_dense_d(self._h, C.c_int(which), C.c_int64(dim), C.c_int64(idim), C.c_int(0),
+                                                C.c_void_p(ptr.data_ptr()), C.c_void_p(ind.data_ptr()), C.c_void_p(v.data_ptr()),
+                                                C.c_int64(nnz), C.byref(cnt)))
+        cur.wait_stream(hs)
+        ctor = torch.sparse_csr_tensor if which == _lib.ROWMAJOR else torch.sparse_csc_tensor
+        return ctor(ptr, ind, v, size=(m, n))
+
 
 def dynamicsparse(I=None, J=None, V=None, m=None, n=None, fill_mode=True, combine="+", row_codec=None, col_codec=None):
     """dynamicsparse(I, J, V, [m, n]) (matrix.jl:15-19) or dynamicsparse(Ti, Tj, Tv; fill_mode) (matrix.jl:31-41)."""

@@ -754,32 +754,21 @@ int dsa_vec_info(const dsa_vec_t* v, int64_t* out6) {
     out6[3] = v->pma.nnz; out6[4] = v->pma.g.height; out6[5] = v->n;
     return DSA_OK;
 }
-static int64_t compact_range(PcsrWorkspace& ws, const int64_t* d_keys, const double* d_vals, int64_t len, int skip_sem, int64_t* out_k,
-                             double* out_v, int64_t cap_out, cudaStream_t st) {
-    // returns the number of stored cells; fills the host outputs when they fit
-    if (len <= 0) return 0;
-    int32_t* flag = ws.flag32.ensure((size_t)len);
-    int32_t* idx = ws.idx32.ensure((size_t)len);
-    int64_t* tot = ws.nuniq.ensure(4);
-    const unsigned gr = grid_for(len, 256);
-    DSA_LAUNCH("flag_live", k_flag_live, gr, 256, 0, st, d_keys, len, flag, skip_sem);
-    exclusive_scan_i32<int32_t>(ws.batch.scan, flag, idx, len, tot, st);
-    int64_t h_tot = 0;
-    DSA_CUDA(cudaMemcpyAsync(&h_tot, tot, 8, cudaMemcpyDeviceToHost, st));
-    DSA_CUDA(cudaStreamSynchronize(st));
-    if (h_tot > 0 && out_k && h_tot <= cap_out) {
-        int64_t* ck = ws.tmp_k.ensure((size_t)h_tot);
-        double* cv = ws.tmp_v.ensure((size_t)h_tot);
-        DSA_LAUNCH("compact_cells", k_compact_cells, gr, 256, 0, st, d_keys, d_vals, len, idx, skip_sem, ck, cv);
-        DSA_CUDA(cudaMemcpyAsync(out_k, ck, (size_t)h_tot * 8, cudaMemcpyDeviceToHost, st));
-        DSA_CUDA(cudaMemcpyAsync(out_v, cv, (size_t)h_tot * 8, cudaMemcpyDeviceToHost, st));
-        DSA_CUDA(cudaStreamSynchronize(st));
-    }
-    return h_tot;
-}
 int dsa_vec_nonzeros(dsa_vec_t* v, int64_t* keys_out, double* vals_out, int64_t cap, int64_t* count_out) {
     DSA_TRY
-    *count_out = compact_range(v->ws, v->pma.keys.p, v->pma.vals.p, v->pma.g.capacity, 0, keys_out, vals_out, cap, v->sh.st);
+    // the compaction of the matrices' compressed snapshot without semaphores: a vector keeps every non-gap cell
+    const int64_t n = v->pma.nnz;
+    *count_out = n;
+    if (n > 0 && keys_out && n <= cap) {
+        cudaStream_t st = v->sh.st;
+        int64_t* ck = v->ws.tmp_k.ensure((size_t)n);
+        double* cv = v->ws.tmp_v.ensure((size_t)n);
+        compress_cells<false>(v->ws.cmp, v->pma.keys.p, v->pma.vals.p, v->pma.g.capacity, CompressBounds{}, 0, nullptr, nullptr, 0, n, ck,
+                              cv, st);
+        DSA_CUDA(cudaMemcpyAsync(keys_out, ck, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaMemcpyAsync(vals_out, cv, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaStreamSynchronize(st));
+    }
     return DSA_OK;
     DSA_CATCH
 }
@@ -1149,6 +1138,87 @@ int dsa_matrix_export(dsa_matrix_t* A, int which, uint8_t* occupied, int64_t* ke
             col_live[s] = P.slot_live[(size_t)s];
         }
     }
+    return DSA_OK;
+    DSA_CATCH
+}
+
+// ---- compressed snapshot (K8, pcsr.cuh) -------------------------------------------------------------------------------
+static Pcsr& orientation(dsa_matrix_t* A, int which) {
+    if (which != DSA_COLMAJOR && which != DSA_ROWMAJOR) throw DsaError{DSA_ERR_ARGUMENT, "which must be DSA_COLMAJOR or DSA_ROWMAJOR"};
+    return which == DSA_COLMAJOR ? A->colmajor : A->rowmajor;
+}
+// both counts are known on the host; a buffer whose required length is 0 may be NULL
+static bool compress_fits(Pcsr& P, const int64_t* part_keys, const int64_t* ptr, const int64_t* keys, const double* vals, int64_t cap_parts,
+                          int64_t cap_nnz, int64_t* counts_out2) {
+    const int64_t np = P.nlive(), nnz = P.nnz();
+    counts_out2[0] = np;
+    counts_out2[1] = nnz;
+    return ptr && cap_parts >= np && cap_nnz >= nnz && (np == 0 || part_keys) && (nnz == 0 || (keys && vals));
+}
+static bool compress_dense_fits(Pcsr& P, int64_t dim, int64_t idim, int base, const int64_t* ptr, const int64_t* ind, const double* vals,
+                                int64_t cap_nnz, int64_t* nnz_out) {
+    if (base != 0 && base != 1) throw DsaError{DSA_ERR_ARGUMENT, "compress_dense: base must be 0 or 1"};
+    if (dim < 0 || idim < 0) throw DsaError{DSA_ERR_ARGUMENT, "compress_dense: dim and idim must be >= 0"};
+    const int64_t nnz = P.nnz();
+    *nnz_out = nnz;
+    return ptr && cap_nnz >= nnz && (nnz == 0 || (ind && vals));
+}
+int dsa_matrix_compress(dsa_matrix_t* A, int which, int64_t* part_keys, int64_t* ptr, int64_t* keys, double* vals, int64_t cap_parts,
+                        int64_t cap_nnz, int64_t* counts_out2) {
+    DSA_TRY
+    Pcsr& P = orientation(A, which);
+    if (!compress_fits(P, part_keys, ptr, keys, vals, cap_parts, cap_nnz, counts_out2)) return DSA_OK;
+    cudaStream_t st = A->sh.st;
+    const int64_t np = counts_out2[0], nnz = counts_out2[1];
+    int64_t* dptr = A->stg.b.ensure((size_t)np + 1);
+    int64_t* dk = A->stg.a.ensure((size_t)std::max<int64_t>(nnz, 1));
+    double* dv = A->stg.v.ensure((size_t)std::max<int64_t>(nnz, 1));
+    P.compress_sparse(A->ws, nullptr, dptr, dk, dv, st);
+    if (np > 0) memcpy(part_keys, P.live_keys_h.data(), (size_t)np * 8);
+    DSA_CUDA(cudaMemcpyAsync(ptr, dptr, (size_t)(np + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (nnz > 0) {
+        DSA_CUDA(cudaMemcpyAsync(keys, dk, (size_t)nnz * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaMemcpyAsync(vals, dv, (size_t)nnz * 8, cudaMemcpyDeviceToHost, st));
+    }
+    DSA_CUDA(cudaStreamSynchronize(st));
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_compress_d(dsa_matrix_t* A, int which, int64_t* d_part_keys, int64_t* d_ptr, int64_t* d_keys, double* d_vals, int64_t cap_parts,
+                          int64_t cap_nnz, int64_t* counts_out2) {
+    DSA_TRY
+    Pcsr& P = orientation(A, which);
+    if (compress_fits(P, d_part_keys, d_ptr, d_keys, d_vals, cap_parts, cap_nnz, counts_out2))
+        P.compress_sparse(A->ws, d_part_keys, d_ptr, d_keys, d_vals, A->sh.st);
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_compress_dense(dsa_matrix_t* A, int which, int64_t dim, int64_t idim, int base, int64_t* ptr, int64_t* ind, double* vals,
+                              int64_t cap_nnz, int64_t* nnz_out) {
+    DSA_TRY
+    Pcsr& P = orientation(A, which);
+    if (!compress_dense_fits(P, dim, idim, base, ptr, ind, vals, cap_nnz, nnz_out)) return DSA_OK;
+    cudaStream_t st = A->sh.st;
+    const int64_t nnz = *nnz_out;
+    int64_t* dptr = A->stg.b.ensure((size_t)dim + 1);
+    int64_t* di = A->stg.a.ensure((size_t)std::max<int64_t>(nnz, 1));
+    double* dv = A->stg.v.ensure((size_t)std::max<int64_t>(nnz, 1));
+    P.compress_dense(A->ws, dim, idim, base, dptr, di, dv, st);
+    DSA_CUDA(cudaMemcpyAsync(ptr, dptr, (size_t)(dim + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (nnz > 0) {
+        DSA_CUDA(cudaMemcpyAsync(ind, di, (size_t)nnz * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaMemcpyAsync(vals, dv, (size_t)nnz * 8, cudaMemcpyDeviceToHost, st));
+    }
+    DSA_CUDA(cudaStreamSynchronize(st));
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_compress_dense_d(dsa_matrix_t* A, int which, int64_t dim, int64_t idim, int base, int64_t* d_ptr, int64_t* d_ind, double* d_vals,
+                                int64_t cap_nnz, int64_t* nnz_out) {
+    DSA_TRY
+    Pcsr& P = orientation(A, which);
+    if (compress_dense_fits(P, dim, idim, base, d_ptr, d_ind, d_vals, cap_nnz, nnz_out))
+        P.compress_dense(A->ws, dim, idim, base, d_ptr, d_ind, d_vals, A->sh.st);
     return DSA_OK;
     DSA_CATCH
 }

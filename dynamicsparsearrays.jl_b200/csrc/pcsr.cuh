@@ -796,6 +796,273 @@ __global__ void __launch_bounds__(256) k_scatter_x(const int64_t* __restrict__ x
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// K8 compressed snapshot: order-preserving compaction of the element cells of an orientation (gaps and semaphore cells
+// dropped) = canonical CSC of the column-major twin / CSR of the row-major one, because partitions lie in the array in
+// ascending key order and cells in ascending in-array key inside a partition (iterate, pma.jl:165-180; the column / row
+// gathers of pcsr.jl:234-291 for every partition at once).  A vector keeps every non-gap cell (nonzeros, vector.jl:93-109).
+// Stream compaction with in-band segment heads, bound by HBM, in two passes over the keys:
+//   count  one warp per 256-cell chunk, 8 contiguous cells per lane (256-bit loads): element count per CTA tile of 2048 cells,
+//          and (dense form, when the host cannot rule it out) the bounds flag
+//   scan   int64 offsets of the tiles: exclusive scan inside blocks of 8192 tiles + the block totals (an emitting CTA adds the
+//          totals of the blocks before its own): no 32-bit count anywhere, a 2^31-cell orientation can hold > 2^31 entries
+//   emit   same chunks: a lane ranks its elements with a warp scan on top of the tile offset and the counts of the warps before
+//          it, stages them in shared memory at their rank, and the warp writes its contiguous output range coalesced.  A lane
+//          that meets a semaphore cell (value = partition id = slot + 1) writes ptr[live_rank[slot]] = rank of the next element.
+// ---------------------------------------------------------------------------------------------
+constexpr int CMP_C = 8;                                  // cells per lane
+constexpr int CMP_WARPS = 8;                              // warps per CTA
+constexpr int CMP_TILE = 32 * CMP_C * CMP_WARPS;          // cells per CTA tile
+constexpr int CMP_STAGE = 32 * CMP_C + 32 * CMP_C / 8;    // staging slots per warp: rank r at r + r / 8 (no 16-way bank conflicts)
+constexpr int CMP_SCAN_THREADS = 1024, CMP_SCAN_ITEMS = 8, CMP_LG_SCAN_BLOCK = 13;   // tiles per scan block = 1024 x 8
+static_assert(CMP_SCAN_THREADS * CMP_SCAN_ITEMS == 1 << CMP_LG_SCAN_BLOCK, "scan block");
+
+// matrices: in-array keys are >= 1 (0 = semaphore); vectors: any key but the gap sentinel
+template <bool SEMS>
+__device__ __forceinline__ bool cmp_elem(int64_t k) { return SEMS ? k > 0 : k != GAP_KEY; }
+
+__device__ __forceinline__ void cmp_load_keys(const int64_t* keys, int64_t cap, int64_t p0, int64_t (&k)[CMP_C], uint64_t pol) {
+#pragma unroll
+    for (int c = 0; c < CMP_C; c += 4) {
+        if (p0 + c + 4 <= cap) {
+            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], pol);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 4; ++e) k[c + e] = p0 + c + e < cap ? keys[p0 + c + e] : GAP_KEY;
+        }
+    }
+}
+
+// bound_flag (nullable): set when an element lies at or after position sem[bound_slot] (bound_slot = the first live partition
+// whose key exceeds the dense dimension: every partition after it in the array has a larger key; -1 = none) or has an
+// in-array key > idim
+template <bool SEMS>
+__global__ void __launch_bounds__(256) k_compress_count(const int64_t* __restrict__ keys, int64_t cap, int32_t* __restrict__ tile_cnt,
+                                                         const int64_t* __restrict__ sem, int32_t bound_slot, int64_t idim,
+                                                         int32_t* __restrict__ bound_flag) {
+    __shared__ int32_t wc[CMP_WARPS];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t p0 = (int64_t)blockIdx.x * CMP_TILE + (int64_t)wid * (32 * CMP_C) + (int64_t)lane * CMP_C;
+    int64_t k[CMP_C];
+    cmp_load_keys(keys, cap, p0, k, l2_evict_first_policy());
+    int cnt = 0;
+#pragma unroll
+    for (int c = 0; c < CMP_C; ++c) cnt += cmp_elem<SEMS>(k[c]) ? 1 : 0;
+    if (bound_flag) {   // uniform
+        const int64_t pdim = bound_slot >= 0 ? sem[bound_slot] : INT64_MAX;
+        bool over = false;
+#pragma unroll
+        for (int c = 0; c < CMP_C; ++c) over |= cmp_elem<SEMS>(k[c]) && (p0 + c >= pdim || k[c] > idim);
+        if (__any_sync(0xffffffffu, over) && lane == 0) atomicOr(bound_flag, 1);
+    }
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if (lane == 0) wc[wid] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int s = 0;
+#pragma unroll
+        for (int w = 0; w < CMP_WARPS; ++w) s += wc[w];
+        tile_cnt[blockIdx.x] = s;
+    }
+}
+
+// tile_off[t] = sum of the counts of the tiles before t in its scan block; blk_sum[b] = total of scan block b
+__global__ void __launch_bounds__(CMP_SCAN_THREADS) k_compress_scan(const int32_t* __restrict__ tile_cnt, int64_t ntiles,
+                                                                     int64_t* __restrict__ tile_off, int64_t* __restrict__ blk_sum) {
+    __shared__ int64_t wt[CMP_SCAN_THREADS / 32];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t base = ((int64_t)blockIdx.x << CMP_LG_SCAN_BLOCK) + (int64_t)threadIdx.x * CMP_SCAN_ITEMS;
+    int64_t v[CMP_SCAN_ITEMS];
+    int64_t s = 0;
+#pragma unroll
+    for (int i = 0; i < CMP_SCAN_ITEMS; ++i) {
+        v[i] = base + i < ntiles ? tile_cnt[base + i] : 0;
+        s += v[i];
+    }
+    int64_t incl = s;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int64_t t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) wt[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+        int64_t w = wt[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t t = __shfl_up_sync(0xffffffffu, w, o);
+            if (lane >= o) w += t;
+        }
+        wt[lane] = w;
+    }
+    __syncthreads();
+    int64_t run = (wid ? wt[wid - 1] : 0) + incl - s;
+#pragma unroll
+    for (int i = 0; i < CMP_SCAN_ITEMS; ++i) {
+        if (base + i < ntiles) tile_off[base + i] = run;
+        run += v[i];
+    }
+    if (threadIdx.x == CMP_SCAN_THREADS - 1) blk_sum[blockIdx.x] = wt[CMP_SCAN_THREADS / 32 - 1];
+}
+
+// out_k = element key + key_shift (dense form: in-array key - 1 + base).  SEMS: ptr[live_rank[slot]] at every semaphore cell,
+// ptr[np] = total (by the last tile).  Outputs at ranks >= limit are not written (the caller's capacity).
+template <bool SEMS>
+__global__ void __launch_bounds__(256) k_compress_emit(const int64_t* __restrict__ keys, const double* __restrict__ vals, int64_t cap,
+                                                        const int64_t* __restrict__ tile_off, const int64_t* __restrict__ blk_sum,
+                                                        int64_t key_shift, const int32_t* __restrict__ live_rank, int64_t* __restrict__ ptr,
+                                                        int64_t np, int64_t limit, int64_t* __restrict__ out_k, double* __restrict__ out_v) {
+    __shared__ int64_t sk[CMP_WARPS][CMP_STAGE];
+    __shared__ double sv[CMP_WARPS][CMP_STAGE];
+    __shared__ int32_t wc[CMP_WARPS];
+    __shared__ int64_t s_toff;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t tile = blockIdx.x;
+    const int64_t p0 = tile * CMP_TILE + (int64_t)wid * (32 * CMP_C) + (int64_t)lane * CMP_C;
+    const uint64_t pol = l2_evict_first_policy();
+    int64_t k[CMP_C];
+    double t[CMP_C];
+#pragma unroll
+    for (int c = 0; c < CMP_C; c += 4) {
+        if (p0 + c + 4 <= cap) {
+            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], pol);
+            ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], pol);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const int64_t p = p0 + c + e;
+                k[c + e] = p < cap ? keys[p] : GAP_KEY;
+                t[c + e] = p < cap ? vals[p] : 0.0;
+            }
+        }
+    }
+    int cnt = 0;
+#pragma unroll
+    for (int c = 0; c < CMP_C; ++c) cnt += cmp_elem<SEMS>(k[c]) ? 1 : 0;
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int u = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += u;
+    }
+    const int wtot = __shfl_sync(0xffffffffu, incl, 31);
+    if (lane == 0) wc[wid] = wtot;
+    if (wid == 0) {   // tile offset = offset inside its scan block + totals of the scan blocks before it
+        const int64_t nb = tile >> CMP_LG_SCAN_BLOCK;
+        int64_t a = 0;
+        for (int64_t b = lane; b < nb; b += 32) a += blk_sum[b];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+        if (lane == 0) s_toff = tile_off[tile] + a;
+    }
+    __syncthreads();
+    int64_t wbase = s_toff;
+    int ttot = 0;
+#pragma unroll
+    for (int w = 0; w < CMP_WARPS; ++w) {
+        if (w < wid) wbase += wc[w];
+        ttot += wc[w];
+    }
+    int r = incl - cnt;   // warp-local rank of the lane's first element
+#pragma unroll
+    for (int c = 0; c < CMP_C; ++c) {
+        if (cmp_elem<SEMS>(k[c])) {
+            const int q = r + (r >> 3);
+            sk[wid][q] = k[c] + key_shift;
+            sv[wid][q] = t[c];
+            ++r;
+        } else if (SEMS && k[c] == 0) {
+            ptr[live_rank[(int32_t)t[c] - 1]] = wbase + r;
+        }
+    }
+    __syncwarp();
+    for (int i = lane; i < wtot; i += 32) {
+        const int64_t d = wbase + i;
+        if (d < limit) {
+            out_k[d] = sk[wid][i + (i >> 3)];
+            out_v[d] = sv[wid][i + (i >> 3)];
+        }
+    }
+    if (SEMS && threadIdx.x == 0 && tile == (int64_t)gridDim.x - 1) ptr[np] = s_toff + ttot;
+}
+
+__global__ void __launch_bounds__(256) k_compress_live_rank(const int32_t* __restrict__ live_slot, int64_t nlive, int32_t* __restrict__ live_rank) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < nlive) live_rank[live_slot[i]] = (int32_t)i;
+}
+
+// dense pointer over partition keys 1..dim: out[k] = base + ptr[first live partition with key >= k + 1] for k = 0..dim (the
+// entries of key k end where the next present key starts); a present key is one load of the direct-address map, others (and
+// handles without the map) a binary search over the sorted live keys
+__global__ void __launch_bounds__(256) k_compress_dense_ptr(const int64_t* __restrict__ ptr, const int64_t* __restrict__ live_keys,
+                                                             const int32_t* __restrict__ live_rank, int64_t nlive,
+                                                             const int32_t* __restrict__ keymap, int64_t keymap_min, int64_t keymap_len,
+                                                             int64_t dim, int64_t base, int64_t* __restrict__ out) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k > dim) return;
+    const int64_t key = k + 1;
+    int64_t i = -1;
+    if (keymap) {
+        const int64_t m = key - keymap_min;
+        const int32_t s = (m >= 0 && m < keymap_len) ? keymap[m] : -1;
+        if (s >= 0) i = live_rank[s];
+    }
+    if (i < 0) {
+        int64_t lo = 0, hi = nlive;
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (live_keys[mid] < key) lo = mid + 1;
+            else hi = mid;
+        }
+        i = lo;
+    }
+    out[k] = base + ptr[i];
+}
+
+struct CompressWorkspace {
+    DBuf<int32_t> tile_cnt, live_rank, flag;
+    DBuf<int64_t> tile_off, blk_sum, ptr;
+    HPinned<int32_t> h_flag;
+};
+
+// The dense form's bounds check (see k_compress_count).  check = false: the host has ruled a violation out.
+struct CompressBounds {
+    bool check = false;
+    const int64_t* sem = nullptr;
+    int32_t slot = -1;
+    int64_t idim = INT64_MAX;
+};
+
+// Count, [bounds read-back], scan, emit of the element cells of keys/vals[cap] on st.  A bounds violation throws DSA_ERR_BOUNDS
+// before the emit pass: nothing has been written then.
+template <bool SEMS>
+inline void compress_cells(CompressWorkspace& w, const int64_t* keys, const double* vals, int64_t cap, const CompressBounds& b,
+                           int64_t key_shift, const int32_t* live_rank, int64_t* ptr, int64_t np, int64_t limit, int64_t* out_k,
+                           double* out_v, cudaStream_t st) {
+    const int64_t ntiles = std::max<int64_t>(1, (cap + CMP_TILE - 1) / CMP_TILE);
+    const int64_t nblk = (ntiles + (1 << CMP_LG_SCAN_BLOCK) - 1) >> CMP_LG_SCAN_BLOCK;
+    int32_t* tile_cnt = w.tile_cnt.ensure((size_t)ntiles);
+    int64_t* tile_off = w.tile_off.ensure((size_t)ntiles);
+    int64_t* blk_sum = w.blk_sum.ensure((size_t)nblk);
+    int32_t* flag = nullptr;
+    if (b.check) {
+        flag = w.flag.ensure(1);
+        DSA_CUDA(cudaMemsetAsync(flag, 0, 4, st));
+    }
+    DSA_LAUNCH("compress_count", k_compress_count<SEMS>, (unsigned)ntiles, 256, 0, st, keys, cap, tile_cnt, b.sem, b.slot, b.idim, flag);
+    if (b.check) {
+        int32_t* h = w.h_flag.ensure(1);
+        DSA_CUDA(cudaMemcpyAsync(h, flag, 4, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaStreamSynchronize(st));
+        if (*h)
+            throw DsaError{DSA_ERR_BOUNDS, "compress_dense: an entry lies outside dim x idim (a partition key > dim or an in-array key > idim)"};
+    }
+    DSA_LAUNCH("compress_scan", k_compress_scan, (unsigned)nblk, CMP_SCAN_THREADS, 0, st, tile_cnt, ntiles, tile_off, blk_sum);
+    DSA_LAUNCH("compress_emit", k_compress_emit<SEMS>, (unsigned)ntiles, 256, 0, st, keys, vals, cap, tile_off, blk_sum, key_shift, live_rank,
+               ptr, np, limit, out_k, out_v);
+}
+
 // ---- tile-streamed batches (tile.cuh): geometry of a tile and the record an op is bucketed as ----
 #ifndef DSA_TILE_LG
 #define DSA_TILE_LG 10
@@ -836,6 +1103,7 @@ struct PcsrWorkspace {
     DBuf<uint32_t> perm;
     DBuf<uint8_t> xmask;
     DBuf<int32_t> ycnt, carry_cnt, chunk_last;
+    CompressWorkspace cmp;
     HPinned<int64_t> h_cs;
     std::vector<int64_t> h_tmp;
 };
@@ -1040,6 +1308,41 @@ struct Pcsr {
         if (ns > 0)
             DSA_LAUNCH("spmm_fix_to_dense", k_spmm_fix_to_dense, grid_for(ns * W, 256), 256, 0, st, yslot, carry, clast, d_sem.p,
                        d_next_slot.p, d_slot_key.p, ns, cap, nchunks, SPMV_LG_CHUNK, W, ncols, d_Y, ldy, key_lo, key_hi);
+    }
+
+    // slot -> index among the live slots (= rank in array order): built per call, the update path keeps no such map
+    const int32_t* compress_live_rank(PcsrWorkspace& ws, cudaStream_t st) {
+        int32_t* lr = ws.cmp.live_rank.ensure((size_t)nslots() + 1);
+        if (nlive() > 0)
+            DSA_LAUNCH("compress_live_rank", k_compress_live_rank, grid_for(nlive(), 256), 256, 0, st, d_live_slot.p, nlive(), lr);
+        return lr;
+    }
+    // sparse-pointer form (K8): part_keys[nlive] (nullable: the host copies its mirror), ptr[nlive + 1], keys / vals[nnz]
+    void compress_sparse(PcsrWorkspace& ws, int64_t* d_part_keys, int64_t* d_ptr, int64_t* d_keys, double* d_vals, cudaStream_t st) {
+        const int64_t np = nlive();
+        if (d_part_keys && np > 0) DSA_CUDA(cudaMemcpyAsync(d_part_keys, d_live_keys.p, (size_t)np * 8, cudaMemcpyDeviceToDevice, st));
+        compress_cells<true>(ws.cmp, pma.keys.p, pma.vals.p, pma.g.capacity, CompressBounds{}, 0, compress_live_rank(ws, st), d_ptr, np,
+                             nnz(), d_keys, d_vals, st);
+    }
+    // dense-pointer form (K8): ptr[dim + 1] over partition keys 1..dim, ind = in-array key - 1 + base.  DSA_ERR_BOUNDS (nothing
+    // written) if an entry lies in a partition with key > dim or has an in-array key > idim; synchronises only when the host
+    // cannot rule that out (a live partition with key > dim, or an in-array key above idim may be stored)
+    void compress_dense(PcsrWorkspace& ws, int64_t dim, int64_t idim, int64_t base, int64_t* d_ptr, int64_t* d_ind, double* d_vals,
+                        cudaStream_t st) {
+        const int64_t np = nlive();
+        const int64_t i0 = std::upper_bound(live_keys_h.begin(), live_keys_h.end(), dim) - live_keys_h.begin();
+        CompressBounds b;
+        b.check = i0 < np || max_inkey > idim;
+        if (b.check) {
+            b.sem = d_sem.p;
+            b.slot = i0 < np ? live_slot_h[(size_t)i0] : -1;
+            b.idim = idim;
+        }
+        const int32_t* lr = compress_live_rank(ws, st);
+        int64_t* sptr = ws.cmp.ptr.ensure((size_t)np + 1);
+        compress_cells<true>(ws.cmp, pma.keys.p, pma.vals.p, pma.g.capacity, b, base - 1, lr, sptr, np, nnz(), d_ind, d_vals, st);
+        DSA_LAUNCH("compress_dense_ptr", k_compress_dense_ptr, grid_for(dim + 1, 256), 256, 0, st, sptr, d_live_keys.p, lr, np, keymap(),
+                   keymap_min, keymap_len, dim, base, d_ptr);
     }
 
     void clone_from(const Pcsr& o, cudaStream_t st) {

@@ -836,29 +836,6 @@ __global__ void __launch_bounds__(256) k_copyback_big(MergeArgs A, Levels L, int
     });
 }
 
-// ---------------------------------------------------------------------------------------------
-// order-preserving compaction of the stored cells of [from, to) (iterate pma.jl:165-180, nonzeroinds/nonzeros
-// vector.jl:93-109): per-cell flags -> scan -> scatter
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_flag_live(const int64_t* __restrict__ keys, int64_t n, int32_t* __restrict__ flag, int skip_sem) {
-    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (p < n) {
-        const int64_t k = keys[p];
-        flag[p] = (k != GAP_KEY && !(skip_sem && k == 0)) ? 1 : 0;
-    }
-}
-__global__ void __launch_bounds__(256) k_compact_cells(const int64_t* __restrict__ keys, const double* __restrict__ vals, int64_t n,
-                                                        const int32_t* __restrict__ idx, int skip_sem, int64_t* __restrict__ ok,
-                                                        double* __restrict__ ov) {
-    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (p < n) {
-        const int64_t k = keys[p];
-        if (k != GAP_KEY && !(skip_sem && k == 0)) {
-            ok[idx[p]] = k;
-            ov[idx[p]] = vals[p];
-        }
-    }
-}
 __global__ void __launch_bounds__(256) k_export_cells(const int64_t* __restrict__ keys, const double* __restrict__ vals, int64_t cap,
                                                        uint8_t* __restrict__ occ, int64_t* __restrict__ ok, double* __restrict__ ov) {
     const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;

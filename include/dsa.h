@@ -149,6 +149,30 @@ int dsa_matrix_info(const dsa_matrix_t* A, int which, int64_t* out10);
 /* raw layout dump: occupied/keys/vals[capacity], semaphores[len] (1-based position, 0 = nothing), col_keys[len], col_live[len] */
 int dsa_matrix_export(dsa_matrix_t* A, int which, uint8_t* occupied, int64_t* keys, double* vals, int64_t* semaphores,
                       int64_t* col_keys, uint8_t* col_live);
+/* Compressed snapshot of ONE orientation: the column / row gathers of every partition at once (pcsr.jl:234-291) in iteration
+ * order (pma.jl:165-180), gaps and semaphore cells dropped.  which = DSA_COLMAJOR gives CSC (partition = column, index = row),
+ * DSA_ROWMAJOR gives CSR (partition = row, index = column).  Partitions in ascending key, entries in ascending in-array key
+ * inside each: sorted indices, no duplicates.  Values are copied bit for bit (stored zeros, NaN payloads and -0.0 kept); nnz is
+ * that of dsa_matrix_info.
+ * Sparse-pointer form, any keys: counts_out2 = {np, nnz}; part_keys[np] = keys of the live partitions (empty ones included),
+ * ptr[np + 1] = 0-based offsets of their entries, keys[nnz] = raw in-array keys, vals[nnz].  Two-call size query: when an
+ * output is NULL (one whose length is 0 may be) or cap_parts < np (part_keys holds cap_parts, ptr cap_parts + 1) or
+ * cap_nnz < nnz, only the counts are returned and nothing is written. */
+int dsa_matrix_compress(dsa_matrix_t* A, int which, int64_t* part_keys, int64_t* ptr, int64_t* keys, double* vals, int64_t cap_parts,
+                        int64_t cap_nnz, int64_t* counts_out2);
+int dsa_matrix_compress_d(dsa_matrix_t* A, int which, int64_t* d_part_keys, int64_t* d_ptr, int64_t* d_keys, double* d_vals,
+                          int64_t cap_parts, int64_t cap_nnz, int64_t* counts_out2);
+/* Dense-pointer form (scipy / torch / cuSPARSE / SparseMatrixCSC): the entries of partition key k (1 <= k <= dim) are
+ * ptr[k-1]-base .. ptr[k]-base-1 of ind / vals; ptr has dim + 1 entries, ind = in-array key - 1 + base; base = 0 or 1, else
+ * DSA_ERR_ARGUMENT (as is dim < 0 or idim < 0).  nnz_out = nnz; size query as above (NULL output or cap_nnz < nnz).
+ * DSA_ERR_BOUNDS, nothing written, if a partition holding an entry has key > dim or an entry's in-array key is > idim
+ * (dynamicsparse(I, J, V, m, n) stores entries outside m x n); an EMPTY live partition above dim is simply not represented.
+ * The `_d` variant synchronises only when the host cannot rule such an entry out (a live partition key > dim, or an in-array
+ * key > idim may be stored): the count pass reports it, and the host reads that report before anything is written. */
+int dsa_matrix_compress_dense(dsa_matrix_t* A, int which, int64_t dim, int64_t idim, int base, int64_t* ptr, int64_t* ind, double* vals,
+                              int64_t cap_nnz, int64_t* nnz_out);
+int dsa_matrix_compress_dense_d(dsa_matrix_t* A, int which, int64_t dim, int64_t idim, int base, int64_t* d_ptr, int64_t* d_ind,
+                                double* d_vals, int64_t cap_nnz, int64_t* nnz_out);
 
 /* ---------------------------------------------------------------- multi-GPU (SURVEY.md §8e) ---- */
 /* One process per GPU.  A dsa_dist_t is this rank's seat in a group of `world` ranks on one NVLink box; a dsa_dmatrix_t is a

@@ -324,6 +324,25 @@ end
 Base.:(*)(A::DynamicSparseMatrix, X::Matrix{Float64}) = _mul_dense(A, false, X)                           # size (size(A, 1), k)
 Base.:(*)(t::Transposed, X::Matrix{Float64}) = _mul_dense(t.array, true, X)                               # size (size(A, 2), k)
 
+# ------------------------------------------------------------------------------------------ compressed snapshot
+# The column-major orientation compacted on the device with 1-based pointers (dim = n, idim = m): colptr, rowval and nzval come
+# back exactly as SparseMatrixCSC stores them (sorted row indices, stored zeros kept).  Entries outside size(A)
+# (dynamicsparse(I, J, V, m, n) with m < maximum(I)) throw a BoundsError.
+function SparseArrays.SparseMatrixCSC(A::DynamicSparseMatrix)
+    A.fillmode && error("Matrix is in fill mode")
+    flush!(A)
+    m, n = size(A)
+    cnt = Ref{Int64}(0)
+    f(colptr, rowval, nzval, cap) = ccall((:dsa_matrix_compress_dense, libdsa), Cint,
+                                          (Ptr{Cvoid}, Cint, Int64, Int64, Cint, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Int64, Ref{Int64}),
+                                          A.h, 0, n, m, 1, colptr, rowval, nzval, cap, cnt)
+    _check(f(C_NULL, C_NULL, C_NULL, 0))                                                                  # size query: nnz
+    colptr = Vector{Int64}(undef, n + 1); rowval = Vector{Int64}(undef, cnt[]); nzval = Vector{Float64}(undef, cnt[])
+    _check(f(colptr, rowval, nzval, length(nzval)))
+    return SparseMatrixCSC(m, n, colptr, rowval, nzval)
+end
+SparseArrays.sparse(A::DynamicSparseMatrix) = SparseMatrixCSC(A)
+
 
 # ------------------------------------------------------------------------------------------ multi-GPU (include/dsa.h "multi-GPU")
 # One Julia process per GPU (e.g. under MPI.jl or Distributed).  A ShardedDynamicSparseMatrix is the same DynamicSparseMatrix
