@@ -634,9 +634,8 @@ class DynamicSparseMatrix:
         return DynamicSparseMatrix(h, row_codec=self._rc, col_codec=self._cc)
 
     # -- products -----------------------------------------------------------------------------
-    def _mul(self, x, trans, n):
-        self._not_fillmode("Matrix is in fill mode")
-        self.flush()
+    def _sparse_operand(self, x, trans):
+        """(encoded keys, values) of a sparse x in any form the products take, and the codec of the output keys"""
         xcodec, ycodec = (self._rc, self._cc) if trans else (self._cc, self._rc)
         if isinstance(x, DynamicSparseVector):   # its key type is the matrix's key type on that axis: same codec
             xk, xv = x._raw_nonzeros()
@@ -648,15 +647,63 @@ class DynamicSparseMatrix:
             xk, xv = xk[o], _f64(list(x.values()))[o]
         else:
             xk, xv = x
-        xk, xv = _i64(xk), _f64(xv)
+        return _i64(xk), _f64(xv), ycodec
+
+    def _sparse_product(self, fn, x, trans, n):
+        """a host-pointer sparse product (dsa_matrix_spmv or dsa_matrix_spmspv), returned as _mul_output does"""
+        self._not_fillmode("Matrix is in fill mode")
+        self.flush()
+        xk, xv, ycodec = self._sparse_operand(x, trans)
         cap = self.info(_lib.COLMAJOR if trans else _lib.ROWMAJOR)["nb_semaphores"]
         yk, yv = np.zeros(max(cap, 1), np.int64), np.zeros(max(cap, 1), np.float64)
         cnt = C.c_int64()
-        check(lib().dsa_matrix_spmv(self._h, C.c_int(1 if trans else 0), _p(xk), _p(xv), C.c_int64(len(xk)), _p(yk), _p(yv),
-                                    C.c_int64(cap), C.byref(cnt)))
+        check(fn(self._h, C.c_int(1 if trans else 0), _p(xk), _p(xv), C.c_int64(len(xk)), _p(yk), _p(yv), C.c_int64(cap), C.byref(cnt)))
         if not ycodec.identity:   # _mul_output for non-integer keys: the Dict itself (operations.jl:11; test/unit/spmv.jl:19-24)
             return dict(zip(ycodec.decode(yk[:cnt.value]), yv[:cnt.value].tolist()))
         return SparseVector(n, yk[:cnt.value].copy(), yv[:cnt.value].copy())
+
+    def _mul(self, x, trans, n):
+        return self._sparse_product(lib().dsa_matrix_spmv, x, trans, n)
+
+    def mul_sparse(self, x, trans=False):
+        """mat * x (or transpose(mat) * x with trans=True) for a sparse x, computed like the reference's own loop
+        (_mul_dyn_mat_col_loop!, operations.jl:62-105): x's entries in ascending key select partitions, and each touched key
+        sums its products left to right in that order, so the result equals the reference's `mat * v` bit for bit.  Its cost is
+        the stored cells of the selected columns (rows), not the size of the matrix: the product to use when x has few
+        entries.  x takes every form `A @ x` takes, with strictly ascending keys (ArgumentError otherwise), and so does the
+        result.  A pair (keys, values) of torch CUDA tensors stays on the device: the product runs after the work already
+        queued on torch's current stream, and the (int64 keys, float64 values) tensors it returns are ready on that stream.
+        That path takes and returns Int64 keys only: on a matrix with a key codec it is refused (ArgumentError)."""
+        torch = sys.modules.get("torch")
+        if torch is not None and isinstance(x, tuple) and len(x) == 2 and all(isinstance(t, torch.Tensor) and t.is_cuda for t in x):
+            return self._mul_sparse_cuda(torch, x, trans)
+        dims = self._dims()
+        return self._sparse_product(lib().dsa_matrix_spmspv, x, trans, dims[1] if trans else dims[0])
+
+    def _mul_sparse_cuda(self, torch, x, trans):
+        self._not_fillmode("Matrix is in fill mode")
+        if not (self._rc.identity and self._cc.identity):
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, "mul_sparse with torch tensors needs integer row and column keys (this matrix "
+                                                       "has a key codec): pass the keys as a list, a dict or a numpy array")
+        self.flush()
+        xk, xv = x[0].to(torch.int64).contiguous(), x[1].to(torch.float64).contiguous()
+        if xk.dim() != 1 or xv.shape != xk.shape:
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, "mul_sparse takes 1-D keys and values of the same length")
+        cap = self.info(_lib.COLMAJOR if trans else _lib.ROWMAJOR)["nb_semaphores"]
+        yk = torch.empty(max(cap, 1), dtype=torch.int64, device=xk.device)
+        yv = torch.empty(max(cap, 1), dtype=torch.float64, device=xk.device)
+        st = C.c_void_p()
+        check(lib().dsa_matrix_get_stream(self._h, C.byref(st)))
+        # the handle keeps its own stream: order it against torch's both ways (as _mul_dense_cuda does)
+        cur = torch.cuda.current_stream(xk.device)
+        hs = torch.cuda.ExternalStream(st.value or 0, device=xk.device)
+        hs.wait_stream(cur)
+        cnt = C.c_int64()
+        check(lib().dsa_matrix_spmspv_d(self._h, C.c_int(1 if trans else 0), C.c_void_p(xk.data_ptr()), C.c_void_p(xv.data_ptr()),
+                                        C.c_int64(xk.shape[0]), C.c_void_p(yk.data_ptr()), C.c_void_p(yv.data_ptr()), C.c_int64(cap),
+                                        C.byref(cnt)))
+        cur.wait_stream(hs)
+        return yk[:cnt.value], yv[:cnt.value]
 
     def __matmul__(self, x):   # mat * v  (operations.jl:14-24)
         return self._mul(x, trans=False, n=self._dims()[0])

@@ -1028,6 +1028,38 @@ int dsa_matrix_spmv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const dou
     return DSA_OK;
     DSA_CATCH
 }
+// the orientation whose partitions x selects: columns for mat * x, rows for transpose(mat) * x (operations.jl:14-36)
+static Pcsr& spmspv_orientation(dsa_matrix_t* A, int trans, int64_t nx) {
+    if (nx < 0) throw DsaError{DSA_ERR_ARGUMENT, "spmspv: nx must be >= 0"};
+    return trans ? A->rowmajor : A->colmajor;
+}
+int dsa_matrix_spmspv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const double* x_vals, int64_t nx, int64_t* y_keys, double* y_vals,
+                      int64_t cap, int64_t* count_out) {
+    DSA_TRY
+    *count_out = 0;
+    Pcsr& P = spmspv_orientation(A, trans, nx);
+    cudaStream_t st = A->sh.st;
+    const int64_t* dk = h2d(A->stg.a, x_keys, nx, st);
+    const double* dv = h2d(A->stg.v, x_vals, nx, st);
+    const int64_t cnt = P.spmspv(A->ws, dk, dv, nx, true, nullptr, nullptr, 0, st);
+    *count_out = cnt;
+    if (cnt > 0 && y_keys && y_vals && cnt <= cap) {
+        DSA_CUDA(cudaMemcpyAsync(y_keys, A->ws.tmp_k.p, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaMemcpyAsync(y_vals, A->ws.tmp_v.p, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+        DSA_CUDA(cudaStreamSynchronize(st));
+    }
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_spmspv_d(dsa_matrix_t* A, int trans, const int64_t* d_x_keys, const double* d_x_vals, int64_t nx, int64_t* d_y_keys,
+                        double* d_y_vals, int64_t cap, int64_t* count_out) {
+    DSA_TRY
+    *count_out = 0;
+    Pcsr& P = spmspv_orientation(A, trans, nx);
+    *count_out = P.spmspv(A->ws, d_x_keys, d_x_vals, nx, false, d_y_keys, d_y_vals, cap, A->sh.st);
+    return DSA_OK;
+    DSA_CATCH
+}
 static void spmv_dense_dev(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t ny) {
     cudaStream_t st = A->sh.st;
     Pcsr& P = trans ? A->colmajor : A->rowmajor;

@@ -1063,6 +1063,154 @@ inline void compress_cells(CompressWorkspace& w, const int64_t* keys, const doub
                ptr, np, limit, out_k, out_v);
 }
 
+// ---------------------------------------------------------------------------------------------
+// K9 sparse-x product driven by x's entries: mat * x over the column-major orientation, transpose(mat) * x over the row-major
+// one, exactly as _mul_dyn_mat_col_loop! does it (operations.jl:62-105): for every x entry in ascending key, the cells of that
+// partition's span, result[key] = fl(result[key] + fl(x_j * a)).  The cost is the cells of the selected partitions, not the
+// size of the matrix.
+//   locate  one thread per x entry: slot (direct-address map or binary search), span [sem + 1, span_end), the span cut into
+//           pieces of at most SPX_PIECE cells (one warp per piece: a 60 000-cell partition does not serialise one warp), and
+//           the check that x is strictly ascending
+//   count   one warp per piece: stored cells; int64 exclusive scan of the piece counts (k_compress_scan) + total
+//   emit    one warp per piece, cells in order: (key - 1, product, product index), the product index order being x order
+//   group   stable LSD radix sort by key - 1 with the product index as payload: a key's products stay in ascending x order
+//   fold    run heads flagged and ranked; one thread per run folds it left to right from 0.0 and writes (key, value)
+// ---------------------------------------------------------------------------------------------
+constexpr int SPX_LG_PIECE = 11, SPX_PIECE = 1 << SPX_LG_PIECE;
+enum { SPX_ERR = 0, SPX_NPROD = 1, SPX_NPIECES = 2, SPX_NOUT = 3, SPX_WORDS = 4 };
+// grid of the piece kernels (warp-per-piece, grid-stride): 8 CTAs of 8 warps per SM of a 148-SM part at most
+inline unsigned spx_piece_grid(int64_t npieces) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((npieces + 7) / 8, 148 * 8)); }
+
+__global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ xk, int64_t nx, const int64_t* __restrict__ live_keys,
+                                                     const int32_t* __restrict__ live_slot, int64_t nlive, const int32_t* __restrict__ keymap,
+                                                     int64_t keymap_min, int64_t keymap_len, const int64_t* __restrict__ sem,
+                                                     const int32_t* __restrict__ next_slot, int64_t cap, int64_t* __restrict__ span_from,
+                                                     int64_t* __restrict__ span_to, int32_t* __restrict__ npieces, int64_t* __restrict__ info) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nx) return;
+    const int64_t key = xk[i];
+    if (i > 0 && xk[i - 1] >= key) info[SPX_ERR] = 1;
+    int32_t s;
+    if (keymap) {
+        const uint64_t r = (uint64_t)key - (uint64_t)keymap_min;   // any Int64 key: no signed overflow
+        s = r < (uint64_t)keymap_len ? keymap[r] : -1;
+    } else {
+        s = live_lookup(live_keys, live_slot, nlive, key);
+    }
+    int64_t from = 0, to = 0;
+    if (s >= 0) {
+        from = sem[s] + 1;
+        to = span_end(sem, next_slot, s, cap);
+    }
+    span_from[i] = from;
+    span_to[i] = to;
+    npieces[i] = (int32_t)((to - from + SPX_PIECE - 1) >> SPX_LG_PIECE);
+}
+
+// piece q -> x entry i and cells [c0, c1); false for a q that names no piece (past the total, or offsets of a rejected x)
+__device__ __forceinline__ bool spx_piece(int64_t q, const int32_t* __restrict__ piece_off, const int32_t* __restrict__ npieces, int64_t nx,
+                                          const int64_t* __restrict__ span_from, const int64_t* __restrict__ span_to, int64_t& i,
+                                          int64_t& c0, int64_t& c1) {
+    int64_t lo = 0, hi = nx;   // last entry whose first piece is <= q
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (piece_off[mid] <= q) lo = mid + 1;
+        else hi = mid;
+    }
+    i = lo - 1;
+    if (i < 0) return false;
+    const int64_t j = q - piece_off[i];
+    if (j < 0 || j >= npieces[i]) return false;
+    c0 = span_from[i] + (j << SPX_LG_PIECE);
+    c1 = min(span_to[i], c0 + SPX_PIECE);
+    return true;
+}
+
+// pcnt[q] for every q < nq (zeros past the pieces: the scan reads nq counts)
+__global__ void __launch_bounds__(256) k_spx_count(const int64_t* __restrict__ keys, const int32_t* __restrict__ piece_off,
+                                                    const int32_t* __restrict__ npieces, int64_t nx, const int64_t* __restrict__ span_from,
+                                                    const int64_t* __restrict__ span_to, const int64_t* __restrict__ info, int64_t nq,
+                                                    int32_t* __restrict__ pcnt) {
+    const int lane = threadIdx.x & 31;
+    const int64_t ntot = min(info[SPX_NPIECES], nq);
+    const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
+    for (int64_t q = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; q < nq; q += nw) {
+        int64_t i, c0, c1;
+        int c = 0;
+        if (q < ntot && spx_piece(q, piece_off, npieces, nx, span_from, span_to, i, c0, c1))
+            for (int64_t p = c0 + lane; p < c1; p += 32) c += keys[p] != GAP_KEY;
+        c = __reduce_add_sync(0xffffffffu, c);
+        if (lane == 0) pcnt[q] = c;
+    }
+}
+
+// info[SPX_NPROD] = sum of the scan blocks' totals (one warp)
+__global__ void k_spx_total(const int64_t* __restrict__ blk_sum, int64_t nblk, int64_t* __restrict__ info) {
+    int64_t a = 0;
+    for (int64_t b = threadIdx.x; b < nblk; b += 32) a += blk_sum[b];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    if (threadIdx.x == 0) info[SPX_NPROD] = a;
+}
+
+__global__ void __launch_bounds__(256) k_spx_emit(const int64_t* __restrict__ keys, const double* __restrict__ vals,
+                                                   const int32_t* __restrict__ piece_off, const int32_t* __restrict__ npieces,
+                                                   const int64_t* __restrict__ span_from, const int64_t* __restrict__ span_to,
+                                                   const double* __restrict__ xv, int64_t nx, const int64_t* __restrict__ poff,
+                                                   const int64_t* __restrict__ blk_sum, const int64_t* __restrict__ info, int64_t nq,
+                                                   uint64_t* __restrict__ sk, uint32_t* __restrict__ perm, double* __restrict__ prod) {
+    const int lane = threadIdx.x & 31;
+    const int64_t ntot = min(info[SPX_NPIECES], nq);
+    const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const unsigned lt = lanemask_lt();
+    for (int64_t q = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; q < ntot; q += nw) {
+        int64_t i, c0, c1;
+        if (!spx_piece(q, piece_off, npieces, nx, span_from, span_to, i, c0, c1)) continue;
+        int64_t a = 0;   // offset = offset inside its scan block + totals of the scan blocks before it
+        for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+        int64_t o = poff[q] + a;
+        const double x = xv[i];
+        for (int64_t base = c0; base < c1; base += 32) {
+            const int64_t p = base + lane;
+            const int64_t k = p < c1 ? keys[p] : GAP_KEY;
+            const unsigned b = __ballot_sync(0xffffffffu, k != GAP_KEY);
+            if (k != GAP_KEY) {
+                const int64_t d = o + __popc(b & lt);
+                sk[d] = (uint64_t)(k - 1);
+                perm[d] = (uint32_t)d;
+                prod[d] = __dmul_rn(x, vals[p]);
+            }
+            o += __popc(b);
+        }
+    }
+}
+
+// one thread per run of equal keys (sk sorted, perm = product indices in x order within a run): the left fold from 0.0;
+// written only when out_k is set and the output count (info[SPX_NOUT]) fits cap
+__global__ void __launch_bounds__(256) k_spx_fold(const uint64_t* __restrict__ sk, const uint32_t* __restrict__ perm,
+                                                   const double* __restrict__ prod, const int32_t* __restrict__ head,
+                                                   const int32_t* __restrict__ rank, int64_t n, const int64_t* __restrict__ info, int64_t cap,
+                                                   int64_t* __restrict__ out_k, double* __restrict__ out_v) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n || !head[t] || !out_k || info[SPX_NOUT] > cap) return;
+    const uint64_t key = sk[t];
+    double acc = 0.0;
+    for (int64_t u = t; u < n && sk[u] == key; ++u) acc = __dadd_rn(acc, prod[perm[u]]);
+    out_k[rank[t]] = (int64_t)key + 1;
+    out_v[rank[t]] = acc;
+}
+
+struct SpmspvWorkspace {
+    DBuf<int64_t> span_from, span_to, poff, blk_sum, info;
+    DBuf<int32_t> npieces, piece_off, pcnt, head, rank;
+    DBuf<uint64_t> sk;
+    DBuf<uint32_t> perm;
+    DBuf<double> prod;
+    HPinned<int64_t> h_info;
+};
+
 // ---- tile-streamed batches (tile.cuh): geometry of a tile and the record an op is bucketed as ----
 #ifndef DSA_TILE_LG
 #define DSA_TILE_LG 10
@@ -1104,6 +1252,7 @@ struct PcsrWorkspace {
     DBuf<uint8_t> xmask;
     DBuf<int32_t> ycnt, carry_cnt, chunk_last;
     CompressWorkspace cmp;
+    SpmspvWorkspace spx;
     HPinned<int64_t> h_cs;
     std::vector<int64_t> h_tmp;
 };
@@ -1345,6 +1494,12 @@ struct Pcsr {
                    keymap_min, keymap_len, dim, base, d_ptr);
     }
 
+    // sparse-x product (K9): x = (d_xk, d_xv)[nx] with strictly ascending keys (DSA_ERR_ARGUMENT otherwise, nothing written);
+    // returns the output count.  stage: the output goes to ws.tmp_k / ws.tmp_v; otherwise to d_yk / d_yv, written only when
+    // both are set and the count is <= cap.  Two host synchronisations at most (nx > 0 and a product exists).
+    int64_t spmspv(PcsrWorkspace& ws, const int64_t* d_xk, const double* d_xv, int64_t nx, bool stage, int64_t* d_yk, double* d_yv,
+                   int64_t cap, cudaStream_t st);
+
     void clone_from(const Pcsr& o, cudaStream_t st) {
         pma.g = o.pma.g;
         pma.nnz = o.pma.nnz;
@@ -1411,6 +1566,59 @@ __global__ void __launch_bounds__(256) k_build_flatten(const uint64_t* __restric
         out_k[u] = inkeys[src];
         out_v[u] = acc;
     }
+}
+
+inline int64_t Pcsr::spmspv(PcsrWorkspace& ws, const int64_t* d_xk, const double* d_xv, int64_t nx, bool stage, int64_t* d_yk, double* d_yv,
+                            int64_t cap, cudaStream_t st) {
+    if (nx <= 0) return 0;
+    SpmspvWorkspace& w = ws.spx;
+    // spans of distinct partitions are disjoint: an ascending x has at most nx + capacity / SPX_PIECE pieces
+    const int64_t nq = nx + (pma.g.capacity >> SPX_LG_PIECE) + 1;
+    if (nq > INT32_MAX)   // piece counts and offsets are scanned in int32
+        throw DsaError{DSA_ERR_ARGUMENT, "spmspv: nx + capacity / " + std::to_string(SPX_PIECE) + " exceeds the 2^31 - 1 pieces the piece scan indexes"};
+    const int64_t nblk = (nq + (1 << CMP_LG_SCAN_BLOCK) - 1) >> CMP_LG_SCAN_BLOCK;
+    int64_t* info = w.info.ensure(SPX_WORDS);
+    int64_t* from = w.span_from.ensure((size_t)nx);
+    int64_t* to = w.span_to.ensure((size_t)nx);
+    int32_t* np = w.npieces.ensure((size_t)nx);
+    int32_t* poff32 = w.piece_off.ensure((size_t)nx);
+    int32_t* pcnt = w.pcnt.ensure((size_t)nq);
+    int64_t* poff = w.poff.ensure((size_t)nq);
+    int64_t* blk = w.blk_sum.ensure((size_t)nblk);
+    DSA_CUDA(cudaMemsetAsync(info, 0, SPX_WORDS * sizeof(int64_t), st));
+    DSA_LAUNCH("spmspv_locate", k_spx_locate, grid_for(nx, 256), 256, 0, st, d_xk, nx, d_live_keys.p, d_live_slot.p, nlive(), keymap(),
+               keymap_min, keymap_len, d_sem.p, d_next_slot.p, pma.g.capacity, from, to, np, info);
+    exclusive_scan_i32<int32_t>(ws.batch.scan, np, poff32, nx, info + SPX_NPIECES, st);
+    DSA_LAUNCH("spmspv_count", k_spx_count, spx_piece_grid(nq), 256, 0, st, pma.keys.p, poff32, np, nx, from, to, info, nq, pcnt);
+    DSA_LAUNCH("spmspv_scan", k_compress_scan, (unsigned)nblk, CMP_SCAN_THREADS, 0, st, pcnt, nq, poff, blk);
+    DSA_LAUNCH("spmspv_total", k_spx_total, 1, 32, 0, st, blk, nblk, info);
+    int64_t* h = w.h_info.ensure(SPX_WORDS);
+    DSA_CUDA(cudaMemcpyAsync(h, info, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    DSA_CUDA(cudaStreamSynchronize(st));   // host synchronisation 1: the ascending-x check and the product count, which sizes the sort
+    if (h[SPX_ERR]) throw DsaError{DSA_ERR_ARGUMENT, "x keys must be strictly ascending"};
+    const int64_t n = h[SPX_NPROD];
+    if (n == 0) return 0;
+    if (n > INT32_MAX)
+        throw DsaError{DSA_ERR_ARGUMENT, "spmspv: " + std::to_string(n) + " products exceed the 2^31 - 1 the grouping sort indexes"};
+    uint64_t* sk = w.sk.ensure((size_t)n);
+    uint32_t* perm = w.perm.ensure((size_t)n);
+    double* prod = w.prod.ensure((size_t)n);
+    int32_t* head = w.head.ensure((size_t)n);
+    int32_t* rank = w.rank.ensure((size_t)n);
+    DSA_LAUNCH("spmspv_emit", k_spx_emit, spx_piece_grid(nq), 256, 0, st, pma.keys.p, pma.vals.p, poff32, np, from, to, d_xv, nx, poff, blk,
+               info, nq, sk, perm, prod);
+    radix_sort_pairs(ws.sort, sk, perm, n, bits_for((uint64_t)std::max<int64_t>(max_inkey - 1, 0)), st);
+    DSA_LAUNCH("flag_run_first", k_flag_run_first, grid_for(n, 256), 256, 0, st, sk, n, head);
+    exclusive_scan_i32<int32_t>(ws.batch.scan, head, rank, n, info + SPX_NOUT, st);
+    if (stage) {
+        d_yk = ws.tmp_k.ensure((size_t)n);
+        d_yv = ws.tmp_v.ensure((size_t)n);
+        cap = n;
+    }
+    DSA_LAUNCH("spmspv_fold", k_spx_fold, grid_for(n, 256), 256, 0, st, sk, perm, prod, head, rank, n, info, cap, d_yv ? d_yk : nullptr, d_yv);
+    DSA_CUDA(cudaMemcpyAsync(h + SPX_NOUT, info + SPX_NOUT, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    DSA_CUDA(cudaStreamSynchronize(st));   // host synchronisation 2: the output count
+    return h[SPX_NOUT];
 }
 
 inline void Pcsr::build_coo_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals, int64_t n,

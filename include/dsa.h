@@ -129,6 +129,22 @@ int dsa_matrix_row(dsa_matrix_t* A, int64_t row, int64_t* keys_out, double* vals
  * (operations.jl:14-36, 62-135). Output = touched rows only, ascending, stored zeros kept (sparsevec(::Dict, n)). */
 int dsa_matrix_spmv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const double* x_vals, int64_t nx, int64_t* y_keys,
                     double* y_vals, int64_t cap, int64_t* count_out);
+/* The same products driven by x's entries, in the reference's own order (operations.jl:14-36, _mul_dyn_mat_col_loop! :62-105):
+ * trans = 0 walks the columns x selects in the column-major orientation (mat * x), trans = 1 the rows in the row-major one
+ * (transpose(mat) * x).  The cost is the stored cells of the selected partitions, not the size of the matrix.  x keys must be
+ * strictly ascending (any Int64; absent keys and deleted partitions select nothing), else DSA_ERR_ARGUMENT with nothing
+ * written.  Stored zeros and NaN in x still touch their rows.  Output: the touched keys ascending, stored zeros kept; the value
+ * of a key is the left fold fl(...fl(fl(0.0 + p_1) + p_2)... + p_L) of its products p = fl(x_j * a) in ascending x key: bit for
+ * bit the reference's `mat * v`.  count_out is always set; the outputs are written only when both are non-NULL and
+ * cap >= count (nb_partitions of the other orientation always suffices).  Device workspace: 40 B per product (stored cell of a
+ * selected partition; 56 B for the host variant, which also stages the output), 28 B per x entry and 12 B per piece
+ * (nx + capacity / 2048 pieces at most); more than 2^31 - 1 products or pieces is DSA_ERR_ARGUMENT, nothing written.  The
+ * `_d` variant takes device pointers,
+ * enqueues on the handle's stream and synchronises at most twice: for the product count and for the output count. */
+int dsa_matrix_spmspv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const double* x_vals, int64_t nx, int64_t* y_keys,
+                      double* y_vals, int64_t cap, int64_t* count_out);
+int dsa_matrix_spmspv_d(dsa_matrix_t* A, int trans, const int64_t* d_x_keys, const double* d_x_vals, int64_t nx, int64_t* d_y_keys,
+                        double* d_y_vals, int64_t cap, int64_t* count_out);
 /* dense-x variant: x_j = x[j-1] for j in 1..nx (every entry stored); y[i-1] for i in 1..ny, 0.0 where no entry */
 int dsa_matrix_spmv_dense(dsa_matrix_t* A, int trans, const double* x, int64_t nx, double* y, int64_t ny);
 int dsa_matrix_spmv_dense_d(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t ny);

@@ -11,6 +11,7 @@ using SparseArrays
 export DynamicSparseVector, DynamicSparseMatrix, DynamicMatrixColView, dynamicsparsevec, dynamicsparse, nbpartitions,
        deletecolumn!, deleterow!, addrow!, closefillmode!, shrink_size!,
        set_batch!, stage_batch!, apply_staged!        # additions: batched and double-buffered writes (no reference counterpart)
+export spmspv                                          # addition: sparse product in the reference's summation order
 
 const libdsa = get(ENV, "LIBDSA", joinpath(@__DIR__, "..", "dynamicsparsearrays.jl_b200", "libdsa.so"))
 const COMBINE = Dict{Any,Cint}(+ => 0, * => 1, max => 5, min => 4)
@@ -306,6 +307,21 @@ Base.:(*)(A::DynamicSparseMatrix, v::VecLike) = _mul(A, false, _xs(v)..., size(A
 Base.:(*)(t::Transposed, v::VecLike) = _mul(t.array, true, _xs(v)..., size(t.array, 2))                   # operations.jl:26-36
 Base.:(*)(v::VecLike, t::Transposed) = _mul(t.array, false, _xs(v)..., size(t.array, 1))                  # operations.jl:38-48
 Base.:(*)(v::VecLike, A::DynamicSparseMatrix) = _mul(A, true, _xs(v)..., size(A, 2))                      # operations.jl:50-60
+
+# The same products driven by v's entries, in the reference's own loop order (_mul_dyn_mat_col_loop!, operations.jl:62-105):
+# the cost is the stored cells of the columns (rows) v selects, and the result is bit for bit the reference's `mat * v`.
+function _spmspv(A::DynamicSparseMatrix, trans::Bool, xk::Vector{Int64}, xv::Vector{Float64}, n)
+    A.fillmode && error("Matrix is in fill mode")
+    flush!(A)
+    cap = _minfo(A, trans ? 0 : 1)[7]
+    yk = Vector{Int64}(undef, cap); yv = Vector{Float64}(undef, cap); cnt = Ref{Int64}(0)
+    _check(ccall((:dsa_matrix_spmspv, libdsa), Cint,
+                 (Ptr{Cvoid}, Cint, Ptr{Int64}, Ptr{Float64}, Int64, Ptr{Int64}, Ptr{Float64}, Int64, Ref{Int64}),
+                 A.h, trans ? 1 : 0, xk, xv, length(xk), yk, yv, cap, cnt))
+    return SparseVector(n, yk[1:cnt[]], yv[1:cnt[]])
+end
+spmspv(A::DynamicSparseMatrix, v::VecLike) = _spmspv(A, false, _xs(v)..., size(A, 1))                     # operations.jl:14-24
+spmspv(t::Transposed, v::VecLike) = _spmspv(t.array, true, _xs(v)..., size(t.array, 2))                   # operations.jl:26-36
 
 # k dense right-hand sides in one call (one pass over the matrix per 32 columns); column c of the result equals the product
 # with X[:, c] bit for bit.  The library takes row-major buffers: permutedims turns the column-major X into one (ldx = k).
