@@ -673,10 +673,26 @@ class DynamicSparseMatrix:
         entries.  x takes every form `A @ x` takes, with strictly ascending keys (ArgumentError otherwise), and so does the
         result.  A pair (keys, values) of torch CUDA tensors stays on the device: the product runs after the work already
         queued on torch's current stream, and the (int64 keys, float64 values) tensors it returns are ready on that stream.
-        That path takes and returns Int64 keys only: on a matrix with a key codec it is refused (ArgumentError)."""
+        That path takes and returns Int64 keys only: on a matrix with a key codec it is refused (ArgumentError).
+
+        x may also be a matrix X of k sparse columns, multiplied in one call: column c of the result equals mul_sparse(X[:, c])
+        bit for bit.  A scipy.sparse matrix or array (any format; duplicates are summed, row r is key r + 1) gives a
+        scipy.sparse.csc_matrix of shape (size[0], k) (size[1] with trans); a DynamicSparseMatrix B gives A·B through
+        B.to_csc(); a torch sparse CSC CUDA tensor stays on the device, ordered against torch's current stream as above, and
+        gives an int64-indexed torch sparse CSC tensor.  X's row count is not checked against the matrix: as with a vector,
+        keys that name no column (row) of the matrix select nothing.  A result key above the output dimension (the matrix
+        stores entries outside its size) is BoundsError.  The matrix forms need integer keys: a key codec is ArgumentError."""
         torch = sys.modules.get("torch")
         if torch is not None and isinstance(x, tuple) and len(x) == 2 and all(isinstance(t, torch.Tensor) and t.is_cuda for t in x):
             return self._mul_sparse_cuda(torch, x, trans)
+        if torch is not None and isinstance(x, torch.Tensor) and x.layout == torch.sparse_csc:
+            return self._mul_sparse_csc_cuda(torch, x, trans)
+        if isinstance(x, DynamicSparseMatrix):
+            self._matrix_operand_checks()
+            x = x.to_csc()
+        scipy_sparse = sys.modules.get("scipy.sparse")
+        if scipy_sparse is not None and scipy_sparse.issparse(x):
+            return self._mul_sparse_matrix(scipy_sparse, x, trans)
         dims = self._dims()
         return self._sparse_product(lib().dsa_matrix_spmspv, x, trans, dims[1] if trans else dims[0])
 
@@ -704,6 +720,69 @@ class DynamicSparseMatrix:
                                         C.byref(cnt)))
         cur.wait_stream(hs)
         return yk[:cnt.value], yv[:cnt.value]
+
+    def _matrix_operand_checks(self):
+        self._not_fillmode("Matrix is in fill mode")
+        if not (self._rc.identity and self._cc.identity):
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, "mul_sparse with a matrix operand needs integer row and column keys (this "
+                                                       "matrix has a key codec): multiply its columns one by one")
+        self.flush()
+
+    @staticmethod
+    def _check_result_keys(top, ny):
+        if top > ny:
+            raise _lib.BoundsError(_lib.DSA_ERR_BOUNDS, f"mul_sparse: result key {top} is above the output dimension {ny} (the matrix "
+                                                        "stores entries outside its size)")
+
+    def _mul_sparse_matrix(self, sp, X, trans):
+        """A·X / Aᵀ·X for a scipy.sparse X through dsa_matrix_spmspm: a size query, then the fill"""
+        self._matrix_operand_checks()
+        ny = self._dims()[1 if trans else 0]
+        X = sp.csc_matrix(X, dtype=np.float64, copy=True)
+        X.sum_duplicates()                                   # canonical: duplicates summed, indices sorted in each column
+        k = X.shape[1]
+        xp, xk, xv = _i64(X.indptr), _i64(X.indices) + 1, _f64(X.data)
+        t, cnt = C.c_int(1 if trans else 0), C.c_int64()
+        args = (self._h, t, _p(xp), _p(xk), _p(xv), C.c_int64(k), C.c_int64(len(xk)))
+        check(lib().dsa_matrix_spmspm(*args, None, None, None, C.c_int64(0), C.byref(cnt)))
+        nnz = cnt.value
+        yp, yk, yv = np.zeros(k + 1, np.int64), np.zeros(max(nnz, 1), np.int64), np.zeros(max(nnz, 1), np.float64)
+        check(lib().dsa_matrix_spmspm(*args, _p(yp), _p(yk), _p(yv), C.c_int64(nnz), C.byref(cnt)))
+        yk, yv = yk[:nnz], yv[:nnz]
+        if nnz:
+            self._check_result_keys(int(yk.max()), ny)
+        return sp.csc_matrix((yv, yk - 1, yp), shape=(ny, k))
+
+    def _mul_sparse_csc_cuda(self, torch, X, trans):
+        """A·X / Aᵀ·X for a torch sparse CSC CUDA tensor through dsa_matrix_spmspm_d: a size query, then the fill"""
+        if not X.is_cuda or X.dim() != 2:
+            raise ArgumentError(_lib.DSA_ERR_ARGUMENT, "mul_sparse takes a 2-D torch sparse CSC tensor on a CUDA device")
+        self._matrix_operand_checks()
+        ny = self._dims()[1 if trans else 0]
+        dev, k = X.device, X.shape[1]
+        xp = X.ccol_indices().to(torch.int64).contiguous()
+        xk = (X.row_indices().to(torch.int64) + 1).contiguous()
+        xv = X.values().to(torch.float64).contiguous()
+        yp = torch.empty(k + 1, dtype=torch.int64, device=dev)
+        st = C.c_void_p()
+        check(lib().dsa_matrix_get_stream(self._h, C.byref(st)))
+        # the handle keeps its own stream: order it against torch's both ways (as _mul_dense_cuda does)
+        cur = torch.cuda.current_stream(dev)
+        hs = torch.cuda.ExternalStream(st.value or 0, device=dev)
+        t, cnt = C.c_int(1 if trans else 0), C.c_int64()
+        args = (self._h, t, C.c_void_p(xp.data_ptr()), C.c_void_p(xk.data_ptr()), C.c_void_p(xv.data_ptr()), C.c_int64(k),
+                C.c_int64(xk.shape[0]), C.c_void_p(yp.data_ptr()))
+        hs.wait_stream(cur)
+        check(lib().dsa_matrix_spmspm_d(*args, None, None, C.c_int64(0), C.byref(cnt)))
+        nnz = cnt.value
+        yk = torch.empty(nnz, dtype=torch.int64, device=dev)
+        yv = torch.empty(nnz, dtype=torch.float64, device=dev)
+        hs.wait_stream(cur)                                  # yk / yv were allocated on torch's stream
+        check(lib().dsa_matrix_spmspm_d(*args, C.c_void_p(yk.data_ptr()), C.c_void_p(yv.data_ptr()), C.c_int64(nnz), C.byref(cnt)))
+        cur.wait_stream(hs)
+        if nnz:
+            self._check_result_keys(int(yk.max()), ny)
+        return torch.sparse_csc_tensor(yp, yk - 1, yv, size=(ny, k))
 
     def __matmul__(self, x):   # mat * v  (operations.jl:14-24)
         return self._mul(x, trans=False, n=self._dims()[0])

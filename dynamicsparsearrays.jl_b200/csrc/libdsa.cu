@@ -1041,7 +1041,7 @@ int dsa_matrix_spmspv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const d
     cudaStream_t st = A->sh.st;
     const int64_t* dk = h2d(A->stg.a, x_keys, nx, st);
     const double* dv = h2d(A->stg.v, x_vals, nx, st);
-    const int64_t cnt = P.spmspv(A->ws, dk, dv, nx, true, nullptr, nullptr, 0, st);
+    const int64_t cnt = P.spmspv(A->ws, dk, dv, nx, true, nullptr, nullptr, y_keys && y_vals ? cap : 0, st);
     *count_out = cnt;
     if (cnt > 0 && y_keys && y_vals && cnt <= cap) {
         DSA_CUDA(cudaMemcpyAsync(y_keys, A->ws.tmp_k.p, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
@@ -1057,6 +1057,45 @@ int dsa_matrix_spmspv_d(dsa_matrix_t* A, int trans, const int64_t* d_x_keys, con
     *count_out = 0;
     Pcsr& P = spmspv_orientation(A, trans, nx);
     *count_out = P.spmspv(A->ws, d_x_keys, d_x_vals, nx, false, d_y_keys, d_y_vals, cap, A->sh.st);
+    return DSA_OK;
+    DSA_CATCH
+}
+// k sparse right-hand sides: column c of the result is the spmspv product with X[:, c] (checks of x_ptr and of the key order
+// in Pcsr::spmspm, on the device)
+static Pcsr& spmspm_orientation(dsa_matrix_t* A, int trans, const int64_t* x_ptr, int64_t k, int64_t nnz_x) {
+    if (k < 0 || nnz_x < 0) throw DsaError{DSA_ERR_ARGUMENT, "spmspm: k and nnz_x must be >= 0"};
+    if (!x_ptr) throw DsaError{DSA_ERR_ARGUMENT, "spmspm: x_ptr must hold k + 1 offsets"};
+    return trans ? A->rowmajor : A->colmajor;
+}
+int dsa_matrix_spmspm(dsa_matrix_t* A, int trans, const int64_t* x_ptr, const int64_t* x_keys, const double* x_vals, int64_t k,
+                      int64_t nnz_x, int64_t* y_ptr, int64_t* y_keys, double* y_vals, int64_t cap, int64_t* count_out) {
+    DSA_TRY
+    *count_out = 0;
+    Pcsr& P = spmspm_orientation(A, trans, x_ptr, k, nnz_x);
+    cudaStream_t st = A->sh.st;
+    const int64_t* dp = h2d(A->stg.b, x_ptr, k + 1, st);
+    const int64_t* dk = h2d(A->stg.a, x_keys, nnz_x, st);
+    const double* dv = h2d(A->stg.v, x_vals, nnz_x, st);
+    const bool want = y_keys && y_vals;
+    const int64_t cnt = P.spmspm(A->ws, dp, dk, dv, k, nnz_x, true, nullptr, nullptr, nullptr, want ? cap : 0, st);
+    *count_out = cnt;
+    if (cnt <= cap && (y_ptr || want)) {
+        if (y_ptr) DSA_CUDA(cudaMemcpyAsync(y_ptr, A->ws.spx.yptr.p, (size_t)(k + 1) * 8, cudaMemcpyDeviceToHost, st));
+        if (want && cnt > 0) {
+            DSA_CUDA(cudaMemcpyAsync(y_keys, A->ws.tmp_k.p, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+            DSA_CUDA(cudaMemcpyAsync(y_vals, A->ws.tmp_v.p, (size_t)cnt * 8, cudaMemcpyDeviceToHost, st));
+        }
+        DSA_CUDA(cudaStreamSynchronize(st));
+    }
+    return DSA_OK;
+    DSA_CATCH
+}
+int dsa_matrix_spmspm_d(dsa_matrix_t* A, int trans, const int64_t* d_x_ptr, const int64_t* d_x_keys, const double* d_x_vals, int64_t k,
+                        int64_t nnz_x, int64_t* d_y_ptr, int64_t* d_y_keys, double* d_y_vals, int64_t cap, int64_t* count_out) {
+    DSA_TRY
+    *count_out = 0;
+    Pcsr& P = spmspm_orientation(A, trans, d_x_ptr, k, nnz_x);
+    *count_out = P.spmspm(A->ws, d_x_ptr, d_x_keys, d_x_vals, k, nnz_x, false, d_y_ptr, d_y_keys, d_y_vals, cap, A->sh.st);
     return DSA_OK;
     DSA_CATCH
 }

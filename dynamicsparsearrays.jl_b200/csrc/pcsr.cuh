@@ -1067,29 +1067,56 @@ inline void compress_cells(CompressWorkspace& w, const int64_t* keys, const doub
 // K9 sparse-x product driven by x's entries: mat * x over the column-major orientation, transpose(mat) * x over the row-major
 // one, exactly as _mul_dyn_mat_col_loop! does it (operations.jl:62-105): for every x entry in ascending key, the cells of that
 // partition's span, result[key] = fl(result[key] + fl(x_j * a)).  The cost is the cells of the selected partitions, not the
-// size of the matrix.
-//   locate  one thread per x entry: slot (direct-address map or binary search), span [sem + 1, span_end), the span cut into
-//           pieces of at most SPX_PIECE cells (one warp per piece: a 60 000-cell partition does not serialise one warp), and
-//           the check that x is strictly ascending
-//   count   one warp per piece: stored cells; int64 exclusive scan of the piece counts (k_compress_scan) + total
-//   emit    one warp per piece, cells in order: (key - 1, product, product index), the product index order being x order
-//   group   stable LSD radix sort by key - 1 with the product index as payload: a key's products stay in ascending x order
-//   fold    run heads flagged and ranked; one thread per run folds it left to right from 0.0 and writes (key, value)
+// size of the matrix.  k right-hand sides (X in CSC over keys: x_ptr[k + 1], keys ascending in each column) go through the same
+// kernels in one call: every product is tagged with its column, and column c of the result is the one-vector product with
+// X[:, c].  The one-vector product is the case k = 1 with no x_ptr.
+//   locate  one thread per x entry: its column (binary search in x_ptr), slot (direct-address map or binary search), span
+//           [sem + 1, span_end), the span cut into pieces of at most SPX_PIECE cells (one warp per piece: a 60 000-cell
+//           partition does not serialise one warp), and the check that x is strictly ascending inside its column
+//   count   one warp per piece: stored cells; int64 exclusive scan of the piece counts (k_compress_scan)
+//   cols    one warp per column boundary c: the check of x_ptr, its first piece and its first product (product offsets of
+//           the columns, read back with the error flag)
+//   rounds  the host cuts the columns into consecutive rounds of at most SPX_ROUND_PRODUCTS products (one column may exceed
+//           it alone) and at most 2^(64 - keybits) columns, so that the sort key (column - round start) << keybits | key - 1
+//           fits 64 bits.  Per round, with no host synchronisation between rounds:
+//     emit  one warp per piece of the round, cells in order: (sort key, product, product index), the index order being x order
+//     group stable LSD radix sort over colbits + keybits bits with the product index as payload: a (column, key)'s products
+//           stay in ascending x order
+//     fold  run heads flagged and ranked; one thread per run folds it left to right from 0.0 and writes (key, value) at the
+//           device-resident running output offset, and the first run of a column writes the column pointers
 // ---------------------------------------------------------------------------------------------
 constexpr int SPX_LG_PIECE = 11, SPX_PIECE = 1 << SPX_LG_PIECE;
-enum { SPX_ERR = 0, SPX_NPROD = 1, SPX_NPIECES = 2, SPX_NOUT = 3, SPX_WORDS = 4 };
+constexpr int64_t SPX_ROUND_PRODUCTS = int64_t(1) << 27;   // products of one round: 40 B each, 5.4 GB of workspace
+// info words; the column product offsets (k + 1) follow them.  NOUT: outputs of the rounds before the last one folded,
+// RUNS: outputs of that round (the next round's emit moves them into NOUT)
+enum { SPX_ERR = 0, SPX_NPIECES = 1, SPX_NOUT = 2, SPX_RUNS = 3, SPX_WORDS = 4 };
 // grid of the piece kernels (warp-per-piece, grid-stride): 8 CTAs of 8 warps per SM of a 148-SM part at most
 inline unsigned spx_piece_grid(int64_t npieces) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((npieces + 7) / 8, 148 * 8)); }
 
-__global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ xk, int64_t nx, const int64_t* __restrict__ live_keys,
+// xptr == nullptr: one column holding all nx entries (xcol not written)
+__global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ xk, int64_t nx, const int64_t* __restrict__ xptr,
+                                                     int64_t ncol, const int64_t* __restrict__ live_keys,
                                                      const int32_t* __restrict__ live_slot, int64_t nlive, const int32_t* __restrict__ keymap,
                                                      int64_t keymap_min, int64_t keymap_len, const int64_t* __restrict__ sem,
                                                      const int32_t* __restrict__ next_slot, int64_t cap, int64_t* __restrict__ span_from,
-                                                     int64_t* __restrict__ span_to, int32_t* __restrict__ npieces, int64_t* __restrict__ info) {
+                                                     int64_t* __restrict__ span_to, int32_t* __restrict__ npieces, int64_t* __restrict__ xcol,
+                                                     int64_t* __restrict__ info) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nx) return;
     const int64_t key = xk[i];
-    if (i > 0 && xk[i - 1] >= key) info[SPX_ERR] = 1;
+    int64_t first = 0;
+    if (xptr) {   // the last column c with xptr[c] <= i (a malformed x_ptr gives some c in [0, ncol): k_spx_cols refuses it)
+        int64_t lo = 0, hi = ncol;
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (xptr[mid] <= i) lo = mid + 1;
+            else hi = mid;
+        }
+        const int64_t c = lo > 0 ? lo - 1 : 0;
+        xcol[i] = c;
+        first = xptr[c];
+    }
+    if (i > first && xk[i - 1] >= key) info[SPX_ERR] = 1;
     int32_t s;
     if (keymap) {
         const uint64_t r = (uint64_t)key - (uint64_t)keymap_min;   // any Int64 key: no signed overflow
@@ -1144,41 +1171,68 @@ __global__ void __launch_bounds__(256) k_spx_count(const int64_t* __restrict__ k
     }
 }
 
-// info[SPX_NPROD] = sum of the scan blocks' totals (one warp)
-__global__ void k_spx_total(const int64_t* __restrict__ blk_sum, int64_t nblk, int64_t* __restrict__ info) {
-    int64_t a = 0;
-    for (int64_t b = threadIdx.x; b < nblk; b += 32) a += blk_sum[b];
+// one warp per column boundary c in [0, ncol]: x_ptr checked (starts at 0, never decreases, ends at nx), col_piece[c] = first
+// piece of column c, info[SPX_WORDS + c] = first product of column c (info[SPX_WORDS + ncol] = the product count).
+// xptr == nullptr: one column [0, nx).  Indices are clamped, so a malformed x (refused at the read-back) reads in bounds.
+__global__ void __launch_bounds__(256) k_spx_cols(const int64_t* __restrict__ xptr, int64_t ncol, int64_t nx,
+                                                   const int32_t* __restrict__ piece_off, const int64_t* __restrict__ poff,
+                                                   const int64_t* __restrict__ blk_sum, int64_t nq, int64_t* __restrict__ info,
+                                                   int64_t* __restrict__ col_piece) {
+    const int lane = threadIdx.x & 31;
+    const int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (c > ncol) return;
+    int64_t e = c == 0 ? 0 : nx;
+    if (xptr) {
+        e = xptr[c];
+        if (lane == 0 && ((c == 0 ? e != 0 : e < xptr[c - 1]) || (c == ncol && e != nx))) info[SPX_ERR] = 1;
+        e = min(max(e, (int64_t)0), nx);
+    }
+    const int64_t q = min(max(e < nx ? (int64_t)piece_off[e] : info[SPX_NPIECES], (int64_t)0), nq - 1);
+    int64_t a = 0;   // as k_spx_emit: offset inside its scan block + totals of the scan blocks before it
+    for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-    if (threadIdx.x == 0) info[SPX_NPROD] = a;
+    if (lane == 0) {
+        col_piece[c] = q;
+        info[SPX_WORDS + c] = poff[q] + a;
+    }
 }
 
+// one round: the pieces of columns [c0, c0 + nc), their products at (global product index - p0).  The sort key of a product is
+// (column - c0) << kb | key - 1 (xcol == nullptr: column 0).  Block 0 first folds the previous round's outputs into NOUT.
 __global__ void __launch_bounds__(256) k_spx_emit(const int64_t* __restrict__ keys, const double* __restrict__ vals,
                                                    const int32_t* __restrict__ piece_off, const int32_t* __restrict__ npieces,
                                                    const int64_t* __restrict__ span_from, const int64_t* __restrict__ span_to,
-                                                   const double* __restrict__ xv, int64_t nx, const int64_t* __restrict__ poff,
-                                                   const int64_t* __restrict__ blk_sum, const int64_t* __restrict__ info, int64_t nq,
-                                                   uint64_t* __restrict__ sk, uint32_t* __restrict__ perm, double* __restrict__ prod) {
+                                                   const double* __restrict__ xv, int64_t nx, const int64_t* __restrict__ xcol,
+                                                   const int64_t* __restrict__ poff, const int64_t* __restrict__ blk_sum,
+                                                   const int64_t* __restrict__ col_piece, int64_t c0, int64_t nc, int kb, int64_t p0,
+                                                   int64_t* __restrict__ info, uint64_t* __restrict__ sk, uint32_t* __restrict__ perm,
+                                                   double* __restrict__ prod) {
     const int lane = threadIdx.x & 31;
-    const int64_t ntot = min(info[SPX_NPIECES], nq);
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        info[SPX_NOUT] += info[SPX_RUNS];
+        info[SPX_RUNS] = 0;
+    }
+    const int64_t q1 = col_piece[c0 + nc];
     const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
     const unsigned lt = lanemask_lt();
-    for (int64_t q = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; q < ntot; q += nw) {
-        int64_t i, c0, c1;
-        if (!spx_piece(q, piece_off, npieces, nx, span_from, span_to, i, c0, c1)) continue;
+    for (int64_t q = col_piece[c0] + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); q < q1; q += nw) {
+        int64_t i, cf, cl;
+        if (!spx_piece(q, piece_off, npieces, nx, span_from, span_to, i, cf, cl)) continue;
         int64_t a = 0;   // offset = offset inside its scan block + totals of the scan blocks before it
         for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-        int64_t o = poff[q] + a;
+        int64_t o = poff[q] + a - p0;
         const double x = xv[i];
-        for (int64_t base = c0; base < c1; base += 32) {
+        const uint64_t tag = xcol ? (uint64_t)(xcol[i] - c0) << kb : 0;
+        for (int64_t base = cf; base < cl; base += 32) {
             const int64_t p = base + lane;
-            const int64_t k = p < c1 ? keys[p] : GAP_KEY;
+            const int64_t k = p < cl ? keys[p] : GAP_KEY;
             const unsigned b = __ballot_sync(0xffffffffu, k != GAP_KEY);
             if (k != GAP_KEY) {
                 const int64_t d = o + __popc(b & lt);
-                sk[d] = (uint64_t)(k - 1);
+                sk[d] = tag | (uint64_t)(k - 1);
                 perm[d] = (uint32_t)d;
                 prod[d] = __dmul_rn(x, vals[p]);
             }
@@ -1187,28 +1241,48 @@ __global__ void __launch_bounds__(256) k_spx_emit(const int64_t* __restrict__ ke
     }
 }
 
-// one thread per run of equal keys (sk sorted, perm = product indices in x order within a run): the left fold from 0.0;
-// written only when out_k is set and the output count (info[SPX_NOUT]) fits cap
+// one thread per run of equal sort keys (sk sorted, perm = product indices in x order within a run): the left fold from 0.0,
+// written at NOUT + rank when out_k is set and the outputs through this round (NOUT + RUNS) fit cap.  yptr (nullable): the
+// first run of a column sets the pointers of the columns since the previous run's, the last run those up to the round's end.
 __global__ void __launch_bounds__(256) k_spx_fold(const uint64_t* __restrict__ sk, const uint32_t* __restrict__ perm,
                                                    const double* __restrict__ prod, const int32_t* __restrict__ head,
                                                    const int32_t* __restrict__ rank, int64_t n, const int64_t* __restrict__ info, int64_t cap,
-                                                   int64_t* __restrict__ out_k, double* __restrict__ out_v) {
+                                                   int64_t* __restrict__ out_k, double* __restrict__ out_v, int kb, int64_t c0, int64_t nc,
+                                                   int64_t* __restrict__ yptr) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= n || !head[t] || !out_k || info[SPX_NOUT] > cap) return;
+    if (t >= n || !head[t]) return;
+    const bool write = out_k && info[SPX_NOUT] + info[SPX_RUNS] <= cap;
+    if (!write && !yptr) return;
     const uint64_t key = sk[t];
-    double acc = 0.0;
-    for (int64_t u = t; u < n && sk[u] == key; ++u) acc = __dadd_rn(acc, prod[perm[u]]);
-    out_k[rank[t]] = (int64_t)key + 1;
-    out_v[rank[t]] = acc;
+    const int64_t o = info[SPX_NOUT] + rank[t];
+    if (write) {
+        double acc = 0.0;
+        for (int64_t u = t; u < n && sk[u] == key; ++u) acc = __dadd_rn(acc, prod[perm[u]]);
+        out_k[o] = (int64_t)(kb ? key & (~uint64_t(0) >> (64 - kb)) : 0) + 1;   // kb = 0: every key is 1
+        out_v[o] = acc;
+    }
+    if (yptr) {
+        const int64_t col = (int64_t)(key >> kb);
+        for (int64_t j = t ? (int64_t)(sk[t - 1] >> kb) + 1 : 0; j <= col; ++j) yptr[c0 + j] = o;
+        if (sk[n - 1] == key)
+            for (int64_t j = col + 1; j <= nc; ++j) yptr[c0 + j] = o + 1;
+    }
+}
+
+// column pointers of a round without products: every one is the running output offset
+__global__ void __launch_bounds__(256) k_spx_ptr_fill(const int64_t* __restrict__ info, int64_t c0, int64_t nc, int64_t* __restrict__ yptr) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j <= nc) yptr[c0 + j] = info[SPX_NOUT] + info[SPX_RUNS];
 }
 
 struct SpmspvWorkspace {
-    DBuf<int64_t> span_from, span_to, poff, blk_sum, info;
+    DBuf<int64_t> span_from, span_to, poff, blk_sum, info, xcol, col_piece, yptr;
     DBuf<int32_t> npieces, piece_off, pcnt, head, rank;
     DBuf<uint64_t> sk;
     DBuf<uint32_t> perm;
     DBuf<double> prod;
     HPinned<int64_t> h_info;
+    std::vector<int64_t> h_cut;   // column boundaries of the rounds
 };
 
 // ---- tile-streamed batches (tile.cuh): geometry of a tile and the record an op is bucketed as ----
@@ -1498,7 +1572,16 @@ struct Pcsr {
     // returns the output count.  stage: the output goes to ws.tmp_k / ws.tmp_v; otherwise to d_yk / d_yv, written only when
     // both are set and the count is <= cap.  Two host synchronisations at most (nx > 0 and a product exists).
     int64_t spmspv(PcsrWorkspace& ws, const int64_t* d_xk, const double* d_xv, int64_t nx, bool stage, int64_t* d_yk, double* d_yv,
-                   int64_t cap, cudaStream_t st);
+                   int64_t cap, cudaStream_t st) {
+        return spmspm(ws, nullptr, d_xk, d_xv, 1, nx, stage, nullptr, d_yk, d_yv, cap, st);
+    }
+    // the same product for k = ncol columns of X (CSC: d_xptr[ncol + 1], keys strictly ascending in each column; a malformed
+    // x_ptr or key order is DSA_ERR_ARGUMENT, nothing written).  d_xptr == nullptr: one column of nx entries.  d_yptr
+    // (nullable, ncol + 1) is written whatever cap; a round writes its keys and values only when the outputs through it fit
+    // cap.  stage: the outputs go to ws.tmp_k / ws.tmp_v (min(cap, products) entries) and ws.spx.yptr (when d_xptr is set).
+    // Two host synchronisations at most: the column product offsets, and the output count.
+    int64_t spmspm(PcsrWorkspace& ws, const int64_t* d_xptr, const int64_t* d_xk, const double* d_xv, int64_t ncol, int64_t nx, bool stage,
+                   int64_t* d_yptr, int64_t* d_yk, double* d_yv, int64_t cap, cudaStream_t st);
 
     void clone_from(const Pcsr& o, cudaStream_t st) {
         pma.g = o.pma.g;
@@ -1568,57 +1651,92 @@ __global__ void __launch_bounds__(256) k_build_flatten(const uint64_t* __restric
     }
 }
 
-inline int64_t Pcsr::spmspv(PcsrWorkspace& ws, const int64_t* d_xk, const double* d_xv, int64_t nx, bool stage, int64_t* d_yk, double* d_yv,
-                            int64_t cap, cudaStream_t st) {
-    if (nx <= 0) return 0;
+inline int64_t Pcsr::spmspm(PcsrWorkspace& ws, const int64_t* d_xptr, const int64_t* d_xk, const double* d_xv, int64_t ncol, int64_t nx,
+                            bool stage, int64_t* d_yptr, int64_t* d_yk, double* d_yv, int64_t cap, cudaStream_t st) {
+    if (!d_xptr && nx <= 0) return 0;
     SpmspvWorkspace& w = ws.spx;
-    // spans of distinct partitions are disjoint: an ascending x has at most nx + capacity / SPX_PIECE pieces
-    const int64_t nq = nx + (pma.g.capacity >> SPX_LG_PIECE) + 1;
-    if (nq > INT32_MAX)   // piece counts and offsets are scanned in int32
-        throw DsaError{DSA_ERR_ARGUMENT, "spmspv: nx + capacity / " + std::to_string(SPX_PIECE) + " exceeds the 2^31 - 1 pieces the piece scan indexes"};
+    // spans of distinct partitions are disjoint: a column ascending in x has at most (its entries) + capacity / SPX_PIECE
+    // pieces, and at most min(ncol, nx) columns have entries
+    const int64_t cap_pieces = pma.g.capacity >> SPX_LG_PIECE, busy = std::min(ncol, nx);
+    if (nx > INT32_MAX || (busy > 0 && cap_pieces > (INT32_MAX - 1 - nx) / busy))   // piece counts and offsets are scanned in int32
+        throw DsaError{DSA_ERR_ARGUMENT, "spmspv: x entries + min(columns, x entries) x capacity / " + std::to_string(SPX_PIECE) +
+                                             " exceed the 2^31 - 1 pieces the piece scan indexes"};
+    const int64_t nq = nx + busy * cap_pieces + 1;
     const int64_t nblk = (nq + (1 << CMP_LG_SCAN_BLOCK) - 1) >> CMP_LG_SCAN_BLOCK;
-    int64_t* info = w.info.ensure(SPX_WORDS);
+    int64_t* info = w.info.ensure((size_t)(SPX_WORDS + ncol + 1));
     int64_t* from = w.span_from.ensure((size_t)nx);
     int64_t* to = w.span_to.ensure((size_t)nx);
     int32_t* np = w.npieces.ensure((size_t)nx);
     int32_t* poff32 = w.piece_off.ensure((size_t)nx);
+    int64_t* xcol = d_xptr ? w.xcol.ensure((size_t)nx) : nullptr;
+    int64_t* col_piece = w.col_piece.ensure((size_t)ncol + 1);
     int32_t* pcnt = w.pcnt.ensure((size_t)nq);
     int64_t* poff = w.poff.ensure((size_t)nq);
     int64_t* blk = w.blk_sum.ensure((size_t)nblk);
     DSA_CUDA(cudaMemsetAsync(info, 0, SPX_WORDS * sizeof(int64_t), st));
-    DSA_LAUNCH("spmspv_locate", k_spx_locate, grid_for(nx, 256), 256, 0, st, d_xk, nx, d_live_keys.p, d_live_slot.p, nlive(), keymap(),
-               keymap_min, keymap_len, d_sem.p, d_next_slot.p, pma.g.capacity, from, to, np, info);
+    if (nx > 0)
+        DSA_LAUNCH("spmspv_locate", k_spx_locate, grid_for(nx, 256), 256, 0, st, d_xk, nx, d_xptr, ncol, d_live_keys.p, d_live_slot.p, nlive(),
+                   keymap(), keymap_min, keymap_len, d_sem.p, d_next_slot.p, pma.g.capacity, from, to, np, xcol, info);
     exclusive_scan_i32<int32_t>(ws.batch.scan, np, poff32, nx, info + SPX_NPIECES, st);
     DSA_LAUNCH("spmspv_count", k_spx_count, spx_piece_grid(nq), 256, 0, st, pma.keys.p, poff32, np, nx, from, to, info, nq, pcnt);
     DSA_LAUNCH("spmspv_scan", k_compress_scan, (unsigned)nblk, CMP_SCAN_THREADS, 0, st, pcnt, nq, poff, blk);
-    DSA_LAUNCH("spmspv_total", k_spx_total, 1, 32, 0, st, blk, nblk, info);
-    int64_t* h = w.h_info.ensure(SPX_WORDS);
-    DSA_CUDA(cudaMemcpyAsync(h, info, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    DSA_CUDA(cudaStreamSynchronize(st));   // host synchronisation 1: the ascending-x check and the product count, which sizes the sort
-    if (h[SPX_ERR]) throw DsaError{DSA_ERR_ARGUMENT, "x keys must be strictly ascending"};
-    const int64_t n = h[SPX_NPROD];
-    if (n == 0) return 0;
-    if (n > INT32_MAX)
-        throw DsaError{DSA_ERR_ARGUMENT, "spmspv: " + std::to_string(n) + " products exceed the 2^31 - 1 the grouping sort indexes"};
-    uint64_t* sk = w.sk.ensure((size_t)n);
-    uint32_t* perm = w.perm.ensure((size_t)n);
-    double* prod = w.prod.ensure((size_t)n);
-    int32_t* head = w.head.ensure((size_t)n);
-    int32_t* rank = w.rank.ensure((size_t)n);
-    DSA_LAUNCH("spmspv_emit", k_spx_emit, spx_piece_grid(nq), 256, 0, st, pma.keys.p, pma.vals.p, poff32, np, from, to, d_xv, nx, poff, blk,
-               info, nq, sk, perm, prod);
-    radix_sort_pairs(ws.sort, sk, perm, n, bits_for((uint64_t)std::max<int64_t>(max_inkey - 1, 0)), st);
-    DSA_LAUNCH("flag_run_first", k_flag_run_first, grid_for(n, 256), 256, 0, st, sk, n, head);
-    exclusive_scan_i32<int32_t>(ws.batch.scan, head, rank, n, info + SPX_NOUT, st);
+    DSA_LAUNCH("spmspv_cols", k_spx_cols, grid_for((ncol + 1) * 32, 256), 256, 0, st, d_xptr, ncol, nx, poff32, poff, blk, nq, info, col_piece);
+    int64_t* h = w.h_info.ensure((size_t)(SPX_WORDS + ncol + 1));
+    DSA_CUDA(cudaMemcpyAsync(h, info, (SPX_WORDS + ncol + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    DSA_CUDA(cudaStreamSynchronize(st));   // host synchronisation 1: the checks of x and the column product offsets, which cut the rounds
+    if (h[SPX_ERR])
+        throw DsaError{DSA_ERR_ARGUMENT, d_xptr ? "x_ptr must start at 0, never decrease and end at nnz_x, and x keys must be strictly "
+                                                  "ascending inside each column"
+                                                : "x keys must be strictly ascending"};
+    const int64_t* hc = h + SPX_WORDS;   // hc[c]: first product of column c
+    for (int64_t c = 0; c < ncol; ++c)
+        if (hc[c + 1] - hc[c] > INT32_MAX)
+            throw DsaError{DSA_ERR_ARGUMENT, "spmspv: column " + std::to_string(c) + " has " + std::to_string(hc[c + 1] - hc[c]) +
+                                                 " products, more than the 2^31 - 1 the grouping sort indexes"};
+    const int64_t total = hc[ncol];
     if (stage) {
-        d_yk = ws.tmp_k.ensure((size_t)n);
-        d_yv = ws.tmp_v.ensure((size_t)n);
-        cap = n;
+        cap = std::min(std::max<int64_t>(cap, 0), total);
+        d_yk = ws.tmp_k.ensure((size_t)std::max<int64_t>(cap, 1));
+        d_yv = ws.tmp_v.ensure((size_t)std::max<int64_t>(cap, 1));
+        d_yptr = d_xptr ? w.yptr.ensure((size_t)ncol + 1) : nullptr;
     }
-    DSA_LAUNCH("spmspv_fold", k_spx_fold, grid_for(n, 256), 256, 0, st, sk, perm, prod, head, rank, n, info, cap, d_yv ? d_yk : nullptr, d_yv);
-    DSA_CUDA(cudaMemcpyAsync(h + SPX_NOUT, info + SPX_NOUT, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    if (total == 0 && !d_yptr) return 0;
+    // rounds: consecutive columns, at most SPX_ROUND_PRODUCTS products (or one column) and 2^(64 - kb) columns each
+    const int kb = bits_for((uint64_t)std::max<int64_t>(max_inkey - 1, 0));
+    const int64_t maxcols = kb <= 1 ? INT64_MAX : int64_t(1) << (64 - kb);
+    std::vector<int64_t>& cut = w.h_cut;
+    cut.assign(1, 0);
+    int64_t maxn = 0;
+    for (int64_t c0 = 0, c1; c0 < ncol; c0 = c1) {
+        for (c1 = c0 + 1; c1 < ncol && c1 - c0 < maxcols && hc[c1 + 1] - hc[c0] <= SPX_ROUND_PRODUCTS; ++c1) {}
+        maxn = std::max(maxn, hc[c1] - hc[c0]);
+        cut.push_back(c1);
+    }
+    if (ncol == 0) cut.push_back(0);   // one round without columns: it writes y_ptr[0]
+    uint64_t* sk = w.sk.ensure((size_t)maxn);
+    uint32_t* perm = w.perm.ensure((size_t)maxn);
+    double* prod = w.prod.ensure((size_t)maxn);
+    int32_t* head = w.head.ensure((size_t)maxn);
+    int32_t* rank = w.rank.ensure((size_t)maxn);
+    int64_t* out_k = d_yv ? d_yk : nullptr;
+    for (size_t r = 0; r + 1 < cut.size(); ++r) {
+        const int64_t c0 = cut[r], nc = cut[r + 1] - c0, n = hc[c0 + nc] - hc[c0];
+        if (n == 0) {
+            if (d_yptr) DSA_LAUNCH("spmspv_ptr_fill", k_spx_ptr_fill, grid_for(nc + 1, 256), 256, 0, st, info, c0, nc, d_yptr);
+            continue;
+        }
+        DSA_LAUNCH("spmspv_emit", k_spx_emit, spx_piece_grid(nq), 256, 0, st, pma.keys.p, pma.vals.p, poff32, np, from, to, d_xv, nx, xcol,
+                   poff, blk, col_piece, c0, nc, kb, hc[c0], info, sk, perm, prod);
+        radix_sort_pairs(ws.sort, sk, perm, n, bits_for((uint64_t)(nc - 1)) + kb, st);
+        DSA_LAUNCH("flag_run_first", k_flag_run_first, grid_for(n, 256), 256, 0, st, sk, n, head);
+        exclusive_scan_i32<int32_t>(ws.batch.scan, head, rank, n, info + SPX_RUNS, st);
+        DSA_LAUNCH("spmspv_fold", k_spx_fold, grid_for(n, 256), 256, 0, st, sk, perm, prod, head, rank, n, info, cap, out_k, d_yv, kb, c0, nc,
+                   d_yptr);
+    }
+    if (total == 0) return 0;
+    DSA_CUDA(cudaMemcpyAsync(h + SPX_NOUT, info + SPX_NOUT, 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     DSA_CUDA(cudaStreamSynchronize(st));   // host synchronisation 2: the output count
-    return h[SPX_NOUT];
+    return h[SPX_NOUT] + h[SPX_RUNS];
 }
 
 inline void Pcsr::build_coo_d(PcsrWorkspace& ws, const int64_t* d_inkeys, const int64_t* d_partkeys, const double* d_vals, int64_t n,

@@ -145,6 +145,27 @@ int dsa_matrix_spmspv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const d
                       double* y_vals, int64_t cap, int64_t* count_out);
 int dsa_matrix_spmspv_d(dsa_matrix_t* A, int trans, const int64_t* d_x_keys, const double* d_x_vals, int64_t nx, int64_t* d_y_keys,
                         double* d_y_vals, int64_t cap, int64_t* count_out);
+/* k sparse right-hand sides in one call: Y = mat * X (trans = 0) or transpose(mat) * X (trans = 1), X in key space as CSC:
+ * x_ptr[k + 1] 0-based offsets, x_keys / x_vals[nnz_x], each column's keys strictly ascending (any Int64; descending across a
+ * column boundary is fine).  Column c of Y equals dsa_matrix_spmspv with X[:, c] bit for bit (same touched keys, stored zeros
+ * kept, same folds).  Y comes back in key space as CSC: y_ptr[k + 1] (0-based, empty columns included), y_keys ascending in
+ * each column, y_vals.  count_out (nnz of Y) is always set; a call with NULL outputs is a size query.
+ * DSA_ERR_ARGUMENT with nothing written: k < 0, nnz_x < 0, a NULL x_ptr, x_ptr[0] != 0, a decreasing x_ptr, x_ptr[k] != nnz_x,
+ * keys not strictly ascending inside a column, a column with more than 2^31 - 1 products, or more than 2^31 - 1 x entries +
+ * pieces (nnz_x + min(k, nnz_x) * capacity / 2048).  k == 0 writes y_ptr[0] = 0 and nothing else.
+ * Host variant: the outputs are written only when count <= cap: y_ptr when non-NULL, y_keys / y_vals when both are non-NULL.
+ * `_d` variant (device pointers; x_ptr and the key order are checked on the device): the columns are cut into rounds of at
+ * most 2^27 products (one column may exceed it alone) and 2^(64 - bits of the largest in-array key) columns, and every round
+ * writes straight into the caller's buffers.  So: d_y_ptr, when non-NULL, is written in full whatever cap; d_y_keys / d_y_vals
+ * (both non-NULL) receive a round only when the outputs through that round fit cap.  Nothing is ever written at or beyond
+ * cap, Y is complete when count <= cap, and the first cap entries are unspecified when count > cap.
+ * Device workspace: 40 B per product of the largest round (+ 16 B per output entry, at most cap, for the host variant),
+ * 36 B per x entry, 12 B per piece and 16 B per column.  Host synchronisations: two (the column product counts and the
+ * output count; one when X selects no stored cell); the host variant adds one for its copies. */
+int dsa_matrix_spmspm(dsa_matrix_t* A, int trans, const int64_t* x_ptr, const int64_t* x_keys, const double* x_vals, int64_t k,
+                      int64_t nnz_x, int64_t* y_ptr, int64_t* y_keys, double* y_vals, int64_t cap, int64_t* count_out);
+int dsa_matrix_spmspm_d(dsa_matrix_t* A, int trans, const int64_t* d_x_ptr, const int64_t* d_x_keys, const double* d_x_vals, int64_t k,
+                        int64_t nnz_x, int64_t* d_y_ptr, int64_t* d_y_keys, double* d_y_vals, int64_t cap, int64_t* count_out);
 /* dense-x variant: x_j = x[j-1] for j in 1..nx (every entry stored); y[i-1] for i in 1..ny, 0.0 where no entry */
 int dsa_matrix_spmv_dense(dsa_matrix_t* A, int trans, const double* x, int64_t nx, double* y, int64_t ny);
 int dsa_matrix_spmv_dense_d(dsa_matrix_t* A, int trans, const double* d_x, int64_t nx, double* d_y, int64_t ny);

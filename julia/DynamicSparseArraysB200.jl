@@ -323,6 +323,28 @@ end
 spmspv(A::DynamicSparseMatrix, v::VecLike) = _spmspv(A, false, _xs(v)..., size(A, 1))                     # operations.jl:14-24
 spmspv(t::Transposed, v::VecLike) = _spmspv(t.array, true, _xs(v)..., size(t.array, 2))                   # operations.jl:26-36
 
+# k sparse right-hand sides in one call: column c of the result equals spmspv(A, X[:, c]) bit for bit.  X's row r is key r; the
+# library returns key-space CSC with 0-based pointers, shifted here to SparseMatrixCSC's 1-based ones.  A result key above n
+# (entries stored outside size(A)) throws a BoundsError.
+function _spmspm(A::DynamicSparseMatrix, trans::Bool, X::SparseMatrixCSC, n)
+    A.fillmode && error("Matrix is in fill mode")
+    flush!(A)
+    k = size(X, 2)
+    xp = Vector{Int64}(X.colptr) .- 1; xk = Vector{Int64}(rowvals(X)); xv = Vector{Float64}(nonzeros(X))
+    cnt = Ref{Int64}(0)
+    f(yp, yk, yv, cap) = ccall((:dsa_matrix_spmspm, libdsa), Cint,
+                               (Ptr{Cvoid}, Cint, Ptr{Int64}, Ptr{Int64}, Ptr{Float64}, Int64, Int64, Ptr{Int64}, Ptr{Int64},
+                                Ptr{Float64}, Int64, Ref{Int64}),
+                               A.h, trans ? 1 : 0, xp, xk, xv, k, length(xk), yp, yk, yv, cap, cnt)
+    _check(f(C_NULL, C_NULL, C_NULL, 0))                                                                  # size query: nnz
+    yp = Vector{Int64}(undef, k + 1); yk = Vector{Int64}(undef, cnt[]); yv = Vector{Float64}(undef, cnt[])
+    _check(f(yp, yk, yv, length(yk)))
+    isempty(yk) || maximum(yk) <= n || throw(BoundsError(A, maximum(yk)))
+    return SparseMatrixCSC(n, k, yp .+ 1, yk, yv)
+end
+spmspv(A::DynamicSparseMatrix, X::SparseMatrixCSC) = _spmspm(A, false, X, size(A, 1))                     # size (size(A, 1), k)
+spmspv(t::Transposed, X::SparseMatrixCSC) = _spmspm(t.array, true, X, size(t.array, 2))                   # size (size(A, 2), k)
+
 # k dense right-hand sides in one call (one pass over the matrix per 32 columns); column c of the result equals the product
 # with X[:, c] bit for bit.  The library takes row-major buffers: permutedims turns the column-major X into one (ldx = k).
 function _mul_dense(A::DynamicSparseMatrix, trans::Bool, X::Matrix{Float64})
