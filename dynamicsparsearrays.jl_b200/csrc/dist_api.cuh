@@ -322,9 +322,9 @@ static void dist_spmv(dsa_dmatrix* D, int trans, const double* d_x, int64_t nx, 
     double* slice = yb + (size_t)d->rank * per;
     DSA_CUDA(cudaMemsetAsync(slice, 0, (size_t)per * 8, st));
     Pcsr& Pm = trans ? A->colmajor : A->rowmajor;
-    // the epilogue (carry fix-up + scatter by key) writes this rank's slice straight into the gather buffer
-    if (hi > lo) Pm.spmv_dense(A->ws, d_x, nx, slice, lo, hi, st);
-    else matrix_spmv_slots(A, trans, d_x, nullptr, nx);
+    // the epilogue (carry fix-up + scatter by key) writes this rank's slice straight into the gather buffer (nothing when the
+    // rank holds no keys: hi <= lo)
+    Pm.spmv_dense(A->ws, d_x, nx, slice, lo, hi, st);
     dist_all_gather(d, slice, yb, (size_t)per, ncclFloat64, st);
     if (ny <= 0) return;
     if (D->even[which]) {

@@ -99,9 +99,8 @@ static void phase1_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
         const int32_t* next_slot = P.nslots() == P.nlive() ? nullptr : P.d_next_slot.p;   // no tombstones: the next slot is s + 1
         // grid-stride over two waves of resident CTAs (6 per SM): 0.449 ms per config-2 step against 0.453 with 16 per SM, 0.464 with 32
         const unsigned assign_grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((c.n + 255) / 256, 148 * 12));
-        DSA_LAUNCH("tile_assign", k_tile_assign, assign_grid, 256, 0, st, c.partkeys, c.inkeys, c.vals, c.n, c.n_dev, P.d_live_keys.p,
-                   P.d_live_slot.p, P.nlive(), P.keymap(), P.keymap_min, P.keymap_len, P.pma.keys.p, P.pma.g.capacity, P.d_sem.p, next_slot,
-                   P.nslots(), cs, blk + 2 * CS_WORDS, rec);
+        DSA_LAUNCH("tile_assign", k_tile_assign, assign_grid, 256, 0, st, c.partkeys, c.inkeys, c.vals, c.n, c.n_dev, P.colmap(),
+                   P.pma.keys.p, P.pma.g.capacity, P.d_sem.p, next_slot, P.nslots(), cs, blk + 2 * CS_WORDS, rec);
         DSA_CUDA(cudaMemcpyAsync(hcs, cs, CS_WORDS * 8, cudaMemcpyDeviceToHost, st));
         return;
     }
@@ -113,8 +112,8 @@ static void phase1_launch(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
     int32_t* bcnt = blk + 2 * CS_WORDS;
     int32_t* lidx = ws.lidx.ensure((size_t)c.n);
     DSA_CUDA(cudaMemsetAsync(blk, 0, ((size_t)ns + 1 + 2 * CS_WORDS) * 4, st));
-    DSA_LAUNCH("col_lookup", k_col_lookup, lookup_grid(c.n), 256, 0, st, c.partkeys, c.inkeys, c.vals, c.n, c.n_dev, P.d_live_keys.p,
-               P.d_live_slot.p, P.nlive(), P.keymap(), P.keymap_min, P.keymap_len, op_slot, cs, bcnt, lidx);
+    DSA_LAUNCH("col_lookup", k_col_lookup, lookup_grid(c.n), 256, 0, st, c.partkeys, c.inkeys, c.vals, c.n, c.n_dev, P.colmap(), op_slot,
+               cs, bcnt, lidx);
     DSA_CUDA(cudaMemcpyAsync(hcs, cs, CS_WORDS * 8, cudaMemcpyDeviceToHost, st));
 }
 
@@ -209,8 +208,7 @@ static void phase1_finish(Pcsr& P, PcsrWorkspace& ws, BatchCtx& c, cudaStream_t 
         // slots changed: look every op up again
         int64_t* cs = ws.cs.ensure(CS_WORDS);   // statistics were already taken
         DSA_LAUNCH("col_lookup", k_col_lookup, lookup_grid(n), 256, 0, st, c.partkeys, (const int64_t*)nullptr, (const double*)nullptr, n,
-                   (const int64_t*)nullptr, P.d_live_keys.p, P.d_live_slot.p, P.nlive(), P.keymap(), P.keymap_min, P.keymap_len, ws.op_slot.p, cs,
-                   (int32_t*)nullptr, (int32_t*)nullptr);
+                   (const int64_t*)nullptr, P.colmap(), ws.op_slot.p, cs, (int32_t*)nullptr, (int32_t*)nullptr);
     }
 }
 
@@ -603,13 +601,6 @@ static void matrix_delete(dsa_matrix* A, bool rows, const int64_t* ids, int64_t 
     primary.delete_slots(A->ws, slots, d_slots, st);   // deletecolumn!(colmajor, col)  (matrix.jl:100)
 }
 
-static void matrix_spmv_slots(dsa_matrix* A, int trans, const double* d_x, const uint8_t* d_mask, int64_t nx) {
-    // mat * x sums, per row, over ascending columns (operations.jl:97-103): that is a segmented reduction over the
-    // ROW-major twin; transpose(mat) * x is the same over the column-major structure.
-    Pcsr& P = trans ? A->colmajor : A->rowmajor;
-    P.spmv_slots(A->ws, d_x, d_mask, nx, A->sh.st);
-}
-
 extern "C" {
 
 int dsa_version(void) { return 100; }
@@ -981,6 +972,8 @@ int dsa_matrix_spmv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const dou
                     int64_t cap, int64_t* count_out) {
     DSA_TRY
     cudaStream_t st = A->sh.st;
+    // mat * x sums, per row, over ascending columns (operations.jl:97-103): that is a segmented reduction over the
+    // ROW-major twin; transpose(mat) * x is the same over the column-major structure.
     Pcsr& P = trans ? A->colmajor : A->rowmajor;
     *count_out = 0;
     const int64_t dim = std::max<int64_t>(P.max_inkey, 1);
@@ -1004,7 +997,7 @@ int dsa_matrix_spmv(dsa_matrix_t* A, int trans, const int64_t* x_keys, const dou
             double* dv = h2d(A->stg.v, x_vals, nx, st);
             DSA_LAUNCH("scatter_x", k_scatter_x, grid_for(nx, 256), 256, 0, st, dk, dv, nx, xd, xm, dim);
         }
-        matrix_spmv_slots(A, trans, xd, xm, dim);
+        P.spmv_slots(A->ws, xd, xm, dim, st);
     }
     const int64_t ns = P.nslots();
     if (ns == 0) return DSA_OK;

@@ -2,6 +2,7 @@
 // bulk deletecolumn! (K5), column gather and the flat SpMV (K7).
 #pragma once
 #include <algorithm>
+#include <type_traits>
 #include <unordered_set>
 #include "pma.cuh"
 #include "sort.cuh"
@@ -24,24 +25,46 @@ __host__ __device__ __forceinline__ int64_t cs_min_decode(int64_t stored) { retu
 // grid of the (grid-stride) column lookup: one op per thread up to 16 CTAs per SM of a 148-SM part, then strided
 inline unsigned lookup_grid(int64_t n) { return (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, 148 * 16)); }
 
-__device__ __forceinline__ int32_t live_lookup(const int64_t* __restrict__ live_keys, const int32_t* __restrict__ live_slot,
-                                               int64_t nlive, int64_t key) {
-    int64_t lo = 0, hi = nlive;
+// index of the first a[i] >= key in the ascending a[0, n) (n if there is none)
+template <typename T>
+__device__ __forceinline__ int64_t lower_bound(const T* a, int64_t n, int64_t key) {
+    int64_t lo = 0, hi = n;
     while (lo < hi) {
         const int64_t mid = (lo + hi) >> 1;
-        if (live_keys[mid] < key) lo = mid + 1;
+        if (a[mid] < key) lo = mid + 1;
         else hi = mid;
     }
-    return (lo < nlive && live_keys[lo] == key) ? live_slot[lo] : -1;
+    return lo;
 }
+
+// The column map of an orientation as the kernels read it (Pcsr::colmap): partition key -> slot through the direct-address
+// table when there is one (keymap != nullptr), else by binary search over the sorted live keys.  Which of the two a map has is
+// decided by Pcsr::rebuild_live_and_upload.
+struct ColMap {
+    const int64_t* live_keys;   // ascending
+    const int32_t* live_slot;
+    int64_t nlive;
+    const int32_t* keymap;      // nullable: keymap[key - keymap_min] = slot or -1
+    int64_t keymap_min, keymap_len;
+
+    // slot of the live partition with this key, -1 if there is none
+    __device__ __forceinline__ int32_t slot(int64_t key) const {
+        if (keymap) {
+            const uint64_t r = (uint64_t)key - (uint64_t)keymap_min;   // any Int64 key: no signed overflow
+            return r < (uint64_t)keymap_len ? keymap[r] : -1;
+        }
+        const int64_t i = lower_rank(key);
+        return (i < nlive && live_keys[i] == key) ? live_slot[i] : -1;
+    }
+    // index of the first live key >= key (nlive if there is none)
+    __device__ __forceinline__ int64_t lower_rank(int64_t key) const { return lower_bound(live_keys, nlive, key); }
+};
 
 // Grid-stride: the launch is sized from an upper bound when the op count only exists on the device (n_dev, distributed batches:
 // the receive counts of the exchange are never read by the host before this kernel runs); cs[CS_N] reports the count used.
 __global__ void __launch_bounds__(256, 6) k_col_lookup(const int64_t* __restrict__ partkeys, const int64_t* __restrict__ inkeys,
                                                      const double* __restrict__ vals, int64_t n_host, const int64_t* __restrict__ n_dev,
-                                                     const int64_t* __restrict__ live_keys, const int32_t* __restrict__ live_slot,
-                                                     int64_t nlive, const int32_t* __restrict__ keymap, int64_t keymap_min,
-                                                     int64_t keymap_len, int32_t* __restrict__ op_slot, int64_t* __restrict__ cs,
+                                                     const ColMap cm, int32_t* __restrict__ op_slot, int64_t* __restrict__ cs,
                                                      int32_t* __restrict__ bcnt, int32_t* __restrict__ lidx) {
     int64_t n = n_host;
     if (n_dev) n = *n_dev < n_host ? *n_dev : n_host;
@@ -52,13 +75,7 @@ __global__ void __launch_bounds__(256, 6) k_col_lookup(const int64_t* __restrict
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t pk = partkeys[i];
         minp = pk < minp ? pk : minp;
-        int32_t s;
-        if (keymap) {   // dense key range: direct-address table (one load instead of a binary search)
-            const int64_t r = pk - keymap_min;
-            s = (r >= 0 && r < keymap_len) ? keymap[r] : -1;
-        } else {
-            s = live_lookup(live_keys, live_slot, nlive, pk);
-        }
+        const int32_t s = cm.slot(pk);
         op_slot[i] = s;
         miss += s < 0;
         if (bcnt && s >= 0) {   // bucket-sort bookkeeping: arrival-independent local index inside the partition's bucket
@@ -417,6 +434,29 @@ __device__ __forceinline__ longlong2 ldg_stream2(const longlong2* p, uint64_t po
     return r;
 }
 
+// A lane's C contiguous cells [p0, p0 + C) of the gapped arrays: 256-bit evict-first loads of keys and of values, cells at or
+// past cap read as gaps.  vals = nullptr: keys only (t is not written).
+template <int C, typename V>
+__device__ __forceinline__ void load_cells(const int64_t* keys, V vals, int64_t cap, int64_t p0, int64_t (&k)[C], double (&t)[C],
+                                           uint64_t pol) {
+    static_assert(C % 4 == 0, "a lane loads its cells in groups of 4 (256 bits)");
+    constexpr bool VALS = !std::is_same<V, std::nullptr_t>::value;
+#pragma unroll
+    for (int c = 0; c < C; c += 4) {
+        if (p0 + c + 4 <= cap) {
+            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], pol);
+            if constexpr (VALS) ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], pol);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+                const int64_t p = p0 + c + e;
+                k[c + e] = p < cap ? keys[p] : GAP_KEY;
+                if constexpr (VALS) t[c + e] = p < cap ? vals[p] : 0.0;
+            }
+        }
+    }
+}
+
 // XMODE: 0 = dense x (x[key - 1], every entry stored); 1 = dense x + presence mask (a sparse x scattered into a dense buffer);
 // 2 = sparse x looked up by binary search in its ascending key list (xkeys[nx], x = the matching values): for key spaces far
 // larger than the number of entries (ids around 1e10 through a key codec), where a dense buffer would not fit.
@@ -427,7 +467,6 @@ __global__ void __launch_bounds__(256) k_spmv_blocked(const int64_t* __restrict_
                                                        double* __restrict__ yslot, int32_t* __restrict__ ycnt,
                                                        double* __restrict__ carry, int32_t* __restrict__ carry_cnt,
                                                        int32_t* __restrict__ chunk_last_slot, int64_t nchunks) {
-    static_assert(C % 4 == 0, "a lane loads its cells in groups of 4 (256 bits)");
     const int64_t chunk = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (chunk >= nchunks) return;
@@ -436,20 +475,7 @@ __global__ void __launch_bounds__(256) k_spmv_blocked(const int64_t* __restrict_
     const int64_t p0 = chunk * (32 * C) + (int64_t)lane * C;
     int64_t k[C];
     double t[C];
-#pragma unroll
-    for (int c = 0; c < C; c += 4) {
-        if (p0 + c + 4 <= cap) {
-            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], l2pol);
-            ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], l2pol);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const int64_t p = p0 + c + e;
-                k[c + e] = p < cap ? keys[p] : GAP_KEY;
-                t[c + e] = p < cap ? vals[p] : 0.0;
-            }
-        }
-    }
+    load_cells(keys, vals, cap, p0, k, t, l2pol);
     // the C gathers of x: independent, branch-free, all in flight together.  t = x[key] * value (separate rounding,
     // operations.jl:101); heads keep their value (the partition id) in t
     double xv[C];
@@ -476,12 +502,7 @@ __global__ void __launch_bounds__(256) k_spmv_blocked(const int64_t* __restrict_
             const int64_t kk = k[c];
             xm[c] = 0;
             if (kk > 0) {
-                int64_t lo = 0, hi = nx;
-                while (lo < hi) {
-                    const int64_t mid = (lo + hi) >> 1;
-                    if (__ldg(xkeys + mid) < kk) lo = mid + 1;
-                    else hi = mid;
-                }
+                const int64_t lo = lower_bound(xkeys, nx, kk);
                 if (lo < nx && __ldg(xkeys + lo) == kk) {
                     xm[c] = 1;
                     xv[c] = __ldg(x + lo);
@@ -570,8 +591,21 @@ __global__ void __launch_bounds__(256) k_spmv_blocked(const int64_t* __restrict_
     }
 }
 
-// chunk c with a head: y[last partition of c] += carry[c+1] + carry[c+2] + ... up to and including the first chunk that has a head
-template <bool COUNTS>
+// The carry walk that completes the partition open at the end of chunk c: a + carry[c + 1] + carry[c + 2] + ..., in chunk order,
+// up to and including the first chunk that has a head.  Column col's carries lie at carry[chunk * W + col].  cnt (nullable): the
+// product counts carry_cnt of the same chunks are added to *cnt.
+__device__ __forceinline__ double add_following_carries(double a, const double* __restrict__ carry, const int32_t* __restrict__ chunk_last_slot,
+                                                        int64_t c, int64_t nchunks, int64_t W, int64_t col,
+                                                        const int32_t* __restrict__ carry_cnt = nullptr, int32_t* cnt = nullptr) {
+    for (int64_t d = c + 1; d < nchunks; ++d) {
+        a = __dadd_rn(a, carry[d * W + col]);
+        if (cnt) *cnt += carry_cnt[d];
+        if (chunk_last_slot[d] >= 0) break;
+    }
+    return a;
+}
+
+// sparse output: per chunk c with a head, the last partition of c is completed by the carry walk, product counts included
 __global__ void __launch_bounds__(256) k_spmv_fixup(double* __restrict__ yslot, int32_t* __restrict__ ycnt, const double* __restrict__ carry,
                                                      const int32_t* __restrict__ carry_cnt, const int32_t* __restrict__ chunk_last_slot,
                                                      int64_t nchunks) {
@@ -581,45 +615,15 @@ __global__ void __launch_bounds__(256) k_spmv_fixup(double* __restrict__ yslot, 
     if (slot < 0) return;
     if (c + 1 >= nchunks) return;
     double a = yslot[slot];
-    int32_t n = COUNTS ? ycnt[slot] : 0;
-    for (int64_t d = c + 1; d < nchunks; ++d) {
-        a = __dadd_rn(a, carry[d]);
-        if (COUNTS) n += carry_cnt[d];
-        if (chunk_last_slot[d] >= 0) break;
-    }
+    int32_t n = ycnt[slot];
+    a = add_following_carries(a, carry, chunk_last_slot, c, nchunks, 1, 0, carry_cnt, &n);
     yslot[slot] = a;
-    if (COUNTS) ycnt[slot] = n;
-}
-
-
-// Dense-output epilogue in ONE kernel, driven by slot: the carry fix-up of k_spmv_fixup (same additions in the same order: the
-// partition that is open at the end of its chunk adds the carries of the following chunks up to and including the first one
-// with a head) and the scatter of y by partition key.  A slot is the last head of its chunk iff its span reaches the chunk's end.
-__global__ void __launch_bounds__(256) k_spmv_fix_to_dense(const double* __restrict__ yslot, const double* __restrict__ carry,
-                                                            const int32_t* __restrict__ chunk_last_slot, const int64_t* __restrict__ sem,
-                                                            const int32_t* __restrict__ next_slot, const int64_t* __restrict__ slot_key,
-                                                            int64_t nslots, int64_t cap, int64_t nchunks, int lg_chunk,
-                                                            double* __restrict__ y, int64_t key_lo, int64_t key_hi) {
-    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= nslots) return;
-    const int64_t ps = sem[s];
-    if (ps < 0) return;
-    const int64_t k = slot_key[s];
-    if (k < key_lo || k >= key_hi) return;   // y holds the partition keys [key_lo, key_hi)
-    double a = yslot[s];
-    const int64_t c0 = ps >> lg_chunk;
-    if (span_end(sem, next_slot, (int32_t)s, cap) >= ((c0 + 1) << lg_chunk)) {
-        for (int64_t d = c0 + 1; d < nchunks; ++d) {
-            a = __dadd_rn(a, carry[d]);
-            if (chunk_last_slot[d] >= 0) break;
-        }
-    }
-    y[k - key_lo] = a;
+    ycnt[slot] = n;
 }
 
 // ---------------------------------------------------------------------------------------------
 // K7b multi-vector product Y = A * X over the gapped array, for one pass of 4 * ngroups columns of a row-major X (row stride
-// ldx % 4 == 0, 32-byte aligned base).  Bit for bit, column c is k_spmv_blocked<0, C> + k_spmv_fix_to_dense on column c alone:
+// ldx % 4 == 0, 32-byte aligned base).  Bit for bit, column c is k_spmv_blocked<0, C> + the epilogue (W = 1) on column c alone:
 // the same 32 * C-cell chunk per warp, the same C contiguous cells per lane summed sequentially, the same segmented scan over
 // the lane aggregates (same shuffle order), the same carries added in chunk order by the epilogue, mul and add rounded
 // separately.  What is shared: the keys / values are streamed once for all columns, and a cell's x becomes one 256-bit load of
@@ -636,7 +640,6 @@ __global__ void __launch_bounds__(256) k_spmm_blocked(const int64_t* __restrict_
                                                        const double* __restrict__ X, int64_t nx, int64_t ldx, int ngroups,
                                                        double* __restrict__ yslot, double* __restrict__ carry,
                                                        int32_t* __restrict__ chunk_last_slot, int64_t nchunks) {
-    static_assert(C % 4 == 0, "a lane loads its cells in groups of 4 (256 bits)");
     const int64_t chunk = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (chunk >= nchunks) return;
@@ -645,20 +648,7 @@ __global__ void __launch_bounds__(256) k_spmm_blocked(const int64_t* __restrict_
     const int64_t p0 = chunk * (32 * C) + (int64_t)lane * C;
     int64_t k[C];
     double t[C];
-#pragma unroll
-    for (int c = 0; c < C; c += 4) {
-        if (p0 + c + 4 <= cap) {
-            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], l2pol);
-            ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], l2pol);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const int64_t p = p0 + c + e;
-                k[c + e] = p < cap ? keys[p] : GAP_KEY;
-                t[c + e] = p < cap ? vals[p] : 0.0;
-            }
-        }
-    }
+    load_cells(keys, vals, cap, p0, k, t, l2pol);
     // the segment structure of the chunk is the same for every column
     bool has_head = false;
     int32_t lastslot = -1;
@@ -744,12 +734,20 @@ __global__ void __launch_bounds__(256) k_spmm_blocked(const int64_t* __restrict_
     }
 }
 
-// k_spmv_fix_to_dense per column: thread (slot, col) of one pass; Y[(key - key_lo) * ldy + col] for col < ncols
+// Dense-output epilogue of the products in ONE kernel, driven by slot: thread (slot, col) of a pass of W columns completes the
+// slot's partial with the carry walk (the additions of k_spmv_fixup, in the same order) and scatters it by partition key to
+// Y[(key - key_lo) * ldy + col] for col < ncols.  A slot is the last head of its chunk iff its span reaches the chunk's end.
+// ONE: the single-vector product, W = ncols = ldy = 1 as constants (no division, no column arithmetic).
+template <bool ONE>
 __global__ void __launch_bounds__(256) k_spmm_fix_to_dense(const double* __restrict__ yslot, const double* __restrict__ carry,
                                                             const int32_t* __restrict__ chunk_last_slot, const int64_t* __restrict__ sem,
                                                             const int32_t* __restrict__ next_slot, const int64_t* __restrict__ slot_key,
                                                             int64_t nslots, int64_t cap, int64_t nchunks, int lg_chunk, int W, int ncols,
                                                             double* __restrict__ Y, int64_t ldy, int64_t key_lo, int64_t key_hi) {
+    if (ONE) {
+        W = ncols = 1;
+        ldy = 1;
+    }
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t s = i / W;
     const int col = (int)(i - s * W);
@@ -757,15 +755,11 @@ __global__ void __launch_bounds__(256) k_spmm_fix_to_dense(const double* __restr
     const int64_t ps = sem[s];
     if (ps < 0) return;
     const int64_t k = slot_key[s];
-    if (k < key_lo || k >= key_hi) return;
+    if (k < key_lo || k >= key_hi) return;   // Y holds the partition keys [key_lo, key_hi)
     double a = yslot[s * W + col];
     const int64_t c0 = ps >> lg_chunk;
-    if (span_end(sem, next_slot, (int32_t)s, cap) >= ((c0 + 1) << lg_chunk)) {
-        for (int64_t d = c0 + 1; d < nchunks; ++d) {
-            a = __dadd_rn(a, carry[d * W + col]);
-            if (chunk_last_slot[d] >= 0) break;
-        }
-    }
+    if (span_end(sem, next_slot, (int32_t)s, cap) >= ((c0 + 1) << lg_chunk))
+        a = add_following_carries(a, carry, chunk_last_slot, c0, nchunks, W, col);
     Y[(k - key_lo) * ldy + col] = a;
 }
 
@@ -821,16 +815,14 @@ static_assert(CMP_SCAN_THREADS * CMP_SCAN_ITEMS == 1 << CMP_LG_SCAN_BLOCK, "scan
 template <bool SEMS>
 __device__ __forceinline__ bool cmp_elem(int64_t k) { return SEMS ? k > 0 : k != GAP_KEY; }
 
-__device__ __forceinline__ void cmp_load_keys(const int64_t* keys, int64_t cap, int64_t p0, int64_t (&k)[CMP_C], uint64_t pol) {
+// Warp-collective, every lane gets it: the sum of the scan-block totals blk_sum[0 .. q >> CMP_LG_SCAN_BLOCK), which turns item
+// q's offset inside its scan block (k_compress_scan) into its global offset.  lane: the caller's threadIdx.x & 31.
+__device__ __forceinline__ int64_t scan_block_base(const int64_t* __restrict__ blk_sum, int64_t q, int lane) {
+    int64_t a = 0;
+    for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
 #pragma unroll
-    for (int c = 0; c < CMP_C; c += 4) {
-        if (p0 + c + 4 <= cap) {
-            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], pol);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) k[c + e] = p0 + c + e < cap ? keys[p0 + c + e] : GAP_KEY;
-        }
-    }
+    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    return a;
 }
 
 // bound_flag (nullable): set when an element lies at or after position sem[bound_slot] (bound_slot = the first live partition
@@ -844,7 +836,8 @@ __global__ void __launch_bounds__(256) k_compress_count(const int64_t* __restric
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int64_t p0 = (int64_t)blockIdx.x * CMP_TILE + (int64_t)wid * (32 * CMP_C) + (int64_t)lane * CMP_C;
     int64_t k[CMP_C];
-    cmp_load_keys(keys, cap, p0, k, l2_evict_first_policy());
+    double unused[CMP_C];   // keys only
+    load_cells(keys, nullptr, cap, p0, k, unused, l2_evict_first_policy());
     int cnt = 0;
 #pragma unroll
     for (int c = 0; c < CMP_C; ++c) cnt += cmp_elem<SEMS>(k[c]) ? 1 : 0;
@@ -923,20 +916,7 @@ __global__ void __launch_bounds__(256) k_compress_emit(const int64_t* __restrict
     const uint64_t pol = l2_evict_first_policy();
     int64_t k[CMP_C];
     double t[CMP_C];
-#pragma unroll
-    for (int c = 0; c < CMP_C; c += 4) {
-        if (p0 + c + 4 <= cap) {
-            ldg_stream4(keys + p0 + c, k[c], k[c + 1], k[c + 2], k[c + 3], pol);
-            ldg_stream4(vals + p0 + c, t[c], t[c + 1], t[c + 2], t[c + 3], pol);
-        } else {
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const int64_t p = p0 + c + e;
-                k[c + e] = p < cap ? keys[p] : GAP_KEY;
-                t[c + e] = p < cap ? vals[p] : 0.0;
-            }
-        }
-    }
+    load_cells(keys, vals, cap, p0, k, t, pol);
     int cnt = 0;
 #pragma unroll
     for (int c = 0; c < CMP_C; ++c) cnt += cmp_elem<SEMS>(k[c]) ? 1 : 0;
@@ -949,11 +929,7 @@ __global__ void __launch_bounds__(256) k_compress_emit(const int64_t* __restrict
     const int wtot = __shfl_sync(0xffffffffu, incl, 31);
     if (lane == 0) wc[wid] = wtot;
     if (wid == 0) {   // tile offset = offset inside its scan block + totals of the scan blocks before it
-        const int64_t nb = tile >> CMP_LG_SCAN_BLOCK;
-        int64_t a = 0;
-        for (int64_t b = lane; b < nb; b += 32) a += blk_sum[b];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+        const int64_t a = scan_block_base(blk_sum, tile, lane);
         if (lane == 0) s_toff = tile_off[tile] + a;
     }
     __syncthreads();
@@ -994,30 +970,14 @@ __global__ void __launch_bounds__(256) k_compress_live_rank(const int32_t* __res
 
 // dense pointer over partition keys 1..dim: out[k] = base + ptr[first live partition with key >= k + 1] for k = 0..dim (the
 // entries of key k end where the next present key starts); a present key is one load of the direct-address map, others (and
-// handles without the map) a binary search over the sorted live keys
-__global__ void __launch_bounds__(256) k_compress_dense_ptr(const int64_t* __restrict__ ptr, const int64_t* __restrict__ live_keys,
-                                                             const int32_t* __restrict__ live_rank, int64_t nlive,
-                                                             const int32_t* __restrict__ keymap, int64_t keymap_min, int64_t keymap_len,
+// maps without the table, whose slot lookup is the same binary search) the binary search over the sorted live keys
+__global__ void __launch_bounds__(256) k_compress_dense_ptr(const int64_t* __restrict__ ptr, const ColMap cm, const int32_t* __restrict__ live_rank,
                                                              int64_t dim, int64_t base, int64_t* __restrict__ out) {
     const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k > dim) return;
     const int64_t key = k + 1;
-    int64_t i = -1;
-    if (keymap) {
-        const int64_t m = key - keymap_min;
-        const int32_t s = (m >= 0 && m < keymap_len) ? keymap[m] : -1;
-        if (s >= 0) i = live_rank[s];
-    }
-    if (i < 0) {
-        int64_t lo = 0, hi = nlive;
-        while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (live_keys[mid] < key) lo = mid + 1;
-            else hi = mid;
-        }
-        i = lo;
-    }
-    out[k] = base + ptr[i];
+    const int32_t s = cm.keymap ? cm.slot(key) : -1;
+    out[k] = base + ptr[s >= 0 ? live_rank[s] : cm.lower_rank(key)];
 }
 
 struct CompressWorkspace {
@@ -1095,9 +1055,7 @@ inline unsigned spx_piece_grid(int64_t npieces) { return (unsigned)std::max<int6
 
 // xptr == nullptr: one column holding all nx entries (xcol not written)
 __global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ xk, int64_t nx, const int64_t* __restrict__ xptr,
-                                                     int64_t ncol, const int64_t* __restrict__ live_keys,
-                                                     const int32_t* __restrict__ live_slot, int64_t nlive, const int32_t* __restrict__ keymap,
-                                                     int64_t keymap_min, int64_t keymap_len, const int64_t* __restrict__ sem,
+                                                     int64_t ncol, const ColMap cm, const int64_t* __restrict__ sem,
                                                      const int32_t* __restrict__ next_slot, int64_t cap, int64_t* __restrict__ span_from,
                                                      int64_t* __restrict__ span_to, int32_t* __restrict__ npieces, int64_t* __restrict__ xcol,
                                                      int64_t* __restrict__ info) {
@@ -1106,24 +1064,13 @@ __global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ 
     const int64_t key = xk[i];
     int64_t first = 0;
     if (xptr) {   // the last column c with xptr[c] <= i (a malformed x_ptr gives some c in [0, ncol): k_spx_cols refuses it)
-        int64_t lo = 0, hi = ncol;
-        while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (xptr[mid] <= i) lo = mid + 1;
-            else hi = mid;
-        }
+        const int64_t lo = lower_bound(xptr, ncol, i + 1);
         const int64_t c = lo > 0 ? lo - 1 : 0;
         xcol[i] = c;
         first = xptr[c];
     }
     if (i > first && xk[i - 1] >= key) info[SPX_ERR] = 1;
-    int32_t s;
-    if (keymap) {
-        const uint64_t r = (uint64_t)key - (uint64_t)keymap_min;   // any Int64 key: no signed overflow
-        s = r < (uint64_t)keymap_len ? keymap[r] : -1;
-    } else {
-        s = live_lookup(live_keys, live_slot, nlive, key);
-    }
+    const int32_t s = cm.slot(key);
     int64_t from = 0, to = 0;
     if (s >= 0) {
         from = sem[s] + 1;
@@ -1138,13 +1085,7 @@ __global__ void __launch_bounds__(256) k_spx_locate(const int64_t* __restrict__ 
 __device__ __forceinline__ bool spx_piece(int64_t q, const int32_t* __restrict__ piece_off, const int32_t* __restrict__ npieces, int64_t nx,
                                           const int64_t* __restrict__ span_from, const int64_t* __restrict__ span_to, int64_t& i,
                                           int64_t& c0, int64_t& c1) {
-    int64_t lo = 0, hi = nx;   // last entry whose first piece is <= q
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (piece_off[mid] <= q) lo = mid + 1;
-        else hi = mid;
-    }
-    i = lo - 1;
+    i = lower_bound(piece_off, nx, q + 1) - 1;   // the last entry whose first piece is <= q
     if (i < 0) return false;
     const int64_t j = q - piece_off[i];
     if (j < 0 || j >= npieces[i]) return false;
@@ -1188,10 +1129,7 @@ __global__ void __launch_bounds__(256) k_spx_cols(const int64_t* __restrict__ xp
         e = min(max(e, (int64_t)0), nx);
     }
     const int64_t q = min(max(e < nx ? (int64_t)piece_off[e] : info[SPX_NPIECES], (int64_t)0), nq - 1);
-    int64_t a = 0;   // as k_spx_emit: offset inside its scan block + totals of the scan blocks before it
-    for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+    const int64_t a = scan_block_base(blk_sum, q, lane);
     if (lane == 0) {
         col_piece[c] = q;
         info[SPX_WORDS + c] = poff[q] + a;
@@ -1219,10 +1157,7 @@ __global__ void __launch_bounds__(256) k_spx_emit(const int64_t* __restrict__ ke
     for (int64_t q = col_piece[c0] + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); q < q1; q += nw) {
         int64_t i, cf, cl;
         if (!spx_piece(q, piece_off, npieces, nx, span_from, span_to, i, cf, cl)) continue;
-        int64_t a = 0;   // offset = offset inside its scan block + totals of the scan blocks before it
-        for (int64_t b = lane; b < (q >> CMP_LG_SCAN_BLOCK); b += 32) a += blk_sum[b];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+        const int64_t a = scan_block_base(blk_sum, q, lane);
         int64_t o = poff[q] + a - p0;
         const double x = xv[i];
         const uint64_t tag = xcol ? (uint64_t)(xcol[i] - c0) << kb : 0;
@@ -1352,7 +1287,9 @@ struct Pcsr {
     int tile_penalty = 0;       // batches to wait before the next tile-streamed attempt (after a refused one)
     int64_t last_batch_n = 0;   // ops of the previous batch (the host only has an upper bound of a distributed batch's size)
 
-    const int32_t* keymap() const { return keymap_len > 0 ? d_keymap.p : nullptr; }
+    ColMap colmap() const {
+        return ColMap{d_live_keys.p, d_live_slot.p, nlive(), keymap_len > 0 ? d_keymap.p : nullptr, keymap_min, keymap_len};
+    }
     int64_t nslots() const { return (int64_t)slot_key.size(); }
     int64_t nlive() const { return (int64_t)live_keys_h.size(); }
     int64_t nnz() const { return pma.nnz - nb_partitions; }   // pcsr.jl:11
@@ -1426,7 +1363,7 @@ struct Pcsr {
         int32_t* op_slot = ws.op_slot.ensure((size_t)n);
         int64_t* cs = ws.cs.ensure(CS_WORDS);   // statistics are not used by reads
         DSA_LAUNCH("col_lookup", k_col_lookup, lookup_grid(n), 256, 0, st, d_partkeys, (const int64_t*)nullptr, (const double*)nullptr, n,
-                   (const int64_t*)nullptr, d_live_keys.p, d_live_slot.p, nlive(), keymap(), keymap_min, keymap_len, op_slot, cs, (int32_t*)nullptr, (int32_t*)nullptr);
+                   (const int64_t*)nullptr, colmap(), op_slot, cs, (int32_t*)nullptr, (int32_t*)nullptr);
         DSA_LAUNCH("get", k_get, grid_for(n, 256), 256, 0, st, pma.keys.p, pma.vals.p, pma.g.capacity, op_slot, d_inkeys, n, d_sem.p,
                        d_next_slot.p, d_out);
     }
@@ -1466,51 +1403,44 @@ struct Pcsr {
         rebuild_live_and_upload(st);
     }
 
-    // Dense x: the product counts (only the sparse output needs them) are not computed.
-    // d_xkeys != nullptr: x = (d_xkeys, d_x)[nx] ascending, looked up by binary search (no dense buffer).
-    template <int C>
-    void spmv_launch_blocked(PcsrWorkspace& ws, const double* d_x, const uint8_t* d_xmask, int64_t nx, cudaStream_t st,
-                             const int64_t* d_xkeys = nullptr, bool fixup = true) {
-        const int64_t cap = pma.g.capacity;
-        const int64_t nchunks = (cap + 32 * C - 1) / (32 * C);
-        const int64_t ns = nslots();
+    // a warp's chunk = 32 lanes x 8 cells (two 256-bit loads of keys, two of values, 8 gathers of x in flight per lane):
+    // product call 71.5 -> 66.5 us at config 2 against 4 cells per lane; 16 cells per lane (114 registers): 83 us
+    static constexpr int SPMV_CELLS_PER_LANE = 8, SPMV_LG_CHUNK = 8;
+    static_assert(32 * SPMV_CELLS_PER_LANE == 1 << SPMV_LG_CHUNK, "a warp's chunk");
+    int64_t spmv_nchunks() const { return (pma.g.capacity + (1 << SPMV_LG_CHUNK) - 1) >> SPMV_LG_CHUNK; }
+
+    // The chunked reduction of mat * x (k_spmv_blocked): partials by slot in ws.yslot, carries in ws.carry / ws.chunk_last, and
+    // with a sparse x the product counts in ws.ycnt / ws.carry_cnt.  The caller launches the epilogue that adds the carries.
+    // x: dense (d_xmask == nullptr), sparse as a dense buffer with a presence mask, or d_xkeys != nullptr: sparse as
+    // (d_xkeys, d_x)[nx] with ascending keys, looked up by binary search (no dense buffer).
+    void spmv_reduce(PcsrWorkspace& ws, const double* d_x, const uint8_t* d_xmask, int64_t nx, cudaStream_t st, const int64_t* d_xkeys) {
+        constexpr int C = SPMV_CELLS_PER_LANE;
+        const int64_t cap = pma.g.capacity, nchunks = spmv_nchunks(), ns = nslots();
         double* yslot = ws.yslot.ensure((size_t)ns + 1);
         int32_t* ycnt = ws.ycnt.ensure((size_t)ns + 1);
         double* carry = ws.carry.ensure((size_t)nchunks);
         int32_t* ccnt = ws.carry_cnt.ensure((size_t)nchunks);
         int32_t* clast = ws.chunk_last.ensure((size_t)nchunks);
-        const unsigned gr = grid_for(nchunks * 32, 256);
-        if (d_xkeys) {
-            DSA_LAUNCH("spmv_blocked", (k_spmv_blocked<2, C>), gr, 256, 0, st, pma.keys.p, pma.vals.p, cap, d_x, d_xmask, d_xkeys, nx, yslot, ycnt,
-                       carry, ccnt, clast, nchunks);
-            DSA_LAUNCH("spmv_fixup", k_spmv_fixup<true>, grid_for(nchunks, 256), 256, 0, st, yslot, ycnt, carry, ccnt, clast, nchunks);
-        } else if (d_xmask) {
-            DSA_LAUNCH("spmv_blocked", (k_spmv_blocked<1, C>), gr, 256, 0, st, pma.keys.p, pma.vals.p, cap, d_x, d_xmask, d_xkeys, nx, yslot, ycnt,
-                       carry, ccnt, clast, nchunks);
-            DSA_LAUNCH("spmv_fixup", k_spmv_fixup<true>, grid_for(nchunks, 256), 256, 0, st, yslot, ycnt, carry, ccnt, clast, nchunks);
-        } else {
-            DSA_LAUNCH("spmv_blocked", (k_spmv_blocked<0, C>), gr, 256, 0, st, pma.keys.p, pma.vals.p, cap, d_x, d_xmask, d_xkeys, nx, yslot, ycnt,
-                       carry, ccnt, clast, nchunks);
-            if (fixup) DSA_LAUNCH("spmv_fixup", k_spmv_fixup<false>, grid_for(nchunks, 256), 256, 0, st, yslot, ycnt, carry, ccnt, clast, nchunks);
-        }
+        const auto kernel = d_xkeys ? k_spmv_blocked<2, C> : d_xmask ? k_spmv_blocked<1, C> : k_spmv_blocked<0, C>;
+        DSA_LAUNCH("spmv_blocked", kernel, grid_for(nchunks * 32, 256), 256, 0, st, pma.keys.p, pma.vals.p, cap, d_x, d_xmask, d_xkeys, nx,
+                   yslot, ycnt, carry, ccnt, clast, nchunks);
     }
-    // SpMV; results by slot in ws.yslot / ws.ycnt
-    // a warp's chunk = 32 lanes x 8 cells (two 256-bit loads of keys, two of values, 8 gathers of x in flight per lane):
-    // product call 71.5 -> 66.5 us at config 2 against 4 cells per lane; 16 cells per lane (114 registers): 83 us
-    static constexpr int SPMV_CELLS_PER_LANE = 8, SPMV_LG_CHUNK = 8;
+    // mat * sparse x (a presence mask, or d_xkeys: see spmv_reduce); results and product counts by slot in ws.yslot / ws.ycnt
     void spmv_slots(PcsrWorkspace& ws, const double* d_x, const uint8_t* d_xmask, int64_t nx, cudaStream_t st,
                     const int64_t* d_xkeys = nullptr) {
-        spmv_launch_blocked<SPMV_CELLS_PER_LANE>(ws, d_x, d_xmask, nx, st, d_xkeys);
+        spmv_reduce(ws, d_x, d_xmask, nx, st, d_xkeys);
+        const int64_t nchunks = spmv_nchunks();
+        DSA_LAUNCH("spmv_fixup", k_spmv_fixup, grid_for(nchunks, 256), 256, 0, st, ws.yslot.p, ws.ycnt.p, ws.carry.p, ws.carry_cnt.p,
+                   ws.chunk_last.p, nchunks);
     }
     // mat * dense x -> dense y over the partition keys [key_lo, key_hi) (y zeroed by the caller): reduction kernel + one
     // epilogue kernel (fix-up and scatter by key)
     void spmv_dense(PcsrWorkspace& ws, const double* d_x, int64_t nx, double* d_y, int64_t key_lo, int64_t key_hi, cudaStream_t st) {
-        spmv_launch_blocked<SPMV_CELLS_PER_LANE>(ws, d_x, nullptr, nx, st, nullptr, /*fixup=*/false);
-        const int64_t ns = nslots(), cap = pma.g.capacity;
-        const int64_t nchunks = (cap + (1 << SPMV_LG_CHUNK) - 1) >> SPMV_LG_CHUNK;
+        spmv_reduce(ws, d_x, nullptr, nx, st, nullptr);
+        const int64_t ns = nslots();
         if (ns > 0)
-            DSA_LAUNCH("spmv_fix_to_dense", k_spmv_fix_to_dense, grid_for(ns, 256), 256, 0, st, ws.yslot.p, ws.carry.p, ws.chunk_last.p, d_sem.p,
-                       d_next_slot.p, d_slot_key.p, ns, cap, nchunks, SPMV_LG_CHUNK, d_y, key_lo, key_hi);
+            DSA_LAUNCH("spmv_fix_to_dense", k_spmm_fix_to_dense<true>, grid_for(ns, 256), 256, 0, st, ws.yslot.p, ws.carry.p, ws.chunk_last.p, d_sem.p,
+                       d_next_slot.p, d_slot_key.p, ns, pma.g.capacity, spmv_nchunks(), SPMV_LG_CHUNK, 1, 1, d_y, (int64_t)1, key_lo, key_hi);
     }
 
     // mat * X -> Y for one pass of ncols (<= 4 * ngroups) columns, over the partition keys [key_lo, key_hi) (Y zeroed by the
@@ -1520,16 +1450,14 @@ struct Pcsr {
                          int64_t key_lo, int64_t key_hi, cudaStream_t st) {
         constexpr int C = SPMV_CELLS_PER_LANE;
         const int ngroups = (ncols + 3) / 4, W = 4 * ngroups;
-        const int64_t cap = pma.g.capacity, ns = nslots();
-        const int64_t nchunks = (cap + (1 << SPMV_LG_CHUNK) - 1) >> SPMV_LG_CHUNK;
-        static_assert(32 * C == 1 << SPMV_LG_CHUNK, "a warp's chunk");
+        const int64_t cap = pma.g.capacity, ns = nslots(), nchunks = spmv_nchunks();
         double* yslot = ws.yslot_mv.ensure((size_t)(ns + 1) * W);
         double* carry = ws.carry_mv.ensure((size_t)nchunks * W);
         int32_t* clast = ws.chunk_last.ensure((size_t)nchunks);
         DSA_LAUNCH("spmm_blocked", k_spmm_blocked<C>, grid_for(nchunks * 32, 256), 256, 0, st, pma.keys.p, pma.vals.p, cap, d_X, nx, ldx,
                    ngroups, yslot, carry, clast, nchunks);
         if (ns > 0)
-            DSA_LAUNCH("spmm_fix_to_dense", k_spmm_fix_to_dense, grid_for(ns * W, 256), 256, 0, st, yslot, carry, clast, d_sem.p,
+            DSA_LAUNCH("spmm_fix_to_dense", k_spmm_fix_to_dense<false>, grid_for(ns * W, 256), 256, 0, st, yslot, carry, clast, d_sem.p,
                        d_next_slot.p, d_slot_key.p, ns, cap, nchunks, SPMV_LG_CHUNK, W, ncols, d_Y, ldy, key_lo, key_hi);
     }
 
@@ -1564,8 +1492,7 @@ struct Pcsr {
         const int32_t* lr = compress_live_rank(ws, st);
         int64_t* sptr = ws.cmp.ptr.ensure((size_t)np + 1);
         compress_cells<true>(ws.cmp, pma.keys.p, pma.vals.p, pma.g.capacity, b, base - 1, lr, sptr, np, nnz(), d_ind, d_vals, st);
-        DSA_LAUNCH("compress_dense_ptr", k_compress_dense_ptr, grid_for(dim + 1, 256), 256, 0, st, sptr, d_live_keys.p, lr, np, keymap(),
-                   keymap_min, keymap_len, dim, base, d_ptr);
+        DSA_LAUNCH("compress_dense_ptr", k_compress_dense_ptr, grid_for(dim + 1, 256), 256, 0, st, sptr, colmap(), lr, dim, base, d_ptr);
     }
 
     // sparse-x product (K9): x = (d_xk, d_xv)[nx] with strictly ascending keys (DSA_ERR_ARGUMENT otherwise, nothing written);
@@ -1675,8 +1602,8 @@ inline int64_t Pcsr::spmspm(PcsrWorkspace& ws, const int64_t* d_xptr, const int6
     int64_t* blk = w.blk_sum.ensure((size_t)nblk);
     DSA_CUDA(cudaMemsetAsync(info, 0, SPX_WORDS * sizeof(int64_t), st));
     if (nx > 0)
-        DSA_LAUNCH("spmspv_locate", k_spx_locate, grid_for(nx, 256), 256, 0, st, d_xk, nx, d_xptr, ncol, d_live_keys.p, d_live_slot.p, nlive(),
-                   keymap(), keymap_min, keymap_len, d_sem.p, d_next_slot.p, pma.g.capacity, from, to, np, xcol, info);
+        DSA_LAUNCH("spmspv_locate", k_spx_locate, grid_for(nx, 256), 256, 0, st, d_xk, nx, d_xptr, ncol, colmap(), d_sem.p, d_next_slot.p,
+                   pma.g.capacity, from, to, np, xcol, info);
     exclusive_scan_i32<int32_t>(ws.batch.scan, np, poff32, nx, info + SPX_NPIECES, st);
     DSA_LAUNCH("spmspv_count", k_spx_count, spx_piece_grid(nq), 256, 0, st, pma.keys.p, poff32, np, nx, from, to, info, nq, pcnt);
     DSA_LAUNCH("spmspv_scan", k_compress_scan, (unsigned)nblk, CMP_SCAN_THREADS, 0, st, pcnt, nq, poff, blk);

@@ -30,9 +30,7 @@ namespace dsa {
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256, 6) k_tile_assign(const int64_t* __restrict__ partkeys, const int64_t* __restrict__ inkeys,
                                                         const double* __restrict__ vals, int64_t n_host, const int64_t* __restrict__ n_dev,
-                                                        const int64_t* __restrict__ live_keys, const int32_t* __restrict__ live_slot,
-                                                        int64_t nlive, const int32_t* __restrict__ keymap, int64_t keymap_min,
-                                                        int64_t keymap_len, const int64_t* __restrict__ keys, int64_t cap,
+                                                        const ColMap cm, const int64_t* __restrict__ keys, int64_t cap,
                                                         const int64_t* __restrict__ sem, const int32_t* __restrict__ next_slot,
                                                         int64_t nslots, int64_t* __restrict__ cs, int32_t* __restrict__ tcnt,
                                                         TileRec* __restrict__ rec) {
@@ -47,13 +45,7 @@ __global__ void __launch_bounds__(256, 6) k_tile_assign(const int64_t* __restric
         const int64_t k = inkeys[i];
         const double v = vals[i];
         minp = pk < minp ? pk : minp;
-        int32_t s;
-        if (keymap) {
-            const int64_t r = pk - keymap_min;
-            s = (r >= 0 && r < keymap_len) ? keymap[r] : -1;
-        } else {
-            s = live_lookup(live_keys, live_slot, nlive, pk);
-        }
+        const int32_t s = cm.slot(pk);
         mink = k < mink ? k : mink;
         maxk = k > maxk ? k : maxk;
         const bool is_set = v != 0.0;   // pcsr.jl:301

@@ -175,7 +175,7 @@ int main() {
             dsa::k_spmv_blocked<0, 8><<<(unsigned)(nch8 * 32 / 256), 256>>>(dk, dv, cap, dx, nullptr, nullptr, nx, yslot, ycnt, carry, ccnt, clast, nch8); });
         timeit("product k_spmv_blocked<false,4> + fixup", [&] {
             dsa::k_spmv_blocked<0, 4><<<(unsigned)(nch4 * 32 / 256), 256>>>(dk, dv, cap, dx, nullptr, nullptr, nx, yslot, ycnt, carry, ccnt, clast, nch4);
-            dsa::k_spmv_fixup<false><<<(unsigned)((nch4 + 255) / 256), 256>>>(yslot, ycnt, carry, ccnt, clast, nch4); });
+            dsa::k_spmv_fixup<<<(unsigned)((nch4 + 255) / 256), 256>>>(yslot, ycnt, carry, ccnt, clast, nch4); });
     }
     return 0;
 }

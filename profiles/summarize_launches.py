@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Summarise an `ncu --metrics gpu__time_duration.sum --csv` launch list into per-kernel shares of one step.
-A step ends with the SpMV epilogue (k_spmv_fix_to_dense, k_spmv_to_dense before it); the last `--steps` complete steps are averaged.
+A step ends with the SpMV epilogue (k_spmm_fix_to_dense<true>, the one-column instance launched as "spmv_fix_to_dense";
+k_spmv_fix_to_dense and k_spmv_to_dense in older captures); the last `--steps` complete steps are averaged.
 usage: python profiles/summarize_launches.py gpurun_out/launches.csv [--steps 2] > profiles/launches_rXX.md"""
 import collections
 import csv
@@ -16,9 +17,10 @@ ki, vi = hdr.index("Kernel Name"), hdr.index("Metric Value")
 data = []
 for r in rows[hi + 1:]:
     if len(r) > vi:
-        name = re.sub(r"\(.*", "", r[ki]).replace("dsa::", "").replace("void ", "")
+        name = r[ki].replace("(bool)1", "true").replace("(bool)0", "false")   # template arguments as ncu may print them
+        name = re.sub(r"\(.*", "", name).replace("dsa::", "").replace("void ", "")
         data.append((name, float(r[vi].replace(",", "")) / 1e3))
-ends = [i for i, (n, _) in enumerate(data) if n.startswith("k_spmv_to_dense") or n.startswith("k_spmv_fix_to_dense")]
+ends = [i for i, (n, _) in enumerate(data) if n.startswith(("k_spmm_fix_to_dense<true>", "k_spmv_fix_to_dense", "k_spmv_to_dense"))]
 if len(ends) < nsteps + 1:
     nsteps = max(len(ends) - 1, 1)
 lo, hi_ = ends[-nsteps - 1] + 1, ends[-1] + 1

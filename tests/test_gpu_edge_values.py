@@ -700,6 +700,29 @@ def test_matrix_keys_near_2_62(high, mode):
     step("creating", bi, bj, spread(rng, 440), {"make_sortkeys"})
 
 
+def test_dense_key_maps_at_extreme_keys():
+    """row and column keys 1..N, so both orientations look partition keys up in the direct-address table: reads naming an
+    extreme row or column, through each orientation, and a batch naming an extreme column is refused with nothing changed"""
+    rng = np.random.default_rng(4900)
+    n = 300
+    live = np.arange(1, n + 1)
+    I, J = np.concatenate([live, rng.integers(1, n + 1, 6000)]), np.concatenate([rng.permutation(live), rng.integers(1, n + 1, 6000)])
+    V = spread(rng, len(I))
+    gm, seq = D.dynamicsparse(I, J, V), O.Matrix(I, J, V)
+    rq = np.concatenate([np.repeat(EXTREME, n), np.tile(live, len(EXTREME))])    # (extreme row, live column), then
+    cq = np.concatenate([np.tile(live, len(EXTREME)), np.repeat(EXTREME, n)])    # (live row, extreme column)
+    for which in (0, 1):
+        assert np.array_equal(bits(gm.get_batch(rq, cq, which=which)), bits(seq.get_many(rq, cq, which=which))), which
+    before = [gm.export(w) for w in (0, 1)]
+    with pytest.raises(D.ArgumentError):
+        gm.set_batch([5, 7], [3, -(2 ** 63) + 1], [1.0, 2.0])
+    for w in (0, 1):
+        after = gm.export(w)
+        for f in ("tag", "key", "val", "semaphores", "col_keys", "col_live"):
+            assert np.array_equal(bits(after[f]) if f == "val" else after[f], bits(before[w][f]) if f == "val" else before[w][f]), (w, f)
+    assert gm.size == seq.size
+
+
 def test_documented_refusals_leave_the_structure_unchanged():
     rng = np.random.default_rng(4800)
     with pytest.raises(D.ArgumentError):
